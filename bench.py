@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the sift path on B200 — the metric of BASELINE.json.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Primary line (one JSON object on stdout, rank 0):
@@ -25,6 +25,9 @@ Primary line (one JSON object on stdout, rank 0):
            100 M-row size (k = 10 and 100, verified) and the config-5 all-pairs graph.
 
 --impl reference times the reference-side CPU implementation only (rank 0), same metric/config.
+--dump-outputs DIR writes what the last timed step returned (rank 0): DIR/scores.npy and
+DIR/indices.npy.  The inputs are seeded, so two builds run with the same arguments can be compared
+output for output.
 """
 
 from __future__ import annotations
@@ -227,6 +230,17 @@ def run_reference(args) -> None:
         "gpu_launches": 0,
     }
     print(json.dumps(line), flush=True)
+
+
+def dump_outputs(out_dir: str, scores, indices) -> None:
+    """Write one timed step's result as `scores.npy` (float32, Q x k) and `indices.npy` (float64,
+    Q x k: every int32 row index is exact in it), so that two builds can be compared output for
+    output on the same seeded inputs.  10 k x 10 entries: 1.2 MB in all."""
+    import numpy as np
+
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "scores.npy"), scores.cpu().numpy().astype(np.float32))
+    np.save(os.path.join(out_dir, "indices.npy"), indices.cpu().numpy().astype(np.float64))
 
 
 def workload_config(n_gpus: int) -> dict:
@@ -794,15 +808,19 @@ def run_b200(args) -> None:
             e1.record(stream)
             ev_pairs.append((e0, e1))
 
+    last_out: list = [None]  # (scores, indices) of the latest step: what --dump-outputs writes
+
     def step(q_dev=queries, record=True):
         if dist_on:
             # row norms + fused search whose finalising pass stores the packed records into every rank's
             # gather buffer over NVLink (symmetric memory) + device barrier + merge; NCCL all-gather of
             # the packed records where peer mapping is unavailable
             sharded._event_sink = ev_pairs if record else None
-            return sharded.search_raw(q_dev, K)
-        search_local(q_dev, record)
-        return scores, idx
+            last_out[0] = sharded.search_raw(q_dev, K)
+        else:
+            search_local(q_dev, record)
+            last_out[0] = (scores, idx)
+        return last_out[0]
 
     # kernels of mine per step: row_rnorm + search + finalise(+scatter) (+ cross-rank merge); the two
     # memsets, the symmetric-memory barrier / NCCL all-gather are library work
@@ -821,6 +839,8 @@ def run_b200(args) -> None:
     with ClockSampler(local_rank) as clocks:
         # warm-up happens inside timed_steps; events recorded during warm-up are dropped below
         sec = timed_steps(step, args.steps, args.warmup, dist_on)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, *last_out[0])
     kernel_ms = [e0.elapsed_time(e1) for e0, e1 in ev_pairs[args.warmup:]]
     clock_summary = clocks.summary()
     value = Q / sec
@@ -1143,7 +1163,14 @@ def main() -> None:
     ap.add_argument("--no-verify", action="store_true", help="skip the untimed sampled brute-force verification")
     ap.add_argument("--preheat", type=float, default=2.0, help="seconds of untimed steps before the timed loop (clock steady state)")
     ap.add_argument("--large-rows-per-gpu", type=int, default=0, help="config-4 leg at N > 1: rows per GPU (0 = 100 M / N when it fits)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the metric's result of the last timed step (scores, indices) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        # the reference arm sizes its query sample from a timing calibration: not the same inputs every run
+        ap.error("--dump-outputs needs --impl b200")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     if args.impl == "reference":
         run_reference(args)

@@ -251,6 +251,24 @@ def test_sharded_gather_plumbing_gloo_world2(tmp_path):
         assert p.returncode == 0 and f"OK {r}" in o, o
 
 
+def test_bench_dump_outputs_and_argument_checks(tmp_path):
+    """bench.py --dump-outputs: scores as float32 and indices as float64, every index exact (2^24 + 1
+    is not representable in float32); --steps below 1 and a dump of the calibrated reference arm are
+    rejected before any device work."""
+    from bench import dump_outputs
+
+    s = torch.tensor([[0.75, -0.125], [float("-inf"), 1.0]])
+    i = torch.tensor([[(1 << 24) + 1, 3], [-1, 999_999]], dtype=torch.int32)
+    dump_outputs(str(tmp_path / "out"), s, i)
+    got_s, got_i = np.load(tmp_path / "out" / "scores.npy"), np.load(tmp_path / "out" / "indices.npy")
+    assert got_s.dtype == np.float32 and np.array_equal(got_s, s.numpy())
+    assert got_i.dtype == np.float64 and np.array_equal(got_i, i.numpy().astype(np.int64))
+    for argv in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", str(tmp_path / "ref")]):
+        r = subprocess.run([sys.executable, os.path.join(REPO, "bench.py"), *argv], capture_output=True, text=True, timeout=120)
+        assert r.returncode == 2 and "error:" in r.stderr, (argv, r.stderr)
+    assert not (tmp_path / "ref").exists()
+
+
 def test_store_format_codec_matches_reference_wire_format():
     """storage/models.py:94-129: float32 C-order bytes; decode(encode(x)) == x and the byte string
     equals numpy's tobytes() of the C×H×W array (what `Embedding.create` writes)."""
