@@ -92,6 +92,12 @@ SIGNATURES: dict[str, tuple] = {
     ),
     "isx_topk_merge": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p]),
     "isx_topk_merge_packed": (c_int, [c_void_p, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p]),
+    "isx_knn_search_grouped": (
+        c_int,
+        [c_void_p, c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_int, c_int, c_int, c_int64, c_void_p, c_void_p,
+         c_void_p, c_void_p, c_size_t, c_void_p],
+    ),
+    "isx_topk_merge_grouped": (c_int, [c_void_p, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p]),
     "isx_roi_rasterize": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int64, c_void_p, c_void_p]),
     "isx_masked_pool": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_int, c_int64, c_void_p, c_void_p]),
 }

@@ -210,6 +210,7 @@ struct KnnParams {
   uint32_t* thr_shared;  // [q] per-query lower bound on the global k-th best (ordered-uint encoding)
   uint32_t throttle_window, throttle_every;
   uint32_t* progress;    // [units] tiles loaded so far by every scheduling unit (lockstep throttle)
+  const int32_t* row_group;  // [n] group id of every store row (grouped search only)
 #ifdef ISX_KNN_PROFILE
   unsigned long long* prof;  // [16] wait-cycle counters (diagnostic build only: -DISX_KNN_PROFILE)
   int debug_skip_select;     // ISX_KNN_SKIP_SELECT=1: the epilogue only loads and releases (floor of the MMA pipeline)
@@ -243,7 +244,7 @@ struct KnnParams {
 // Shared-memory plan.  k <= kSmallK: 32-entry per-row candidate buffers live in shared memory next to
 // a 4-stage operand ring (the buffers are XOR-swizzled by row so that 32 rows appending at the same
 // depth hit different banks).  Larger k: 256-entry buffers in the global workspace.
-template <int CAP, int NCTA, bool RES_ = false>
+template <int CAP, int NCTA, bool RES_ = false, bool GROUPED = false>
 struct KnnSmem {
   // RES: the query tile (all k-blocks, at most kResKb = 4, i.e. d <= 256) stays resident in shared
   // memory for a whole item and the ring holds store tiles only: half the operand traffic per tile.
@@ -262,7 +263,9 @@ struct KnnSmem {
   static constexpr uint32_t kBarOff = kRnormOff + ACC_STAGES * BN * 4;    // mbarriers
   static constexpr uint32_t kNumBars = 2 * STAGES + 2 * ACC_STAGES + 2;  // + resident-query full / empty
   static constexpr uint32_t kTmemPtrOff = kBarOff + kNumBars * 8;
-  static constexpr uint32_t kTotal = kTmemPtrOff + 16;
+  // grouped search: [ACC_STAGES][BN / 32] flags, 1 where all 32 store rows of a chunk are one group
+  static constexpr uint32_t kChunkUniOff = kTmemPtrOff + 16;
+  static constexpr uint32_t kTotal = kChunkUniOff + (GROUPED ? ACC_STAGES * (BN / 32) * 4 : 0);
   // the operand tiles need 1024-byte alignment; the dynamic window normally starts aligned, so only
   // as much slack as the 227 KB limit leaves is requested and the kernel checks that it suffices
   static constexpr uint32_t kMaxDynamic = 232448;
@@ -406,11 +409,164 @@ __device__ __forceinline__ bool prune_row_select(uint2* row_buf, int count, int 
   return true;
 }
 
-template <int CAP, int NCTA, bool RES>
-__global__ void __launch_bounds__(knn_threads(CAP), 1)
-knn_search_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_constant__ CUtensorMap tmap_e,
-                  const KnnParams p) {
-  using L = KnnSmem<CAP, NCTA, RES>;
+// ---- grouped selection (image-level search) ----------------------------------------------------
+// Every store row r carries a group id g(r) >= 0.  A group's score is the best score of its rows and
+// its representative is its first row in (score desc, row asc) order; the result is the k best
+// representatives.  Empty entries are (-inf, INT_MAX) with group -1.  An entry may be dropped as soon
+// as an entry of its group that sorts before it is known: it can never be a representative.
+
+// group of a candidate (global row; the table is indexed by store-local row)
+__device__ __forceinline__ int row_group_of(const int32_t* row_group, int index_base, int idx) {
+  return idx != INT_MAX ? __ldg(row_group + (idx - index_base)) : -1;
+}
+
+// One entry per lane, in any order.  Returns the entry's rank among the entries that are first of
+// their group, or -1 if an entry of the same group sorts before it (or it is empty); `distinct` = the
+// number of groups present.  The rank counting of prune_row plus one compare per step.
+__device__ __forceinline__ int grouped_rank32(float ms, int mi, int mg, int& distinct) {
+  uint32_t before = 0;
+  bool dup = false;
+#pragma unroll
+  for (int j = 0; j < 32; ++j) {
+    const float os = __shfl_sync(kFullMask, ms, j);
+    const int oi = __shfl_sync(kFullMask, mi, j);
+    const int og = __shfl_sync(kFullMask, mg, j);
+    const bool b = pair_before(os, oi, ms, mi);
+    before |= b ? (1u << j) : 0u;
+    dup |= b && og == mg;
+  }
+  const bool alive = mi != INT_MAX && !dup;
+  const uint32_t am = __ballot_sync(kFullMask, alive);
+  distinct = __popc(am);
+  return alive ? __popc(am & before) : -1;
+}
+
+// warp_sort_desc over (score, row, group) triples; BY_GROUP: order by (group asc, score desc, row asc)
+template <bool BY_GROUP>
+__device__ __forceinline__ bool entry_before(float sa, int ia, int ga, float sb, int ib, int gb) {
+  if constexpr (BY_GROUP) return ga < gb || (ga == gb && pair_before(sa, ia, sb, ib));
+  else return pair_before(sa, ia, sb, ib);
+}
+
+template <int E, bool BY_GROUP>
+__device__ __forceinline__ void warp_sort3(float (&s)[E], int (&idx)[E], int (&g)[E]) {
+  const uint32_t lane = lane_id();
+  constexpr int TOTAL = 32 * E;
+#pragma unroll
+  for (int k = 2; k <= TOTAL; k <<= 1) {
+#pragma unroll
+    for (int j = k >> 1; j > 0; j >>= 1) {
+      if (j >= 32) {
+        const int je = j >> 5;
+#pragma unroll
+        for (int e = 0; e < E; ++e) {
+          const int pe = e ^ je;
+          if (pe > e) {
+            const bool desc_block = ((e * 32) & k) == 0;
+            const bool lower_first = entry_before<BY_GROUP>(s[e], idx[e], g[e], s[pe], idx[pe], g[pe]);
+            if (desc_block ? !lower_first : lower_first) {
+              float ts = s[e]; s[e] = s[pe]; s[pe] = ts;
+              int ti = idx[e]; idx[e] = idx[pe]; idx[pe] = ti;
+              int tg = g[e]; g[e] = g[pe]; g[pe] = tg;
+            }
+          }
+        }
+      } else {
+#pragma unroll
+        for (int e = 0; e < E; ++e) {
+          const int i = e * 32 + static_cast<int>(lane);
+          const float os = __shfl_xor_sync(kFullMask, s[e], j);
+          const int oi = __shfl_xor_sync(kFullMask, idx[e], j);
+          const int og = __shfl_xor_sync(kFullMask, g[e], j);
+          const bool desc_block = ((i & k) == 0);
+          const bool i_am_lower = ((lane & j) == 0);
+          const bool mine_first = entry_before<BY_GROUP>(s[e], idx[e], g[e], os, oi, og);
+          const bool keep_mine = (desc_block == i_am_lower) ? mine_first : !mine_first;
+          if (!keep_mine) { s[e] = os; idx[e] = oi; g[e] = og; }
+        }
+      }
+    }
+  }
+}
+
+// 32*E entries (element i = e*32 + lane, any order) -> the first entry of every group, sorted by
+// (score desc, row asc), empties behind them.  Returns the number of groups.  Two sorts: by group
+// to find the non-first entries (a neighbour of the same group sorts before them), then by score.
+template <int E>
+__device__ __forceinline__ int grouped_select(float (&s)[E], int (&idx)[E], int (&g)[E]) {
+  const int lane = static_cast<int>(lane_id());
+  warp_sort3<E, true>(s, idx, g);
+  int distinct = 0;
+  int carry = INT_MIN;  // group of element e*32 - 1
+#pragma unroll
+  for (int e = 0; e < E; ++e) {
+    const int up = __shfl_up_sync(kFullMask, g[e], 1);
+    const int prev = lane ? up : carry;
+    carry = __shfl_sync(kFullMask, g[e], 31);
+    const bool dead = idx[e] == INT_MAX || prev == g[e];
+    distinct += __popc(__ballot_sync(kFullMask, !dead));
+    if (dead) { s[e] = -INFINITY; idx[e] = INT_MAX; g[e] = -1; }
+  }
+  warp_sort3<E, false>(s, idx, g);
+  return distinct;
+}
+
+// Grouped form of prune_row: keep the representatives of the best k groups of the buffer, return the
+// score of the k-th (or -inf while fewer than k groups are present).  No bisection variant: a
+// selection without sorting cannot tell which entries share a group.
+template <int CAP>
+__device__ __forceinline__ void prune_row_grouped(uint2* row_buf, int swz, int count, int k, const int32_t* row_group,
+                                                  int index_base, float& new_thr, int& new_count) {
+  constexpr int E = CAP / 32;
+  const int lane = static_cast<int>(lane_id());
+  float s[E];
+  int idx[E], g[E];
+#pragma unroll
+  for (int e = 0; e < E; ++e) {
+    const int i = e * 32 + lane;
+    s[e] = -INFINITY;
+    idx[e] = INT_MAX;
+    if (i < count) {
+      const uint2 v = row_buf[i ^ swz];
+      s[e] = __uint_as_float(v.x);
+      idx[e] = static_cast<int>(v.y);
+    }
+    g[e] = row_group_of(row_group, index_base, idx[e]);
+  }
+  if constexpr (E == 1) {
+    int distinct;
+    const int rank = grouped_rank32(s[0], idx[0], g[0], distinct);
+    new_count = min(distinct, k);
+    __syncwarp();
+    if (rank >= 0 && rank < k) row_buf[rank ^ swz] = make_uint2(__float_as_uint(s[0]), static_cast<uint32_t>(idx[0]));
+    __syncwarp();
+    const uint32_t km = __ballot_sync(kFullMask, rank == k - 1);
+    new_thr = km ? __shfl_sync(kFullMask, s[0], __ffs(km) - 1) : -INFINITY;
+  } else {
+    const int distinct = grouped_select<E>(s, idx, g);
+    __syncwarp();
+    float kth = -INFINITY;
+#pragma unroll
+    for (int e = 0; e < E; ++e) {
+      const int i = e * 32 + lane;
+      if (i < k && i < distinct) row_buf[i ^ swz] = make_uint2(__float_as_uint(s[e]), static_cast<uint32_t>(idx[e]));
+      const float cand = __shfl_sync(kFullMask, s[e], (k - 1) & 31);
+      if (e == ((k - 1) >> 5)) kth = cand;
+    }
+    __syncwarp();
+    new_count = min(distinct, k);
+    new_thr = (distinct >= k) ? kth : -INFINITY;
+  }
+}
+
+// GROUPED: image-level search (knn_search_grouped_kernel).  The k-th best DISTINCT-GROUP score of
+// any subset of the store is a lower bound of the global one, so the fast path, the shared bound and
+// the item-end skip stay as they are; only where a threshold is derived — the buffer prune, the
+// item-end merge into the running list and the finalising merge — entries are de-duplicated by group
+// before k are counted.
+template <int CAP, int NCTA, bool RES, bool GROUPED>
+__device__ __forceinline__ void knn_search_body(const CUtensorMap& tmap_q, const CUtensorMap& tmap_e, const KnnParams& p) {
+  using L = KnnSmem<CAP, NCTA, RES, GROUPED>;
   constexpr int STAGES = L::STAGES;
   constexpr int kEpiGroups = L::G;
   constexpr int kGroupCols = BN / kEpiGroups;
@@ -645,10 +801,15 @@ knn_search_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_const
       // d = 256 where a tile is only 2048 MMA cycles long).
       float pre_rn = 0.f, pre_rn2 = 0.f;
       uint32_t pre_thr = 0;
+      int pre_g = -1, pre_g2 = -1;  // grouped: groups of the store rows whose inverse norms this thread stages
       auto prefetch_tile = [&](long long nb_) {
         const long long n0_ = nb_ * BN;
         pre_rn = (n0_ + et < p.n) ? __ldg(p.store_rnorm + n0_ + et) : 0.f;
         if (kEpiGroups == 1) pre_rn2 = (n0_ + et + 128 < p.n) ? __ldg(p.store_rnorm + n0_ + et + 128) : 0.f;
+        if constexpr (GROUPED) {
+          pre_g = (n0_ + et < p.n) ? __ldg(p.row_group + n0_ + et) : -1;
+          if (kEpiGroups == 1) pre_g2 = (n0_ + et + 128 < p.n) ? __ldg(p.row_group + n0_ + et + 128) : -1;
+        }
         if (row_valid) pre_thr = *reinterpret_cast<const volatile uint32_t*>(p.thr_shared + qrow);
       };
       prefetch_tile(nb0);
@@ -662,6 +823,18 @@ knn_search_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_const
         float* rn = rnorm_s + acc * BN;
         rn[et] = pre_rn;
         if (kEpiGroups == 1) rn[et + 128] = pre_rn2;
+        int* chunk_uni = reinterpret_cast<int*>(smem + L::kChunkUniOff) + acc * (BN / 32);
+        if constexpr (GROUPED) {
+          // the 32 rows this warp stages are one selection chunk: flag it when they are all one group
+          const int g0 = __shfl_sync(kFullMask, pre_g, 0);
+          const bool uni = __all_sync(kFullMask, pre_g == g0 && pre_g >= 0);
+          if (lane == 0) chunk_uni[et >> 5] = uni ? 1 : 0;
+          if (kEpiGroups == 1) {
+            const int g1 = __shfl_sync(kFullMask, pre_g2, 0);
+            const bool uni1 = __all_sync(kFullMask, pre_g2 == g1 && pre_g2 >= 0);
+            if (lane == 0) chunk_uni[(et + 128) >> 5] = uni1 ? 1 : 0;
+          }
+        }
         if (row_valid) thr = fmaxf(thr, thr_decode_below(pre_thr));
         if (nb + 1 < nb1) prefetch_tile(nb + 1);
         ISX_PROF_BEGIN();
@@ -698,12 +871,15 @@ knn_search_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_const
             float nthr;
             int ncnt;
             bool done = false;
-            if constexpr (!L::kSmemCand) {
+            if constexpr (!L::kSmemCand && !GROUPED) {
               // large buffers: select the k-th best and compact, no sort (c >= k here: a prune is only
               // asked for when the buffer is close to full)
               if (c >= p.k) done = prune_row_select<CAP>(warp_buf + static_cast<size_t>(rr) * cand_stride, c, p.k, nthr, ncnt);
             }
-            if (!done)
+            if constexpr (GROUPED)
+              prune_row_grouped<CAP>(warp_buf + static_cast<size_t>(rr) * cand_stride, L::kSmemCand ? rr : 0, c, p.k,
+                                     p.row_group, p.index_base, nthr, ncnt);
+            else if (!done)
               prune_row<CAP>(warp_buf + static_cast<size_t>(rr) * cand_stride, L::kSmemCand ? rr : 0, c, p.k, nthr, ncnt,
                              s_reg, i_reg);
             __syncwarp();
@@ -742,6 +918,26 @@ knn_search_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_const
           ISX_PROF_COUNT(10, 1);
           ISX_PROF_BEGIN1();
           const bool hit = vmax > thr;
+          if constexpr (GROUPED) {
+            // All 32 rows of the chunk belong to one group (per-cell stores with >= 32 cells per image):
+            // only the chunk's best column can represent that group, so a row appends that one entry
+            // instead of every column above its threshold.  This is what keeps the correlated cells of
+            // the best images, which pass the distinct-group threshold in bulk, from flooding the buffers.
+            if (chunk_uni[cbase >> 5]) {
+              prune_rows(__ballot_sync(kFullMask, hit && cnt >= CAP));
+              if (hit) {
+                int jb = 31;
+#pragma unroll
+                for (int j = 31; j >= 0; --j) jb = (__uint_as_float(r[j]) == vmax) ? j : jb;
+                my_buf[cnt ^ my_swz] = make_uint2(__float_as_uint(vmax), static_cast<uint32_t>(gcol0 + cbase + jb));
+                ++cnt;
+                row_best = fmaxf(row_best, vmax);
+              }
+              __syncwarp();
+              ISX_PROF_END1(13);
+              return;
+            }
+          }
           int ngrp = 0;
 #pragma unroll
           for (int j = 0; j < 8; ++j) ngrp += (g[j] > thr) ? 1 : 0;
@@ -910,8 +1106,12 @@ knn_search_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_const
             const int c = __shfl_sync(kFullMask, cnt, rr);
             float nthr;
             int ncnt;
-            prune_row<CAP>(warp_buf + static_cast<size_t>(rr) * cand_stride, L::kSmemCand ? rr : 0, c, p.k, nthr, ncnt,
-                           s_reg, i_reg);
+            if constexpr (GROUPED)
+              prune_row_grouped<CAP>(warp_buf + static_cast<size_t>(rr) * cand_stride, L::kSmemCand ? rr : 0, c, p.k,
+                                     p.row_group, p.index_base, nthr, ncnt);
+            else
+              prune_row<CAP>(warp_buf + static_cast<size_t>(rr) * cand_stride, L::kSmemCand ? rr : 0, c, p.k, nthr, ncnt,
+                             s_reg, i_reg);
             if (lane == rr) cnt = ncnt;
           }
           __syncwarp();
@@ -969,6 +1169,26 @@ knn_search_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_const
                 iv = static_cast<int>(v.y);
               }
               if (li[b] >= 0) { sv = ls[b]; iv = li[b]; }
+              if constexpr (GROUPED) {
+                // the item's groups and the running list's groups may overlap: rank the union with
+                // de-duplication and store the best k groups; no bound while fewer than k are present
+                int distinct;
+                const int rank = grouped_rank32(sv, iv, row_group_of(p.row_group, p.index_base, iv), distinct);
+                const size_t base = static_cast<size_t>(m0 + ew * 32 + rr) * p.k;
+                __syncwarp();
+                if (rank >= 0 && rank < p.k) {
+                  p.run_scores[base + rank] = sv;
+                  p.run_idx[base + rank] = iv;
+                }
+                if (lane >= distinct && lane < p.k) {
+                  p.run_scores[base + lane] = -INFINITY;
+                  p.run_idx[base + lane] = -1;
+                }
+                const uint32_t km = __ballot_sync(kFullMask, rank == p.k - 1);
+                const float cs = km ? __shfl_sync(kFullMask, sv, __ffs(km) - 1) : -INFINITY;
+                if (lane == rr) { kth_mine = cs; kth_valid_mine = km != 0; }
+                continue;
+              }
               s_reg[0] = sv;
               i_reg[0] = iv;
               warp_merge_desc<E>(s_reg, i_reg);
@@ -1039,7 +1259,12 @@ knn_search_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_const
             __syncwarp();
             float nthr;
             int ncnt;
-            if (kept <= 32) {
+            if constexpr (GROUPED) {
+              if (kept <= 32) prune_row_grouped<32>(buf, 0, kept, p.k, p.row_group, p.index_base, nthr, ncnt);
+              else if (kept <= 64) prune_row_grouped<64>(buf, 0, kept, p.k, p.row_group, p.index_base, nthr, ncnt);
+              else if (kept <= 128) prune_row_grouped<128>(buf, 0, kept, p.k, p.row_group, p.index_base, nthr, ncnt);
+              else prune_row_grouped<CAP>(buf, 0, kept, p.k, p.row_group, p.index_base, nthr, ncnt);
+            } else if (kept <= 32) {
               float s1[1];
               int i1[1];
               prune_row<32>(buf, 0, kept, p.k, nthr, ncnt, s1, i1);
@@ -1108,7 +1333,16 @@ knn_search_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_const
               s_reg[e] = sv;
               i_reg[e] = iv;
             }
-            warp_merge_desc<E>(s_reg, i_reg);
+            if constexpr (GROUPED) {
+              // the union may hold a group twice (once from this item, once from the running list);
+              // dropped entries sort last as (-inf, none), so slot k-1 is empty while fewer than k remain
+              int g_reg[E];
+#pragma unroll
+              for (int e = 0; e < E; ++e) g_reg[e] = row_group_of(p.row_group, p.index_base, i_reg[e]);
+              grouped_select<E>(s_reg, i_reg, g_reg);
+            } else {
+              warp_merge_desc<E>(s_reg, i_reg);
+            }
             float kth = -INFINITY;
             bool kth_valid = false;
 #pragma unroll
@@ -1158,6 +1392,20 @@ knn_search_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_const
     tc_fence_after();
     if (NCTA == 2) tmem_dealloc_pair(tmem_base, 512); else tmem_dealloc(tmem_base, 512);
   }
+}
+
+template <int CAP, int NCTA, bool RES>
+__global__ void __launch_bounds__(knn_threads(CAP), 1)
+knn_search_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_constant__ CUtensorMap tmap_e,
+                  const KnnParams p) {
+  knn_search_body<CAP, NCTA, RES, false>(tmap_q, tmap_e, p);
+}
+
+template <int CAP, int NCTA, bool RES>
+__global__ void __launch_bounds__(knn_threads(CAP), 1)
+knn_search_grouped_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_constant__ CUtensorMap tmap_e,
+                          const KnnParams p) {
+  knn_search_body<CAP, NCTA, RES, true>(tmap_q, tmap_e, p);
 }
 
 // ------------------------------------------------------------------------------------------
@@ -1256,6 +1504,81 @@ int launch_merge(const float* scores, const int32_t* idx, int g, int q, int k, c
   return ISX_OK;
 }
 
+// Grouped form: merge g partial lists of (score, row, group) into the k best groups per query, one
+// entry per group (its first in (score desc, row asc) order).  Input either as 12-byte records
+// {fp32 score bits, row, group} (`records`, what one all-gather of grouped results moves) or as the
+// search's running lists (`scores`, `idx`), whose groups are looked up in `row_group` (store-local
+// rows, idx - index_base) and whose raw scores are scaled by `query_scale`.  A group that appears in
+// several lists (cut by a shard or N-split boundary) comes out once.  Padding: idx < 0.
+template <int CAP>
+__global__ void __launch_bounds__(128)
+topk_merge_grouped_kernel(const int32_t* __restrict__ records, const float* __restrict__ scores,
+                          const int32_t* __restrict__ idx, const int32_t* __restrict__ row_group, int index_base,
+                          int g, int q, int k, const float* __restrict__ query_scale, float* __restrict__ out_scores,
+                          int32_t* __restrict__ out_rows, int32_t* __restrict__ out_groups) {
+  constexpr int E = CAP / 32;
+  const int lane = threadIdx.x & 31;
+  const int query = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  if (query >= q) return;
+  // the window keeps the best k groups of everything read so far; CAP - k slots take fresh entries
+  const int fresh = CAP - k;
+  const float qscale = query_scale ? query_scale[query] : 1.0f;
+  float s[E];
+  int id[E], gr[E];
+#pragma unroll
+  for (int e = 0; e < E; ++e) { s[e] = -INFINITY; id[e] = INT_MAX; gr[e] = -1; }
+  const long long total = static_cast<long long>(g) * k;
+  for (long long base = 0; base < total; base += fresh) {
+#pragma unroll
+    for (int e = 0; e < E; ++e) {
+      const int pos = e * 32 + lane;
+      if (pos >= k) {
+        const long long c = base + (pos - k);
+        s[e] = -INFINITY;
+        id[e] = INT_MAX;
+        gr[e] = -1;
+        if (c < total) {
+          const long long part = c / k, j = c - part * k;
+          const size_t off = (static_cast<size_t>(part) * q + query) * k + j;
+          if (records) {
+            const int3 v = *reinterpret_cast<const int3*>(records + 3 * off);
+            if (v.y >= 0) { s[e] = __int_as_float(v.x) * qscale; id[e] = v.y; gr[e] = v.z; }
+          } else {
+            const int raw = idx[off];
+            if (raw >= 0) { s[e] = scores[off] * qscale; id[e] = raw; gr[e] = row_group[raw - index_base]; }
+          }
+        }
+      }
+    }
+    grouped_select<E>(s, id, gr);
+  }
+#pragma unroll
+  for (int e = 0; e < E; ++e) {
+    const int pos = e * 32 + lane;
+    if (pos < k) {
+      const bool have = id[e] != INT_MAX;
+      const size_t o = static_cast<size_t>(query) * k + pos;
+      out_scores[o] = have ? s[e] : -INFINITY;
+      out_rows[o] = have ? id[e] : -1;
+      out_groups[o] = have ? gr[e] : -1;
+    }
+  }
+}
+
+int launch_merge_grouped(const int32_t* records, const float* scores, const int32_t* idx, const int32_t* row_group,
+                         int index_base, int g, int q, int k, const float* query_scale, float* out_scores,
+                         int32_t* out_rows, int32_t* out_groups, cudaStream_t stream) {
+  const int blocks = (q + 3) / 4;
+  if (k <= 32)
+    topk_merge_grouped_kernel<64><<<blocks, 128, 0, stream>>>(records, scores, idx, row_group, index_base, g, q, k,
+                                                              query_scale, out_scores, out_rows, out_groups);
+  else
+    topk_merge_grouped_kernel<256><<<blocks, 128, 0, stream>>>(records, scores, idx, row_group, index_base, g, q, k,
+                                                               query_scale, out_scores, out_rows, out_groups);
+  ISX_CHECK_CUDA(cudaGetLastError());
+  return ISX_OK;
+}
+
 size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
 struct KnnWorkspace {
@@ -1280,10 +1603,10 @@ KnnWorkspace knn_workspace(int max_grid, int q, int k) {
   return w;
 }
 
-template <int CAP, int NCTA, bool RES = false>
+template <int CAP, int NCTA, bool RES = false, bool GROUPED = false>
 int launch_search(const CUtensorMap& tq, const CUtensorMap& te, const KnnParams& p, int grid, cudaStream_t stream) {
-  auto kern = knn_search_kernel<CAP, NCTA, RES>;
-  const int smem = static_cast<int>(KnnSmem<CAP, NCTA, RES>::kDynamicBytes);
+  auto kern = GROUPED ? knn_search_grouped_kernel<CAP, NCTA, RES> : knn_search_kernel<CAP, NCTA, RES>;
+  const int smem = static_cast<int>(KnnSmem<CAP, NCTA, RES, GROUPED>::kDynamicBytes);
   ISX_CHECK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = dim3(static_cast<unsigned>(grid));
@@ -1370,7 +1693,10 @@ size_t isx_knn_workspace_bytes(int64_t n, int q, int d, int k) {
 static int knn_search_impl(const char* fn, const void* store, const float* store_rnorm, int64_t n, const void* queries,
                            const float* query_rnorm, int q, int d, int k, int64_t index_base,
                            int64_t query_index_base, int flags, float* out_scores, int32_t* out_idx,
-                           void* workspace, size_t workspace_bytes, isx_stream_t stream_, const PeerOut* peers) {
+                           void* workspace, size_t workspace_bytes, isx_stream_t stream_, const PeerOut* peers,
+                           const int32_t* row_group = nullptr, int32_t* out_groups = nullptr) {
+  // row_group != nullptr: grouped search (isx_knn_search_grouped), flags 0, outputs (scores, rows, groups)
+  const bool grouped = row_group != nullptr || out_groups != nullptr;
   const bool cont = (flags & ISX_KNN_CONTINUE) != 0, finalize = (flags & ISX_KNN_NO_FINALIZE) == 0;
   const bool packed = (flags & ISX_KNN_PACKED) != 0, no_self = (flags & ISX_KNN_EXCLUDE_SELF) != 0;
   ISX_REQUIRE((flags & ~(ISX_KNN_CONTINUE | ISX_KNN_NO_FINALIZE | ISX_KNN_EXCLUDE_SELF | ISX_KNN_PACKED)) == 0,
@@ -1383,6 +1709,8 @@ static int knn_search_impl(const char* fn, const void* store, const float* store
   ISX_REQUIRE(index_base >= 0 && index_base + n < (1ll << 31), "%s: index_base + n must fit in int32", fn);
   ISX_REQUIRE(queries && query_rnorm, "%s: null pointer", fn);
   ISX_REQUIRE(!finalize || peers || (out_scores && (packed || out_idx)), "%s: null output pointer", fn);
+  ISX_REQUIRE(!grouped || (out_groups && flags == 0 && !peers), "%s: null output pointer", fn);
+  ISX_REQUIRE(!grouped || n == 0 || row_group, "%s: null row_group pointer", fn);
   ISX_REQUIRE(!no_self || (query_index_base >= 0 && query_index_base + q < (1ll << 31)),
               "%s: query_index_base + q must fit in int32 (got %lld)", fn, (long long)query_index_base);
   ISX_REQUIRE((reinterpret_cast<uintptr_t>(queries) & 15u) == 0 && (reinterpret_cast<uintptr_t>(store) & 15u) == 0,
@@ -1405,6 +1733,9 @@ static int knn_search_impl(const char* fn, const void* store, const float* store
   if (n == 0) {
     // nothing to search in this block: the lists stay as they are
     if (!finalize) return ISX_OK;
+    if (grouped)
+      return launch_merge_grouped(nullptr, run_scores, run_idx, row_group, static_cast<int>(index_base), 1, q, k,
+                                  query_rnorm, out_scores, out_idx, out_groups, stream);
     return launch_merge(run_scores, run_idx, 1, q, k, query_rnorm, out_scores, packed ? nullptr : out_idx, stream, peers);
   }
   ISX_REQUIRE(store && store_rnorm, "%s: null store pointer", fn);
@@ -1432,6 +1763,7 @@ static int knn_search_impl(const char* fn, const void* store, const float* store
   p.thr_shared = zero_base;
   p.progress = p.thr_shared + q;
   p.run_lock = p.progress + 256;
+  p.row_group = row_group;
   // a continued search keeps the lists and the bounds they imply; only the lockstep counters restart
   if (cont) ISX_CHECK_CUDA(cudaMemsetAsync(p.progress, 0, 256 * sizeof(uint32_t), stream));
   // Lockstep window in tiles: measured best 16-32 at d = 1280 (640 KB of store rows per tile); it is a
@@ -1453,9 +1785,20 @@ static int knn_search_impl(const char* fn, const void* store, const float* store
   p.prof = d_prof;
   p.debug_skip_select = getenv("ISX_KNN_SKIP_SELECT") ? atoi(getenv("ISX_KNN_SKIP_SELECT")) : 0;
 #endif
-  if (ncta == 2) {
+  // the grouped search picks the same (CAP, NCTA, RES) variant as the plain one for the same (q, d, k):
+  // same MMA shapes, same scaling, bit-identical scores
+  static const bool no_res = [] { const char* e = getenv("ISX_KNN_RESIDENT"); return e && e[0] == '0'; }();
+  if (grouped) {
+    if (ncta == 2) {
+      if (k <= kSmallK && d <= 256 && !no_res) rc = launch_search<32, 2, true, true>(tq, te, p, plan.grid, stream);
+      else if (k <= kSmallK) rc = launch_search<32, 2, false, true>(tq, te, p, plan.grid, stream);
+      else rc = launch_search<256, 2, false, true>(tq, te, p, plan.grid, stream);
+    } else {
+      if (k <= kSmallK) rc = launch_search<32, 1, false, true>(tq, te, p, plan.grid, stream);
+      else rc = launch_search<256, 1, false, true>(tq, te, p, plan.grid, stream);
+    }
+  } else if (ncta == 2) {
     // short rows, small k: the query tile stays resident (ISX_KNN_RESIDENT=0 switches it off)
-    static const bool no_res = [] { const char* e = getenv("ISX_KNN_RESIDENT"); return e && e[0] == '0'; }();
     if (k <= kSmallK && d <= 256 && !no_res) rc = launch_search<32, 2, true>(tq, te, p, plan.grid, stream);
     else if (k <= kSmallK) rc = launch_search<32, 2>(tq, te, p, plan.grid, stream);
     else rc = launch_search<256, 2>(tq, te, p, plan.grid, stream);
@@ -1487,6 +1830,9 @@ static int knn_search_impl(const char* fn, const void* store, const float* store
   }
 #endif
   if (!finalize) return ISX_OK;
+  if (grouped)
+    return launch_merge_grouped(nullptr, p.run_scores, p.run_idx, row_group, p.index_base, 1, q, k, query_rnorm,
+                                out_scores, out_idx, out_groups, stream);
   // finalize: scale the running lists by the queries' inverse norms, order by the final
   // (score desc, row asc); packed: one 8-byte record per hit (what a single all-gather moves)
   return launch_merge(p.run_scores, p.run_idx, 1, q, k, query_rnorm, out_scores, packed ? nullptr : out_idx, stream, peers);
@@ -1537,6 +1883,26 @@ int isx_topk_merge(const float* scores, const int32_t* idx, int g, int q, int k,
   ISX_REQUIRE(k <= kMaxK, "%s: k = %d exceeds the supported maximum of %d", fn, k, kMaxK);
   ISX_REQUIRE(out_scores && out_idx && (g == 0 || (scores && idx)), "%s: null pointer", fn);
   return launch_merge(scores, idx, g, q, k, nullptr, out_scores, out_idx, stream);
+}
+
+int isx_knn_search_grouped(const void* store, const float* store_rnorm, const int32_t* row_group, int64_t n,
+                           const void* queries, const float* query_rnorm, int q, int d, int k, int64_t index_base,
+                           float* out_scores, int32_t* out_rows, int32_t* out_groups, void* workspace,
+                           size_t workspace_bytes, isx_stream_t stream) {
+  return knn_search_impl("isx_knn_search_grouped", store, store_rnorm, n, queries, query_rnorm, q, d, k, index_base, 0,
+                         0, out_scores, out_rows, workspace, workspace_bytes, stream, nullptr, row_group, out_groups);
+}
+
+int isx_topk_merge_grouped(const int32_t* records, int g, int q, int k, float* out_scores, int32_t* out_rows,
+                           int32_t* out_groups, isx_stream_t stream_) {
+  const char* fn = "isx_topk_merge_grouped";
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  ISX_REQUIRE(g >= 0 && q > 0 && k > 0, "%s: need g >= 0, q > 0, k > 0 (g=%d q=%d k=%d)", fn, g, q, k);
+  ISX_REQUIRE(k <= kMaxK, "%s: k = %d exceeds the supported maximum of %d", fn, k, kMaxK);
+  ISX_REQUIRE(out_scores && out_rows && out_groups && (g == 0 || records), "%s: null pointer", fn);
+  ISX_REQUIRE((reinterpret_cast<uintptr_t>(records) & 3u) == 0, "%s: records must be 4-byte aligned", fn);
+  return launch_merge_grouped(g ? records : nullptr, nullptr, nullptr, nullptr, 0, g, q, k, nullptr, out_scores,
+                              out_rows, out_groups, stream);
 }
 
 int isx_topk_merge_packed(const void* records, int g, int q, int k, float* out_scores, int32_t* out_idx,

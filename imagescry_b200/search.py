@@ -104,6 +104,84 @@ def unpack_records(records: Tensor) -> tuple[Tensor, Tensor]:
     return words[..., 0].contiguous().view(torch.float32), words[..., 1].contiguous()
 
 
+def group_offsets(groups, num_rows: int) -> Tensor:
+    """Validate a store's image layout and return it as `row_offsets` (int64 CPU, images + 1 entries):
+    image i owns rows [offsets[i], offsets[i + 1]).  `groups` is an int `c` (every image has c
+    consecutive rows; num_rows % c == 0) or a 1-D integer tensor of row offsets from 0 to num_rows,
+    non-decreasing (`store_from_mixed_blobs`)."""
+    if isinstance(groups, bool):
+        raise ValueError("groups must be an int (rows per image) or a 1-D tensor of row offsets")
+    if isinstance(groups, int):
+        if groups < 1 or num_rows % groups:
+            raise ValueError(f"groups={groups} rows per image must be >= 1 and divide the store's {num_rows} rows")
+        return torch.arange(0, num_rows + 1, groups, dtype=torch.int64)
+    if not isinstance(groups, Tensor) or groups.ndim != 1 or groups.dtype.is_floating_point or groups.dtype == torch.bool:
+        raise ValueError("groups must be an int (rows per image) or a 1-D integer tensor of row offsets")
+    off = groups.detach().to(device="cpu", dtype=torch.int64)
+    if off.numel() < 1 or int(off[0]) != 0 or int(off[-1]) != num_rows:
+        raise ValueError(f"row offsets must run from 0 to the store's {num_rows} rows")
+    if bool((off[1:] < off[:-1]).any()):
+        raise ValueError("row offsets must be non-decreasing")
+    if off.numel() - 1 >= 2**31:
+        raise ValueError("at most 2^31 - 1 images")
+    return off
+
+
+def row_groups(offsets: Tensor, begin: int, end: int) -> Tensor:
+    """int32 image id of every row in [begin, end) under `offsets` (CPU)."""
+    rows = torch.arange(begin, end, dtype=torch.int64)
+    return (torch.searchsorted(offsets, rows, right=True) - 1).to(torch.int32)
+
+
+def image_cells(rows: Tensor, images: Tensor, first_row: Tensor) -> Tensor:
+    """Cell of every hit inside its image: representative row - the image's first row (int64;
+    -1 where images < 0, i.e. padding).  `first_row[i]` is image i's first row in the rows' numbering."""
+    rows = rows.to(torch.int64)
+    img = images.to(torch.int64)
+    valid = img >= 0
+    cells = rows - first_row.to(rows.device)[img.clamp(min=0)]
+    return torch.where(valid, cells, torch.full_like(cells, -1))
+
+
+def merge_topk_groups(records: Tensor, k: int | None = None) -> tuple[Tensor, Tensor, Tensor]:
+    """Merge G grouped partial results held as G×Q×k×3 int32 records {fp32 score bits, row, group}
+    (row < 0 = padding) into the k best groups per query: (scores fp32 Q×k, rows int32 Q×k, groups
+    int32 Q×k), each group once, ordered by (score desc, row asc)."""
+    _lib.require_cuda(records, "records")
+    if records.ndim != 4 or records.shape[3] != 3 or records.dtype != torch.int32:
+        raise ValueError("records must be a G×Q×k×3 int32 tensor")
+    g, q, kk, _ = records.shape
+    k = kk if k is None else k
+    if k != kk:
+        raise ValueError(f"k={k} does not match the partial lists' width {kk}")
+    r = records.contiguous()
+    out_s = torch.empty((q, k), dtype=torch.float32, device=r.device)
+    out_r = torch.empty((q, k), dtype=torch.int32, device=r.device)
+    out_g = torch.empty((q, k), dtype=torch.int32, device=r.device)
+    if q:
+        with _lib.on_device(r) as stream:
+            rc = _lib.load().isx_topk_merge_grouped(r.data_ptr(), g, q, k, out_s.data_ptr(), out_r.data_ptr(),
+                                                    out_g.data_ptr(), stream)
+        _lib.check(rc, "isx_topk_merge_grouped")
+    return out_s, out_r, out_g
+
+
+def pack_group_records(scores: Tensor, rows: Tensor, groups: Tensor) -> Tensor:
+    """(fp32 score, int32 row, int32 group) Q×k → Q×k×3 int32 records, the form one all-gather moves."""
+    return torch.stack([scores.contiguous().float().view(torch.int32), rows.to(torch.int32), groups.to(torch.int32)], dim=-1)
+
+
+def gather_group_records(records: Tensor, group=None) -> Tensor:
+    """All-gather every rank's Q×k×3 grouped records: returns G×Q×k×3 (one collective)."""
+    import torch.distributed as dist
+
+    world = dist.get_world_size(group)
+    q, k, three = records.shape
+    out = torch.empty((world * q, k, three), dtype=records.dtype, device=records.device)
+    dist.all_gather_into_tensor(out, records.contiguous(), group=group)
+    return out.view(world, q, k, three)
+
+
 def _as_bf16_matrix(x: Tensor, name: str) -> Tensor:
     """bf16, contiguous, and — the kernel's TMA rows are 16-byte units — zero-padded to a multiple of
     8 features.  Zero features change neither dot products nor norms, so cosine scores are unchanged
@@ -129,16 +207,30 @@ class EmbeddingStore:
     products exactly, accumulates in fp32 and applies both inverse norms in the epilogue.
 
     A store may be searched from several CUDA streams: the scratch workspace (running top-k lists,
-    per-query locks and bounds) is cached per stream."""
+    per-query locks and bounds) is cached per stream.
 
-    def __init__(self, embeddings: Tensor, *, index_base: int = 0) -> None:
+    `groups` describes which rows belong to one image (a per-cell store has one row per feature-map
+    cell): an int `c` (rows [i·c, (i+1)·c) are image i) or a 1-D int64 tensor of `row_offsets`
+    (image i owns rows [offsets[i], offsets[i + 1])).  It enables `search_images`."""
+
+    def __init__(self, embeddings: Tensor, *, index_base: int = 0, groups: int | Tensor | None = None) -> None:
         if embeddings.ndim != 2:
             raise ValueError(f"embeddings must be 2-D (rows × features), got shape {tuple(embeddings.shape)}")
+        offsets = None if groups is None else group_offsets(groups, embeddings.shape[0])
         self.num_features = embeddings.shape[1]
         self.embeddings = _as_bf16_matrix(embeddings, "embeddings")
         self.index_base = int(index_base)
         self.rnorm = row_rnorm(self.embeddings)
         self._workspaces: dict[int, Tensor] = {}
+        self.row_group: Tensor | None = None
+        if offsets is not None:
+            self._set_groups(offsets, 0, self.index_base)
+
+    def _set_groups(self, offsets: Tensor, begin: int, row0: int) -> None:
+        """Rows of this store are rows [begin, begin + len) of the layout `offsets`; a hit's row in
+        the results is row0 + its layout row."""
+        self.row_group = row_groups(offsets, begin, begin + len(self)).to(self.device)
+        self.group_first_row = (offsets[:-1] + row0).to(self.device)
 
     def __len__(self) -> int:
         return self.embeddings.shape[0]
@@ -225,6 +317,40 @@ class EmbeddingStore:
         scores, idx = self.search_raw(queries, k)
         return scores, idx.to(torch.int64)
 
+    def search_images_raw(self, queries: Tensor, k: int) -> tuple[Tensor, Tensor, Tensor]:
+        """Local image-level top-k: (scores fp32 Q×k, representative rows int32 Q×k in the store's
+        global numbering, images int32 Q×k); padding (-inf, -1, -1)."""
+        if self.row_group is None:
+            raise ValueError("search_images needs a store built with groups= (rows per image or row offsets)")
+        q = self._queries(queries)
+        self._check_k(k)
+        nq = q.shape[0]
+        scores = torch.empty((nq, k), dtype=torch.float32, device=self.device)
+        rows = torch.empty((nq, k), dtype=torch.int32, device=self.device)
+        images = torch.empty((nq, k), dtype=torch.int32, device=self.device)
+        if nq == 0:
+            return scores, rows, images
+        qr = row_rnorm(q)
+        lib = _lib.load()
+        with torch.cuda.device(self.device):
+            ws = self._ws(max(int(lib.isx_knn_workspace_bytes(max(len(self), 1), nq, q.shape[1], k)), 256))
+        with _lib.on_device(self.embeddings, q, qr, ws, self.row_group) as stream:
+            rc = lib.isx_knn_search_grouped(
+                self.embeddings.data_ptr(), self.rnorm.data_ptr(), self.row_group.data_ptr(), len(self), q.data_ptr(),
+                qr.data_ptr(), nq, q.shape[1], k, self.index_base, scores.data_ptr(), rows.data_ptr(), images.data_ptr(),
+                ws.data_ptr(), ws.numel(), stream,
+            )
+        _lib.check(rc, "isx_knn_search_grouped")
+        return scores, rows, images
+
+    def search_images(self, queries: Tensor, k: int) -> tuple[Tensor, Tensor, Tensor]:
+        """The k most similar IMAGES of every query row: (scores fp32 Q×k, images int64 Q×k, cells
+        int64 Q×k).  An image scores its best cell (the cosine of `search`); `cells` is that cell's
+        position in the image (its row - the image's first row; the lowest such row on ties).  Ordered
+        by (score desc, row asc); if the store has fewer than k images the tail is (-inf, -1, -1)."""
+        scores, rows, images = self.search_images_raw(queries, k)
+        return scores, images.to(torch.int64), image_cells(rows, images, self.group_first_row)
+
     def knn_graph(self, k: int) -> tuple[Tensor, Tensor]:
         """All-pairs similarity graph (BASELINE.json config 5): the k nearest OTHER rows of every row,
         (scores N×k fp32, indices N×k int64).  One fused search with the store's own rows as queries;
@@ -292,9 +418,12 @@ class ShardedEmbeddingStore:
     """Row-sharded store over the ranks of a process group (one process per GPU).
 
     `local_embeddings` are this rank's rows; their global indices start at `index_base` (by default
-    the contiguous partition of `shard_range`).  Queries are replicated on every rank."""
+    the contiguous partition of `shard_range`).  Queries are replicated on every rank.  `groups`
+    (rows per image, or row offsets) describes the GLOBAL rows, as for `EmbeddingStore`; an image may
+    be cut by a shard boundary."""
 
-    def __init__(self, local_embeddings: Tensor, *, total_rows: int | None = None, index_base: int | None = None, group=None) -> None:
+    def __init__(self, local_embeddings: Tensor, *, total_rows: int | None = None, index_base: int | None = None, group=None,
+                 groups: int | Tensor | None = None) -> None:
         import torch.distributed as dist
 
         self.group = group
@@ -311,6 +440,22 @@ class ShardedEmbeddingStore:
             index_base = begin
         self.total_rows = total_rows
         self.local = EmbeddingStore(local_embeddings, index_base=index_base)
+        if groups is not None:
+            if isinstance(groups, int) and not isinstance(groups, bool) and total_rows is None:
+                raise ValueError("groups given as rows per image need total_rows")
+            total = total_rows if total_rows is not None else int(torch.as_tensor(groups)[-1])
+            offsets = group_offsets(groups, total)
+            if index_base + len(self.local) > total:
+                raise ValueError(f"rows [{index_base}, {index_base + len(self.local)}) exceed the layout's {total} rows")
+            self.local._set_groups(offsets, index_base, 0)
+
+    def search_images(self, queries: Tensor, k: int) -> tuple[Tensor, Tensor, Tensor]:
+        """`EmbeddingStore.search_images` over the sharded store: local grouped search, ONE all-gather of
+        the Q×k×3 int32 records {score, row, image}, grouped merge (an image cut by a shard boundary
+        comes out once, with its best cell)."""
+        s, r, g = self.local.search_images_raw(queries, k)
+        merged_s, merged_r, merged_g = merge_topk_groups(gather_group_records(pack_group_records(s, r, g), self.group), k)
+        return merged_s, merged_g.to(torch.int64), image_cells(merged_r, merged_g, self.local.group_first_row)
 
     # ------------------------------------------------------------------ gather over peer memory
     def _peer_buffers(self, nq: int, k: int):

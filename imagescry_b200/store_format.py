@@ -74,10 +74,12 @@ def maps_to_rows(maps: Tensor, *, pool: str | None = None) -> Tensor:
 
 
 def store_from_maps(maps: Tensor, *, pool: str | None = None, index_base: int = 0, device=None) -> EmbeddingStore:
-    """Build a search store from a stack of embedding maps (host or device)."""
+    """Build a search store from a stack of embedding maps (host or device).  The store knows its
+    images (`groups` = H·W rows per image, or 1 when pooled), so `search_images` works on it."""
     if not maps.is_cuda:
         maps = maps.to(device or "cuda", non_blocking=True)
-    return EmbeddingStore(maps_to_rows(maps, pool=pool), index_base=index_base)
+    cells = 1 if pool else maps.shape[2] * maps.shape[3]
+    return EmbeddingStore(maps_to_rows(maps, pool=pool), index_base=index_base, groups=cells)
 
 
 def store_from_blobs(records: Iterable[tuple[bytes, int, int, int]], *, pool: str | None = None, index_base: int = 0, device=None) -> EmbeddingStore:
@@ -117,7 +119,7 @@ def store_from_mixed_blobs(
         n_rows = per_image[batch[0]]
         dst = torch.cat([torch.arange(int(row_offsets[i]), int(row_offsets[i]) + n_rows) for i in batch]).to(dev)
         rows.index_copy_(0, dst, part)
-    return EmbeddingStore(rows, index_base=index_base), row_offsets
+    return EmbeddingStore(rows, index_base=index_base, groups=row_offsets), row_offsets
 
 
 def rows_to_image_cell(rows: Tensor | Sequence[int], cells_per_image: int | Tensor) -> tuple[Tensor, Tensor]:

@@ -217,6 +217,25 @@ int isx_topk_merge(const float* scores, const int32_t* idx, int g, int q, int k,
 int isx_topk_merge_packed(const void* records, int g, int q, int k, float* out_scores, int32_t* out_idx,
                           isx_stream_t stream);
 
+/* Image-level (grouped) search: the k most similar GROUPS of rows, e.g. the images of a store with
+ * one row per feature-map cell.  row_group: int32 n, the group id (>= 0) of every store row; groups
+ * need not be contiguous or sorted.  A group's score is the best cosine score of its rows (the same
+ * score isx_knn_search computes) and its representative is its first row in (score desc, index asc)
+ * order.  out_scores fp32 q x k, out_rows int32 q x k (index_base + local row of the representative),
+ * out_groups int32 q x k, ordered by the representatives' (score desc, index asc); if fewer than k
+ * groups exist the tail is (-inf, -1, -1).  Selection is fused into the search kernel like the
+ * row-level top-k; the workspace is sized by isx_knn_workspace_bytes. */
+int isx_knn_search_grouped(const void* store, const float* store_rnorm, const int32_t* row_group, int64_t n,
+                           const void* queries, const float* query_rnorm, int q, int d, int k, int64_t index_base,
+                           float* out_scores, int32_t* out_rows, int32_t* out_groups,
+                           void* workspace, size_t workspace_bytes, isx_stream_t stream);
+/* Merge g grouped partial results (e.g. every shard's isx_knn_search_grouped output, gathered) into
+ * the k best groups per query, ordered as above.  records: int32 g x q x k x 3
+ * {fp32 score bits, global row, group}; row < 0 marks padding.  A group present in several partial
+ * lists (an image cut by a shard boundary) comes out once, with its best row. */
+int isx_topk_merge_grouped(const int32_t* records, int g, int q, int k, float* out_scores,
+                           int32_t* out_rows, int32_t* out_groups, isx_stream_t stream);
+
 /* ---- ROI masks on the feature-map grid (SURVEY.md 8f-4) ---------------------------------------
  * geometry.py:14-65 `create_roi_mask`: rasterio.features.rasterize(shapes, out_shape=(hf, wf),
  * transform=Affine.scale(w / wf, h / hf), fill=0, all_touched=True) * class_index.  rasterio / GDAL
