@@ -352,13 +352,7 @@ __device__ __forceinline__ void tc_mma_f16_pair_ts(uint32_t d_tmem, uint32_t a_t
       "r"(a_tmem), "l"(b_desc), "r"(idesc), "r"(accumulate)
       : "memory");
 }
-// registers -> TMEM: 32 lanes x 8 consecutive 32-bit columns (one row per thread)
-__device__ __forceinline__ void tmem_st_32x8(uint32_t taddr, const uint32_t (&r)[8]) {
-  asm volatile("tcgen05.st.sync.aligned.32x32b.x8.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8};" ::"r"(taddr),
-               "r"(r[0]), "r"(r[1]), "r"(r[2]), "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7])
-               : "memory");
-}
-// registers -> TMEM: 32 lanes x 4 consecutive 32-bit columns
+// registers -> TMEM: 32 lanes x 4 consecutive 32-bit columns (one row per thread)
 __device__ __forceinline__ void tmem_st_32x4(uint32_t taddr, const uint32_t (&r)[4]) {
   asm volatile("tcgen05.st.sync.aligned.32x32b.x4.b32 [%0], {%1, %2, %3, %4};" ::"r"(taddr), "r"(r[0]), "r"(r[1]),
                "r"(r[2]), "r"(r[3])

@@ -30,7 +30,6 @@
 #include <cuda_fp16.h>
 
 #include <algorithm>
-#include <cstdlib>
 
 namespace isx {
 namespace {
@@ -49,19 +48,18 @@ constexpr uint32_t A_PART_BYTES = PM * PK * 2;           // 16 KB (one of hi / l
 constexpr uint32_t A_STAGE_BYTES_P = 2 * A_PART_BYTES;   // hi + lo
 constexpr int P_ACC_STAGES = 2;
 
-// NCTA == 2 (CTA pair, cta_group::2): each CTA transforms its own 128 cells but stages only half of
-// the weight rows of every k-block, so the L2 -> shared-memory weight stream per SM halves and the
-// freed shared memory buys a third stage for both rings.
-// STAGED (pairs only): the raw fp32 128-cell x 64-feature boxes of the map arrive by TMA into a
-// three-deep ring (96 KB in flight per SM, no registers involved); the transform warps read them
-// from shared memory.  The weight and converted-operand rings have two stages each.
-template <int NCTA, bool STAGED>
+// The per-cell kernels run on CTA pairs (cta_group::2): each CTA transforms its own 128 cells but
+// stages only half of the weight rows of every k-block, so the L2 -> shared-memory weight stream per
+// SM halves and the freed shared memory buys a third stage for both rings of the register path.
+// STAGED: the raw fp32 128-cell x 64-feature boxes of the map arrive by TMA into a three-deep ring
+// (96 KB in flight per SM, no registers involved); the transform warps read them from shared
+// memory.  The weight and converted-operand rings then have two stages each.
+template <bool STAGED>
 struct ProjSmem {
-  static_assert(!STAGED || NCTA == 2, "raw staging needs the shared memory a CTA pair frees");
-  static constexpr uint32_t W_PART_BYTES = (kMaxComponents / NCTA) * PK * 2;  // 32 KB, or 16 KB per CTA of a pair
-  static constexpr uint32_t W_STAGE_BYTES = 2 * W_PART_BYTES;                 // hi + lo
-  static constexpr int A_STAGES = (NCTA == 2 && !STAGED) ? 3 : 2;
-  static constexpr int W_STAGES = (NCTA == 2 && !STAGED) ? 3 : 2;
+  static constexpr uint32_t W_PART_BYTES = (kMaxComponents / 2) * PK * 2;  // 16 KB per CTA of a pair
+  static constexpr uint32_t W_STAGE_BYTES = 2 * W_PART_BYTES;              // hi + lo
+  static constexpr int A_STAGES = STAGED ? 2 : 3;
+  static constexpr int W_STAGES = STAGED ? 2 : 3;
   static constexpr int RAW_STAGES = STAGED ? 3 : 0;
   static constexpr uint32_t RAW_STAGE_BYTES = PM * PK * 4;                   // 32 KB
   static constexpr uint32_t kAOff = 0;
@@ -129,26 +127,24 @@ struct ProjParams {
                       // the three-pass bf16 split; tmap_whi then describes the fp16 weight matrix
   int rowmajor;       // staged kernel: fmap is an n x E row-major matrix (hw == 1); tmap_x is a 2-D
                       // map with 128B-swizzled boxes of 128 rows x 32 features
-  int prefetch;       // 1: tmap_x describes fmap and warp 3 prefetches tiles into L2 ahead of the transform
   int normalize;
   long long tiles;
   const float* bias;
   float* out;
 };
 
-// HW: cells per image known at compile time (256 = 16x16, 64 = 8x8 maps: channel strides become
-// immediate load offsets), or 0 for any shape.  The fast paths also need E % 64 == 0.
-template <int HW, int NCTA>
-__global__ void __launch_bounds__(proj_threads(HW < 0), 1)
+// STAGED: raw tiles of the map staged by TMA (tmap_x); otherwise the register path, which loads the
+// map from global memory and takes any shape (tmap_x unused).
+template <bool STAGED>
+__global__ void __launch_bounds__(proj_threads(STAGED), 1)
 l2norm_project_kernel(const __grid_constant__ CUtensorMap tmap_whi, const __grid_constant__ CUtensorMap tmap_wlo,
                       const __grid_constant__ CUtensorMap tmap_x, const ProjParams p) {
-  constexpr bool STAGED = (HW < 0);  // HW == -1: raw tiles staged by TMA (pairs only)
-  using L = ProjSmem<NCTA, STAGED>;
+  using L = ProjSmem<STAGED>;
   constexpr int A_STAGES = L::A_STAGES, W_STAGES = L::W_STAGES, RAW_STAGES = L::RAW_STAGES;
   constexpr int TW = transform_warps(STAGED);
   constexpr uint32_t W_PART_BYTES = L::W_PART_BYTES, W_STAGE_BYTES = L::W_STAGE_BYTES;
-  const uint32_t rank = (NCTA == 2) ? cluster_ctarank() : 0u;
-  const long long unit = blockIdx.x / NCTA, num_units = gridDim.x / NCTA;
+  const uint32_t rank = cluster_ctarank();
+  const long long unit = blockIdx.x / 2, num_units = gridDim.x / 2;
   extern __shared__ uint8_t smem_raw[];
   // align by offsetting the shared array itself (not through an integer round trip) so the compiler
   // keeps the shared address space and emits LDS/STS instead of generic loads and stores
@@ -180,26 +176,23 @@ l2norm_project_kernel(const __grid_constant__ CUtensorMap tmap_whi, const __grid
     prefetch_tmap(&tmap_wlo);
   }
   if (warp == 1 && lane == 0) {
-    for (int i = 0; i < A_STAGES; ++i) { mbar_init(&a_full[i], TW * NCTA); mbar_init(&a_empty[i], 1); }
-    for (int i = 0; i < W_STAGES; ++i) { mbar_init(&w_full[i], NCTA); mbar_init(&w_empty[i], 1); }
+    for (int i = 0; i < A_STAGES; ++i) { mbar_init(&a_full[i], TW * 2); mbar_init(&a_empty[i], 1); }
+    for (int i = 0; i < W_STAGES; ++i) { mbar_init(&w_full[i], 2); mbar_init(&w_empty[i], 1); }
     for (int i = 0; i < P_ACC_STAGES; ++i) {
       mbar_init(&tmem_full[i], 1);
-      mbar_init(&tmem_empty[i], 4 * NCTA);
+      mbar_init(&tmem_empty[i], 4 * 2);
       mbar_init(&ss_full[i], STAGED ? TW : TW * 32);
       mbar_init(&ss_empty[i], 4);
     }
     for (int i = 0; i < RAW_STAGES; ++i) { mbar_init(&raw_full[i], 1); mbar_init(&raw_empty[i], TW); }
     fence_mbar_init();
   }
-  if (warp == 2) {
-    if (NCTA == 2) { tmem_alloc_pair(tmem_ptr, 512); tmem_relinquish_pair(); }
-    else { tmem_alloc(tmem_ptr, 512); tmem_relinquish(); }
-  }
+  if (warp == 2) { tmem_alloc_pair(tmem_ptr, 512); tmem_relinquish_pair(); }
   tc_fence_before();
-  if (NCTA == 2) cluster_sync_all(); else __syncthreads();
+  cluster_sync_all();
   tc_fence_after();
   const uint32_t tmem_base = *tmem_ptr;
-  const int w_rows = p.k_pad / NCTA;  // weight rows (components) this CTA stages per k-block
+  const int w_rows = p.k_pad / 2;  // weight rows (components) this CTA stages per k-block
   const uint32_t w_part_bytes = static_cast<uint32_t>(w_rows) * PK * 2;
 
   if (warp == 0) {
@@ -211,18 +204,14 @@ l2norm_project_kernel(const __grid_constant__ CUtensorMap tmap_whi, const __grid
         for (int kb = 0; kb < num_kb; ++kb) {
           mbar_wait(&w_empty[stage], phase ^ 1);
           uint8_t* dst = smem + L::kWOff + stage * W_STAGE_BYTES;
-          if (NCTA == 2 && STAGED && p.fast) {
+          if (STAGED && p.fast) {
             // single fp16 pass: one weight matrix (tmap_whi describes the fp16 copy)
             mbar_arrive_expect_tx_leader(&w_full[stage], w_part_bytes);
             tma_load_2d_pair(dst, &tmap_whi, &w_full[stage], kb * PK, row0, kEvictLast);
-          } else if (NCTA == 2) {
+          } else {
             mbar_arrive_expect_tx_leader(&w_full[stage], 2 * w_part_bytes);
             tma_load_2d_pair(dst, &tmap_whi, &w_full[stage], kb * PK, row0, kEvictLast);
             tma_load_2d_pair(dst + W_PART_BYTES, &tmap_wlo, &w_full[stage], kb * PK, row0, kEvictLast);
-          } else {
-            mbar_arrive_expect_tx(&w_full[stage], 2 * w_part_bytes);
-            tma_load_2d(dst, &tmap_whi, &w_full[stage], kb * PK, 0, kEvictLast);
-            tma_load_2d(dst + W_PART_BYTES, &tmap_wlo, &w_full[stage], kb * PK, 0, kEvictLast);
           }
           if (++stage == W_STAGES) { stage = 0; phase ^= 1; }
         }
@@ -231,8 +220,8 @@ l2norm_project_kernel(const __grid_constant__ CUtensorMap tmap_whi, const __grid
   } else if (warp == 1) {
     // ===================== MMA issuer =====================
     if (lane == 0 && rank == 0) {
-      const uint32_t idesc = make_idesc(/*bf16*/ 1, PM * NCTA, static_cast<uint32_t>(p.k_pad));
-      const uint32_t idesc_f16 = make_idesc(/*f16*/ 0, PM * NCTA, static_cast<uint32_t>(p.k_pad));
+      const uint32_t idesc = make_idesc(/*bf16*/ 1, PM * 2, static_cast<uint32_t>(p.k_pad));
+      const uint32_t idesc_f16 = make_idesc(/*f16*/ 0, PM * 2, static_cast<uint32_t>(p.k_pad));
       (void)idesc_f16;
       uint32_t as = 0, aph = 0, ws = 0, wph = 0, acc = 0, acc_phase = 0;
       for (long long tile = unit; tile < p.tiles; tile += num_units) {
@@ -252,39 +241,30 @@ l2norm_project_kernel(const __grid_constant__ CUtensorMap tmap_whi, const __grid
             const uint32_t o = k * P_UMMA_K * 2;
             const uint64_t dah = make_kmajor_sw128_desc(a_hi + o), dal = make_kmajor_sw128_desc(a_lo + o);
             const uint64_t dwh = make_kmajor_sw128_desc(w_hi + o), dwl = make_kmajor_sw128_desc(w_lo + o);
-            if (NCTA == 2 && STAGED && p.fast) {
+            if (STAGED && p.fast) {
               tc_mma_f16_pair(d_tmem, dah, dwh, idesc_f16, (kb | k) != 0);
-            } else if (NCTA == 2) {
+            } else {
               tc_mma_f16_pair(d_tmem, dah, dwh, idesc, (kb | k) != 0);
               tc_mma_f16_pair(d_tmem, dal, dwh, idesc, 1);
               tc_mma_f16_pair(d_tmem, dah, dwl, idesc, 1);
-            } else {
-              tc_mma_f16(d_tmem, dah, dwh, idesc, (kb | k) != 0);
-              tc_mma_f16(d_tmem, dal, dwh, idesc, 1);
-              tc_mma_f16(d_tmem, dah, dwl, idesc, 1);
             }
           }
-          if (NCTA == 2) { tc_commit_pair(&a_empty[as]); tc_commit_pair(&w_empty[ws]); }
-          else { tc_commit(&a_empty[as]); tc_commit(&w_empty[ws]); }
+          tc_commit_pair(&a_empty[as]);
+          tc_commit_pair(&w_empty[ws]);
           if (++as == A_STAGES) { as = 0; aph ^= 1; }
           if (++ws == W_STAGES) { ws = 0; wph ^= 1; }
         }
-        if (NCTA == 2) tc_commit_pair(&tmem_full[acc]); else tc_commit(&tmem_full[acc]);
+        tc_commit_pair(&tmem_full[acc]);
         if (++acc == P_ACC_STAGES) { acc = 0; acc_phase ^= 1; }
       }
     }
   } else if (warp == 3) {
-    // ===================== L2 prefetcher =====================
-    // The transform warps can keep only one k-block of loads in flight (registers); this lane asks
-    // the TMA unit to pull whole 128-cell x 64-feature boxes of the map into L2 kPrefetchDepth
-    // k-blocks ahead, paced by the same a_empty barriers the transform waits on, so that those loads
-    // find their lines in L2 instead of HBM.
     if (STAGED) {
-      // ===================== raw-tile TMA producer (staged mode) =====================
+      // ===================== raw-tile TMA producer (staged kernel) =====================
       if (lane == 0) {
         uint32_t rs = 0, rph = 0;
         for (long long tile = unit; tile < p.tiles; tile += num_units) {
-          const long long R0 = (tile * NCTA + rank) * PM;
+          const long long R0 = (tile * 2 + rank) * PM;
           const long long img = R0 / p.hw;
           const int cell = static_cast<int>(R0 - img * p.hw);
           for (int kb = 0; kb < num_kb; ++kb) {
@@ -302,27 +282,6 @@ l2norm_project_kernel(const __grid_constant__ CUtensorMap tmap_whi, const __grid
             if (++rs == static_cast<uint32_t>(RAW_STAGES)) { rs = 0; rph ^= 1; }
           }
         }
-      }
-    } else if (lane == 0 && p.prefetch) {
-      constexpr int kPrefetchDepth = 6;
-      const long long my_tiles = (p.tiles - unit + num_units - 1) / num_units;
-      const long long total_seq = my_tiles * num_kb;
-      auto prefetch = [&](long long seq) {
-        const long long tile_iter = seq / num_kb;
-        const int kb = static_cast<int>(seq - tile_iter * num_kb);
-        const long long R0 = ((unit + tile_iter * num_units) * NCTA + rank) * PM;
-        if (R0 >= p.m_total) return;
-        const long long img = R0 / p.hw;
-        const int cell = static_cast<int>(R0 - img * p.hw);
-        asm volatile("cp.async.bulk.prefetch.tensor.3d.L2.global.tile [%0, {%1, %2, %3}];" ::"l"(
-                         reinterpret_cast<uint64_t>(&tmap_x)),
-                     "r"(cell), "r"(kb * PK), "r"(static_cast<int32_t>(img))
-                     : "memory");
-      };
-      for (long long s2 = 0; s2 < kPrefetchDepth && s2 < total_seq; ++s2) prefetch(s2);
-      for (long long seq = 0; seq + kPrefetchDepth < total_seq; ++seq) {
-        mbar_wait(&a_empty[seq % A_STAGES], static_cast<uint32_t>(((seq / A_STAGES) & 1) ^ 1));
-        prefetch(seq + kPrefetchDepth);
       }
     }
   } else if (warp >= kTransformWarp0) {
@@ -399,9 +358,7 @@ l2norm_project_kernel(const __grid_constant__ CUtensorMap tmap_whi, const __grid
         }
         fence_proxy_async_smem();  // generic-proxy writes -> visible to the tensor core's async proxy
         __syncwarp();
-        if (lane == 0) {
-          if (NCTA == 2) mbar_arrive_leader(&a_full[stage]); else mbar_arrive(&a_full[stage]);
-        }
+        if (lane == 0) mbar_arrive_leader(&a_full[stage]);
         if (++stage == static_cast<uint32_t>(A_STAGES)) { stage = 0; phase ^= 1; }
         if (++pr_kb == num_kb) {
           // last k-block of the tile: publish the row's sum of squares over this warp's two quarters
@@ -431,7 +388,7 @@ l2norm_project_kernel(const __grid_constant__ CUtensorMap tmap_whi, const __grid
     bool ld_valid = false;
     auto seek_tile = [&](long long tile_iter) {
       const long long tile = unit + tile_iter * num_units;
-      const long long R = (tile * NCTA + rank) * PM + m;
+      const long long R = (tile * 2 + rank) * PM + m;
       ld_valid = tile_iter < my_tiles && R < p.m_total;
       const long long img = ld_valid ? R / p.hw : 0;  // once per tile
       const long long cell = ld_valid ? R - img * p.hw : 0;
@@ -445,23 +402,11 @@ l2norm_project_kernel(const __grid_constant__ CUtensorMap tmap_whi, const __grid
     };
     auto load_block = [&](float (&x)[32]) {
       const int f0 = ld.kb * PK + half * 32;
-      if (HW > 0) {
-        // E % 64 == 0: every feature of the block exists; channel stride is a compile-time constant
-        const float* src = ld_base + static_cast<long long>(f0) * HW;
-        if (ld_valid) {
+      const float* src = ld_base + static_cast<long long>(f0) * p.hw;
 #pragma unroll
-          for (int i = 0; i < 32; ++i) x[i] = ld_f32(src + i * HW);
-        } else {
-#pragma unroll
-          for (int i = 0; i < 32; ++i) x[i] = 0.f;
-        }
-      } else {
-        const float* src = ld_base + static_cast<long long>(f0) * p.hw;
-#pragma unroll
-        for (int i = 0; i < 32; ++i) {
-          x[i] = (ld_valid && f0 + i < p.E) ? ld_f32(src) : 0.f;
-          src += p.hw;
-        }
+      for (int i = 0; i < 32; ++i) {
+        x[i] = (ld_valid && f0 + i < p.E) ? ld_f32(src) : 0.f;
+        src += p.hw;
       }
       if (++ld.kb == num_kb) { ld.kb = 0; seek_tile(++ld.tile_iter); }
     };
@@ -496,9 +441,7 @@ l2norm_project_kernel(const __grid_constant__ CUtensorMap tmap_whi, const __grid
       }
       fence_proxy_async_smem();  // generic-proxy writes -> visible to the tensor core's async proxy
       __syncwarp();
-      if (lane == 0) {
-        if (NCTA == 2) mbar_arrive_leader(&a_full[stage]); else mbar_arrive(&a_full[stage]);
-      }
+      if (lane == 0) mbar_arrive_leader(&a_full[stage]);
       if (++stage == static_cast<uint32_t>(A_STAGES)) { stage = 0; phase ^= 1; }
       if (++pr_kb == num_kb) {
         // last k-block of the tile: publish this thread's share of the row's sum of squares
@@ -529,7 +472,7 @@ l2norm_project_kernel(const __grid_constant__ CUtensorMap tmap_whi, const __grid
     uint32_t acc = 0, acc_phase = 0;
     const bool vec_ok = (p.k & 3) == 0 && (reinterpret_cast<uintptr_t>(p.out) & 15u) == 0;
     for (long long tile = unit; tile < p.tiles; tile += num_units) {
-      const long long R = (tile * NCTA + rank) * PM + row;
+      const long long R = (tile * 2 + rank) * PM + row;
       mbar_wait(&ss_full[acc], acc_phase);
       float rn = 1.0f;
       if (p.normalize) {
@@ -564,268 +507,8 @@ l2norm_project_kernel(const __grid_constant__ CUtensorMap tmap_whi, const __grid
       }
       tc_fence_before();
       __syncwarp();
-      if (lane == 0) {
-        if (NCTA == 2) mbar_arrive_leader(&tmem_empty[acc]); else mbar_arrive(&tmem_empty[acc]);
-      }
+      if (lane == 0) mbar_arrive_leader(&tmem_empty[acc]);
       if (++acc == P_ACC_STAGES) { acc = 0; acc_phase ^= 1; }
-    }
-  }
-
-  tc_fence_before();
-  if (NCTA == 2) cluster_sync_all(); else __syncthreads();
-  if (warp == 2) {
-    tc_fence_after();
-    if (NCTA == 2) tmem_dealloc_pair(tmem_base, 512); else tmem_dealloc(tmem_base, 512);
-  }
-}
-
-// ------------------------------------------------------------------------------------------
-// K3t: the per-cell kernel with the A operand in TENSOR MEMORY (CTA pairs only).
-// The converted bf16 hi/lo operand never touches shared memory: the transform warps write it with
-// tcgen05.st straight into TMEM columns next to the accumulator and the MMAs take A from there
-// (tcgen05.mma ... [d], [a_tmem], b_desc).  Per k-block that removes 32 KB of shared-memory stores,
-// 48 KB of operand reads and the generic->async proxy fence from the one 128 B/clk shared-memory
-// port, and frees 64 KB for a deeper raw ring (4 x 32 KB in flight per SM).
-//   TMEM columns: [0, 256) accumulator (single stage: the epilogue of tile t runs before the MMAs of
-//   tile t + 1; the transform of t + 1 overlaps it), [256, 256 + 64 s) A stages (hi 32 | lo 32 cols).
-//   warp 0 weight TMA (half of the rows per CTA), warp 1 MMA issuer (leader), warp 2 TMEM alloc,
-//   warp 3 raw-tile TMA, warps 4-7 epilogue, warps 8-23 transform: warp tw owns TMEM lane quarter
-//   tw % 4 (rows = cells 32 (tw % 4) + lane) and features 16 (tw / 4) .. + 15 of every k-block.
-// ------------------------------------------------------------------------------------------
-struct ProjTSmem {
-  static constexpr int A_STAGES = 3, W_STAGES = 2, RAW_STAGES = 4;
-  static constexpr uint32_t W_PART_BYTES = (kMaxComponents / 2) * PK * 2;  // 16 KB
-  static constexpr uint32_t W_STAGE_BYTES = 2 * W_PART_BYTES;              // hi + lo
-  static constexpr uint32_t RAW_STAGE_BYTES = PM * PK * 4;                 // 32 KB
-  static constexpr uint32_t kWOff = 0;
-  static constexpr uint32_t kRawOff = kWOff + W_STAGES * W_STAGE_BYTES;
-  static constexpr uint32_t kSsOff = kRawOff + RAW_STAGES * RAW_STAGE_BYTES;  // [2][4 feature groups][128 rows]
-  static constexpr uint32_t kBarOff = kSsOff + 2 * 4 * PM * 4;
-  static constexpr uint32_t kNumBars = 2 * A_STAGES + 2 * W_STAGES + 2 * RAW_STAGES + 2 + 4;
-  static constexpr uint32_t kTmemPtrOff = kBarOff + kNumBars * 8;
-  static constexpr uint32_t kTotal = kTmemPtrOff + 16;
-  static constexpr uint32_t kDynamicBytes = kTotal + 1024;
-  static constexpr uint32_t kAColumn0 = kMaxComponents;  // first A column in TMEM
-};
-constexpr int kProjTThreads = (kTransformWarp0 + 16) * 32;
-
-__global__ void __launch_bounds__(kProjTThreads, 1)
-l2norm_project_tmem_kernel(const __grid_constant__ CUtensorMap tmap_whi, const __grid_constant__ CUtensorMap tmap_wlo,
-                           const __grid_constant__ CUtensorMap tmap_x, const ProjParams p) {
-  using L = ProjTSmem;
-  constexpr int A_STAGES = L::A_STAGES, W_STAGES = L::W_STAGES, RAW_STAGES = L::RAW_STAGES;
-  const uint32_t rank = cluster_ctarank();
-  const long long unit = blockIdx.x / 2, num_units = gridDim.x / 2;
-  extern __shared__ uint8_t smem_raw[];
-  uint8_t* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
-  uint64_t* bars = reinterpret_cast<uint64_t*>(smem + L::kBarOff);
-  uint64_t* a_full = bars;                       // [A]   16 transform warps x 2 CTAs (on the leader)
-  uint64_t* a_empty = a_full + A_STAGES;         // [A]   tcgen05.commit (both CTAs)
-  uint64_t* w_full = a_empty + A_STAGES;         // [W]   TMA of both CTAs (on the leader)
-  uint64_t* w_empty = w_full + W_STAGES;         // [W]   tcgen05.commit (both CTAs)
-  uint64_t* raw_full = w_empty + W_STAGES;       // [RAW] TMA
-  uint64_t* raw_empty = raw_full + RAW_STAGES;   // [RAW] 16 transform warps
-  uint64_t* tmem_full = raw_empty + RAW_STAGES;  // accumulator complete (both CTAs)
-  uint64_t* tmem_empty = tmem_full + 1;          // 4 epilogue warps x 2 CTAs (on the leader)
-  uint64_t* ss_full = tmem_empty + 1;            // [2]   16 transform warps
-  uint64_t* ss_empty = ss_full + 2;              // [2]   4 epilogue warps
-  uint32_t* tmem_ptr = reinterpret_cast<uint32_t*>(smem + L::kTmemPtrOff);
-  float* ss_s = reinterpret_cast<float*>(smem + L::kSsOff);
-
-  const int warp = threadIdx.x >> 5;
-  const int lane = threadIdx.x & 31;
-  const int num_kb = (p.E + PK - 1) / PK;
-
-  if (warp == 0 && lane == 0) {
-    prefetch_tmap(&tmap_whi);
-    prefetch_tmap(&tmap_wlo);
-    prefetch_tmap(&tmap_x);
-  }
-  if (warp == 1 && lane == 0) {
-    for (int i = 0; i < A_STAGES; ++i) { mbar_init(&a_full[i], 16 * 2); mbar_init(&a_empty[i], 1); }
-    for (int i = 0; i < W_STAGES; ++i) { mbar_init(&w_full[i], 2); mbar_init(&w_empty[i], 1); }
-    for (int i = 0; i < RAW_STAGES; ++i) { mbar_init(&raw_full[i], 1); mbar_init(&raw_empty[i], 16); }
-    mbar_init(tmem_full, 1);
-    mbar_init(tmem_empty, 4 * 2);
-    for (int i = 0; i < 2; ++i) { mbar_init(&ss_full[i], 16); mbar_init(&ss_empty[i], 4); }
-    fence_mbar_init();
-  }
-  if (warp == 2) { tmem_alloc_pair(tmem_ptr, 512); tmem_relinquish_pair(); }
-  tc_fence_before();
-  cluster_sync_all();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_ptr;
-  const int w_rows = p.k_pad / 2;
-  const uint32_t w_part_bytes = static_cast<uint32_t>(w_rows) * PK * 2;
-  const long long my_tiles = (p.tiles - unit + num_units - 1) / num_units;
-  const long long total_seq = my_tiles * num_kb;
-
-  if (warp == 0) {
-    // ===================== weight TMA producer =====================
-    if (lane == 0) {
-      uint32_t stage = 0, phase = 0;
-      const int32_t row0 = static_cast<int32_t>(rank) * w_rows;
-      for (long long seq = 0; seq < total_seq; ++seq) {
-        const int kb = static_cast<int>(seq % num_kb);
-        mbar_wait(&w_empty[stage], phase ^ 1);
-        uint8_t* dst = smem + L::kWOff + stage * L::W_STAGE_BYTES;
-        mbar_arrive_expect_tx_leader(&w_full[stage], 2 * w_part_bytes);
-        tma_load_2d_pair(dst, &tmap_whi, &w_full[stage], kb * PK, row0, kEvictLast);
-        tma_load_2d_pair(dst + L::W_PART_BYTES, &tmap_wlo, &w_full[stage], kb * PK, row0, kEvictLast);
-        if (++stage == W_STAGES) { stage = 0; phase ^= 1; }
-      }
-    }
-  } else if (warp == 1) {
-    // ===================== MMA issuer (leader CTA) =====================
-    if (lane == 0 && rank == 0) {
-      const uint32_t idesc = make_idesc(/*bf16*/ 1, PM * 2, static_cast<uint32_t>(p.k_pad));
-      uint32_t as = 0, aph = 0, ws = 0, wph = 0, tph = 0;
-      for (long long tile = 0; tile < my_tiles; ++tile) {
-        mbar_wait(tmem_empty, tph ^ 1);  // the epilogues of both CTAs drained the accumulator
-        tc_fence_after();
-        for (int kb = 0; kb < num_kb; ++kb) {
-          mbar_wait(&w_full[ws], wph);
-          mbar_wait(&a_full[as], aph);
-          tc_fence_after();
-          const uint32_t a_hi = tmem_base + L::kAColumn0 + as * 64;
-          const uint32_t a_lo = a_hi + 32;
-          const uint32_t w_hi = smem_u32(smem + L::kWOff + ws * L::W_STAGE_BYTES);
-          const uint32_t w_lo = w_hi + L::W_PART_BYTES;
-#pragma unroll
-          for (int k = 0; k < PK / P_UMMA_K; ++k) {
-            const uint64_t dwh = make_kmajor_sw128_desc(w_hi + k * P_UMMA_K * 2);
-            const uint64_t dwl = make_kmajor_sw128_desc(w_lo + k * P_UMMA_K * 2);
-            tc_mma_f16_pair_ts(tmem_base, a_hi + k * 8, dwh, idesc, (kb | k) != 0);
-            tc_mma_f16_pair_ts(tmem_base, a_lo + k * 8, dwh, idesc, 1);
-            tc_mma_f16_pair_ts(tmem_base, a_hi + k * 8, dwl, idesc, 1);
-          }
-          tc_commit_pair(&a_empty[as]);
-          tc_commit_pair(&w_empty[ws]);
-          if (++as == A_STAGES) { as = 0; aph ^= 1; }
-          if (++ws == W_STAGES) { ws = 0; wph ^= 1; }
-        }
-        tc_commit_pair(tmem_full);
-        tph ^= 1;
-      }
-    }
-  } else if (warp == 3) {
-    // ===================== raw-tile TMA producer =====================
-    if (lane == 0) {
-      uint32_t rs = 0, rph = 0;
-      for (long long tile = unit; tile < p.tiles; tile += num_units) {
-        const long long R0 = (tile * 2 + rank) * PM;
-        const long long img = R0 / p.hw;
-        const int cell = static_cast<int>(R0 - img * p.hw);
-        for (int kb = 0; kb < num_kb; ++kb) {
-          mbar_wait(&raw_empty[rs], rph ^ 1);
-          mbar_arrive_expect_tx(&raw_full[rs], L::RAW_STAGE_BYTES);
-          tma_load_3d(smem + L::kRawOff + rs * L::RAW_STAGE_BYTES, &tmap_x, &raw_full[rs], cell, kb * PK,
-                      static_cast<int32_t>(img), kEvictFirst);
-          if (++rs == RAW_STAGES) { rs = 0; rph ^= 1; }
-        }
-      }
-    }
-  } else if (warp >= kTransformWarp0) {
-    // ===================== transform: raw fp32 (smem) -> bf16 hi/lo (TMEM) =====================
-    const int tw = warp - kTransformWarp0;
-    const int lq = tw & 3;            // == warp % 4: the TMEM lane quarter this warp may access
-    const int fg = tw >> 2;           // feature group: 16 features of the k-block
-    const int m = lq * 32 + lane;     // row (cell) inside the tile
-    const int cb = min(p.hw, PM);     // raw box layout: [image][feature][cell], cb cells per image row
-    const int m_off = (m / cb) * (PK * cb) + (m % cb) + fg * 16 * cb;
-    const uint32_t t_row = tmem_base + (static_cast<uint32_t>(lq * 32) << 16) + L::kAColumn0 + fg * 8;
-    float ss = 0.f;
-    uint32_t as = 0, aph = 0, rs = 0, rph = 0, sst = 0, ssph = 0;
-    int pr_kb = 0;
-    for (long long seq = 0; seq < total_seq; ++seq) {
-      mbar_wait(&raw_full[rs], rph);
-      const float* raw = reinterpret_cast<const float*>(smem + L::kRawOff + rs * L::RAW_STAGE_BYTES) + m_off;
-      float x[16];
-#pragma unroll
-      for (int i = 0; i < 16; ++i) x[i] = raw[i * cb];
-      __syncwarp();
-      if (lane == 0) mbar_arrive(&raw_empty[rs]);  // release: this warp's reads of the stage are done
-      if (++rs == RAW_STAGES) { rs = 0; rph ^= 1; }
-      uint32_t hi[8], lo[8];
-#pragma unroll
-      for (int i = 0; i < 8; ++i) {
-        const float a = x[2 * i], b = x[2 * i + 1];
-        ss = fmaf(a, a, ss);
-        ss = fmaf(b, b, ss);
-        // hi = x truncated to bf16 (a mask); lo = RN_bf16(x - hi): |x - hi - lo| <= 2^-16 |x|
-        const uint32_t ab = __float_as_uint(a), bb = __float_as_uint(b);
-        hi[i] = __byte_perm(ab, bb, 0x7632);
-        const float la = a - __uint_as_float(ab & 0xFFFF0000u);
-        const float lb = b - __uint_as_float(bb & 0xFFFF0000u);
-        const __nv_bfloat162 l2 = __floats2bfloat162_rn(la, lb);
-        lo[i] = *reinterpret_cast<const uint32_t*>(&l2);
-      }
-      mbar_wait(&a_empty[as], aph ^ 1);
-      tc_fence_after();
-      tmem_st_32x8(t_row + as * 64, hi);
-      tmem_st_32x8(t_row + as * 64 + 32, lo);
-      tc_wait_st();
-      tc_fence_before();
-      __syncwarp();
-      if (lane == 0) mbar_arrive_leader(&a_full[as]);
-      if (++as == A_STAGES) { as = 0; aph ^= 1; }
-      if (++pr_kb == num_kb) {
-        // last k-block of the tile: publish this warp's share of the rows' sums of squares
-        pr_kb = 0;
-        mbar_wait(&ss_empty[sst], ssph ^ 1);
-        ss_s[(sst * 4 + fg) * PM + m] = ss;
-        __syncwarp();
-        if (lane == 0) mbar_arrive(&ss_full[sst]);
-        ss = 0.f;
-        if (++sst == 2) { sst = 0; ssph ^= 1; }
-      }
-    }
-  } else if (warp >= 4 && warp < 8) {
-    // ===================== epilogue =====================
-    const int ew = warp - 4;  // == warp % 4: TMEM lane quarter
-    const int row = ew * 32 + lane;
-    uint32_t sst = 0, ssph = 0, tph = 0;
-    const bool vec_ok = (p.k & 3) == 0 && (reinterpret_cast<uintptr_t>(p.out) & 15u) == 0;
-    for (long long tile = unit; tile < p.tiles; tile += num_units) {
-      const long long R = (tile * 2 + rank) * PM + row;
-      mbar_wait(&ss_full[sst], ssph);
-      float rn = 1.0f;
-      if (p.normalize) {
-        const float* sp = ss_s + sst * 4 * PM + row;
-        const float ssum = (sp[0] + sp[PM]) + (sp[2 * PM] + sp[3 * PM]);
-        rn = 1.0f / fmaxf(sqrtf(ssum), 1e-12f);
-      }
-      __syncwarp();
-      if (lane == 0) mbar_arrive(&ss_empty[sst]);
-      if (++sst == 2) { sst = 0; ssph ^= 1; }
-      mbar_wait(tmem_full, tph);
-      tph ^= 1;
-      tc_fence_after();
-      const uint32_t taddr = tmem_base + (static_cast<uint32_t>(ew * 32) << 16);
-      float* orow = p.out + R * p.k;
-#pragma unroll 1
-      for (int c0 = 0; c0 < p.k_pad; c0 += 16) {
-        uint32_t r[16];
-        tmem_ld_32x16(taddr + c0, r);
-        tc_wait_ld();
-        if (R < p.m_total) {
-          float v[16];
-#pragma unroll
-          for (int j = 0; j < 16; ++j) v[j] = fmaf(__uint_as_float(r[j]), rn, __ldg(p.bias + c0 + j));
-          if (vec_ok && c0 + 16 <= p.k) {
-#pragma unroll
-            for (int j = 0; j < 4; ++j)
-              *reinterpret_cast<float4*>(orow + c0 + 4 * j) = make_float4(v[4 * j], v[4 * j + 1], v[4 * j + 2], v[4 * j + 3]);
-          } else {
-#pragma unroll
-            for (int j = 0; j < 16; ++j)
-              if (c0 + j < p.k) orow[c0 + j] = v[j];
-          }
-        }
-      }
-      tc_fence_before();
-      __syncwarp();
-      if (lane == 0) mbar_arrive_leader(tmem_empty);
     }
   }
 
@@ -838,9 +521,11 @@ l2norm_project_tmem_kernel(const __grid_constant__ CUtensorMap tmap_whi, const _
 }
 
 // ------------------------------------------------------------------------------------------
-// K3d: the per-cell kernel with NO raw staging (CTA pairs; the default for map shapes the TMA boxes of
-// the staged kernel cannot express, e.g. 7 x 10 cells; ISX_PROJECT_MODE=direct forces it).
-// Measured at config 3b it runs at the staged kernel's speed (1.79 against 1.78 ms): with the raw ring
+// K3d: the per-cell kernel with NO raw staging (CTA pairs).  It takes the maps the TMA boxes of the
+// staged kernel cannot express (e.g. 7 x 10 cells, or a map pointer off a 16-byte boundary) when its
+// epilogue can: k % 4 == 0 and E % 16 == 0 (launch_project has the rules).
+// Measured at config 3b, which a mode switch (since removed) sent here with an L2 prefetcher in warp 3
+// (also removed), it runs at the staged kernel's speed (1.79 against 1.78 ms): with the raw ring
 // and the A tiles gone from shared memory the port carries 128 KB per k-block instead of 272 KB and
 // nothing got faster, which is what shows that the three tensor passes (1.15 PFLOP/s issued next to
 // 3.6 TB/s of HBM traffic, at the 1 kW cap: 2.06 TFLOP take 1.49 ms at the sustained cuBLAS rate) — not
@@ -851,17 +536,18 @@ l2norm_project_tmem_kernel(const __grid_constant__ CUtensorMap tmap_whi, const _
 //     (two register buffers: 32-64 KB of loads in flight per SM), accumulate the sums of squares, split to bf16 hi/lo and
 //     write the A operand with tcgen05.st into TENSOR MEMORY (4 stages x 64 columns next to the
 //     256-column accumulator); the MMAs take A from there (TS form);
-//   * warp 3 asks the TMA unit to pull the boxes of the map into L2 a few k-blocks ahead;
 //   * the epilogue scales by 1/||x||, adds the bias and hands 128-row x 32-column boxes (128-byte rows,
 //     128B swizzle) to TMA stores: every global write is a full line instead of 16-byte pieces of
 //     1 KB-strided rows.
 // Per k-block a CTA's shared-memory port now moves 32 KB of weights in and 96 KB of weight reads out
 // (its half and the peer's) = 1000 cycles at 128 B/clk, against 1536 tensor cycles: the kernel is bound
 // by the three tensor passes that fp32-class accuracy costs, no longer by shared memory.
-//   warp 0 weight TMA, warp 1 MMA issuer (leader), warp 2 TMEM alloc, warp 3 L2 prefetch,
+//   warp 0 weight TMA, warp 1 MMA issuer (leader), warp 2 TMEM alloc, warp 3 idle,
 //   warps 4-7 epilogue, warps 8-23 transform: warp tw owns TMEM lane quarter tw % 4
 //   (cells 32 (tw % 4) + lane of the tile) and features 16 (tw / 4) .. + 15 of every k-block.
 // ------------------------------------------------------------------------------------------
+constexpr int kProjDThreads = (kTransformWarp0 + 16) * 32;
+
 struct ProjDSmem {
   static constexpr int A_STAGES = 4, W_STAGES = 2, OUT_BUFS = 8;  // one staging buffer per 32-column box of a tile
   static constexpr uint32_t W_PART_BYTES = (kMaxComponents / 2) * PK * 2;  // 16 KB
@@ -878,10 +564,9 @@ struct ProjDSmem {
   static constexpr uint32_t kAColumn0 = kMaxComponents;  // first A column in TMEM
 };
 
-__global__ void __launch_bounds__(kProjTThreads, 1)
+__global__ void __launch_bounds__(kProjDThreads, 1)
 l2norm_project_direct_kernel(const __grid_constant__ CUtensorMap tmap_whi, const __grid_constant__ CUtensorMap tmap_wlo,
-                             const __grid_constant__ CUtensorMap tmap_x, const __grid_constant__ CUtensorMap tmap_out,
-                             const ProjParams p) {
+                             const __grid_constant__ CUtensorMap tmap_out, const ProjParams p) {
   using L = ProjDSmem;
   constexpr int A_STAGES = L::A_STAGES, W_STAGES = L::W_STAGES;
   const uint32_t rank = cluster_ctarank();
@@ -908,7 +593,6 @@ l2norm_project_direct_kernel(const __grid_constant__ CUtensorMap tmap_whi, const
     prefetch_tmap(&tmap_whi);
     prefetch_tmap(&tmap_wlo);
     prefetch_tmap(&tmap_out);
-    if (p.prefetch) prefetch_tmap(&tmap_x);
   }
   if (warp == 1 && lane == 0) {
     for (int i = 0; i < A_STAGES; ++i) { mbar_init(&a_full[i], 16 * 2); mbar_init(&a_empty[i], 1); }
@@ -975,30 +659,6 @@ l2norm_project_direct_kernel(const __grid_constant__ CUtensorMap tmap_whi, const
         }
         tc_commit_pair(tmem_full);
         tph ^= 1;
-      }
-    }
-  } else if (warp == 3) {
-    // ===================== L2 prefetcher =====================
-    // boxes of the map (128 cells x 64 features) are requested kPrefetchDepth k-blocks ahead of the
-    // transform warps, paced by the a_empty barriers, so their loads find the lines in L2
-    if (lane == 0 && p.prefetch) {
-      constexpr int kPrefetchDepth = 8;
-      auto prefetch = [&](long long seq) {
-        const long long tile_iter = seq / num_kb;
-        const int kb = static_cast<int>(seq - tile_iter * num_kb);
-        const long long R0 = ((unit + tile_iter * num_units) * 2 + rank) * PM;
-        if (R0 >= p.m_total) return;
-        const long long img = R0 / p.hw;
-        const int cell = static_cast<int>(R0 - img * p.hw);
-        asm volatile("cp.async.bulk.prefetch.tensor.3d.L2.global.tile [%0, {%1, %2, %3}];" ::"l"(
-                         reinterpret_cast<uint64_t>(&tmap_x)),
-                     "r"(cell), "r"(kb * PK), "r"(static_cast<int32_t>(img))
-                     : "memory");
-      };
-      for (long long s2 = 0; s2 < kPrefetchDepth && s2 < total_seq; ++s2) prefetch(s2);
-      for (long long seq = 0; seq + kPrefetchDepth < total_seq; ++seq) {
-        mbar_wait(&a_empty[seq % A_STAGES], static_cast<uint32_t>(((seq / A_STAGES) & 1) ^ 1));
-        prefetch(seq + kPrefetchDepth);
       }
     }
   } else if (warp >= kTransformWarp0) {
@@ -1397,167 +1057,103 @@ l2norm_pool_tma_kernel(const __grid_constant__ CUtensorMap tmap, int B, int E, i
   }
 }
 
-int project_ncta() {
-  static const int forced = [] {
-    const char* e = getenv("ISX_PROJECT_CTA_PAIR");
-    return (e && (e[0] == '0' || e[0] == '1')) ? (e[0] - '0') : -1;
-  }();
-  return forced == 0 ? 1 : 2;
-}
-
-template <int HW, int NCTA>
-int launch_project_kernel(const CUtensorMap& twh, const CUtensorMap& twl, const CUtensorMap& tx, const ProjParams& p,
-                          int grid, cudaStream_t stream) {
-  auto kern = l2norm_project_kernel<HW, NCTA>;
-  const int smem = static_cast<int>(ProjSmem<NCTA, (HW < 0)>::kDynamicBytes);
-  ISX_CHECK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+// Launches a per-cell projection kernel on CTA pairs (clusters of two CTAs).
+template <typename... Params, typename... Args>
+int launch_pair(void (*kern)(Params...), int threads, uint32_t smem, int grid, cudaStream_t stream, const Args&... args) {
+  ISX_CHECK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = dim3(static_cast<unsigned>(grid));
-  cfg.blockDim = dim3(proj_threads(HW < 0));
+  cfg.blockDim = dim3(static_cast<unsigned>(threads));
   cfg.dynamicSmemBytes = static_cast<size_t>(smem);
   cfg.stream = stream;
   cudaLaunchAttribute attr[1];
   attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = NCTA;
+  attr[0].val.clusterDim.x = 2;
   attr[0].val.clusterDim.y = 1;
   attr[0].val.clusterDim.z = 1;
   cfg.attrs = attr;
   cfg.numAttrs = 1;
-  ISX_CHECK_CUDA(cudaLaunchKernelEx(&cfg, kern, twh, twl, tx, p));
+  ISX_CHECK_CUDA(cudaLaunchKernelEx(&cfg, kern, args...));
   return ISX_OK;
 }
 
-template <int NCTA>
-int launch_project_n(const float* fmap, long long m_total, int E, int hw, int k, int normalize, int fast,
-                     const void* packed, float* out, cudaStream_t stream) {
+// Projects m_total cells of an NCHW map (hw cells per image; hw == 1 for an n x E matrix).  The kernel
+// follows from the input's shape and alignment alone, by the first rule that fits.
+int launch_project(const float* fmap, long long m_total, int E, int hw, int k, int normalize, int fast,
+                   const void* packed, float* out, cudaStream_t stream) {
   const PackedLayout l = packed_layout(E, k);
   const uint8_t* pk = static_cast<const uint8_t*>(packed);
-  CUtensorMap twh, twl;
+  CUtensorMap twh, twl;  // each CTA of a pair stages half of the weight rows
   int rc = encode_tmap_2d(&twh, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, pk + l.hi_off, static_cast<uint64_t>(l.k_pad),
                           static_cast<uint64_t>(l.f_pad), static_cast<uint64_t>(l.f_pad) * 2,
-                          static_cast<uint32_t>(l.k_pad / NCTA), PK, CU_TENSOR_MAP_SWIZZLE_128B);
+                          static_cast<uint32_t>(l.k_pad / 2), PK, CU_TENSOR_MAP_SWIZZLE_128B);
   if (rc != ISX_OK) return rc;
   rc = encode_tmap_2d(&twl, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, pk + l.lo_off, static_cast<uint64_t>(l.k_pad),
                       static_cast<uint64_t>(l.f_pad), static_cast<uint64_t>(l.f_pad) * 2,
-                      static_cast<uint32_t>(l.k_pad / NCTA), PK, CU_TENSOR_MAP_SWIZZLE_128B);
+                      static_cast<uint32_t>(l.k_pad / 2), PK, CU_TENSOR_MAP_SWIZZLE_128B);
   if (rc != ISX_OK) return rc;
   int sms = 148;
   rc = device_sm_count(&sms);
   if (rc != ISX_OK) return rc;
   ProjParams p;
   p.fmap = fmap; p.m_total = m_total; p.E = E; p.hw = hw; p.k = k; p.k_pad = l.k_pad;
+  p.fast = 0;
+  p.rowmajor = 0;
   p.normalize = normalize;
-  p.tiles = (m_total + PM * NCTA - 1) / (PM * NCTA);  // tiles of 128 cells per CTA (256 per pair)
+  p.tiles = (m_total + 2 * PM - 1) / (2 * PM);  // tiles of 128 cells per CTA (256 per pair)
   p.bias = reinterpret_cast<const float*>(pk + l.bias_off);
   p.out = out;
-  const int grid = static_cast<int>(std::min<long long>(sms / NCTA, p.tiles)) * NCTA;
-  // L2 prefetch boxes: a tile of 128 cells is half/quarter/... of one image (hw % 128 == 0) or a
-  // whole number of images (128 % hw == 0); other shapes run without the prefetcher
-  CUtensorMap tx = twh;
-  p.prefetch = 0;
-  p.rowmajor = 0;
-  p.fast = 0;
-  // single fp16 pass: only the staged pair kernel implements it; tmap for the fp16 weight copy
-  CUtensorMap twf = twh;
-  if (fast && NCTA == 2) {
-    rc = encode_tmap_2d(&twf, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, pk + l.h_off, static_cast<uint64_t>(l.k_pad),
-                        static_cast<uint64_t>(l.f_pad), static_cast<uint64_t>(l.f_pad) * 2,
-                        static_cast<uint32_t>(l.k_pad / NCTA), PK, CU_TENSOR_MAP_SWIZZLE_128B);
-    if (rc != ISX_OK) return rc;
-  }
-  if constexpr (NCTA == 2) {
-    // n x E row-major input (PCA.transform's flat vectors, the pooled rows): 2-D map, swizzled boxes
-    if (hw == 1 && E % 4 == 0 && (reinterpret_cast<uintptr_t>(fmap) & 15u) == 0 && m_total < (1ll << 31)) {
+  const int grid = static_cast<int>(std::min<long long>(sms / 2, p.tiles)) * 2;
+  const bool map_aligned = (reinterpret_cast<uintptr_t>(fmap) & 15u) == 0;
+
+  // 1. n x E row-major input (PCA.transform's flat vectors, the pooled rows): the staged kernel on a
+  //    2-D map with 128B-swizzled boxes of 128 rows x 32 features.
+  const bool rowmajor = hw == 1 && E % 4 == 0 && map_aligned && m_total < (1ll << 31);
+  // 2. Rule 1 needs one cell per image.  A map of several cells per image takes the staged kernel on
+  //    a 3-D map over (cell, feature, image) when its strides are whole 16-byte units and a tile of 128
+  //    cells is a fraction of one image (hw % 128 == 0) or a whole number of images (128 % hw == 0).
+  const bool boxes = hw % 4 == 0 && map_aligned && (hw % PM == 0 || PM % hw == 0);
+  if (rowmajor || boxes) {
+    CUtensorMap tx;
+    if (rowmajor) {
       rc = encode_tmap_2d(&tx, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, fmap, static_cast<uint64_t>(m_total),
                           static_cast<uint64_t>(E), static_cast<uint64_t>(E) * 4, PM, 32, CU_TENSOR_MAP_SWIZZLE_128B);
-      if (rc != ISX_OK) return rc;
-      p.rowmajor = 1;
-      p.fast = fast;
-      return launch_project_kernel<-1, 2>(fast ? twf : twh, twl, tx, p, grid, stream);
+    } else {
+      const uint32_t cells_box = static_cast<uint32_t>(std::min(hw, PM));
+      const uint32_t imgs_box = static_cast<uint32_t>(PM / static_cast<int>(cells_box));
+      rc = encode_tmap_3d(&tx, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, fmap, static_cast<uint64_t>(hw), static_cast<uint64_t>(E),
+                          static_cast<uint64_t>(m_total / hw), static_cast<uint64_t>(hw) * 4,
+                          static_cast<uint64_t>(E) * hw * 4, cells_box, PK, imgs_box, CU_TENSOR_MAP_SWIZZLE_NONE);
     }
-  }
-  const long long images = m_total / hw;
-  if (hw % 4 == 0 && (reinterpret_cast<uintptr_t>(fmap) & 15u) == 0 && (hw % PM == 0 || PM % hw == 0) && images >= 1) {
-    const uint32_t cells_box = static_cast<uint32_t>(std::min(hw, PM));
-    const uint32_t imgs_box = static_cast<uint32_t>(PM / static_cast<int>(cells_box));
-    rc = encode_tmap_3d(&tx, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, fmap, static_cast<uint64_t>(hw), static_cast<uint64_t>(E),
-                        static_cast<uint64_t>(images), static_cast<uint64_t>(hw) * 4, static_cast<uint64_t>(E) * hw * 4,
-                        cells_box, PK, imgs_box, CU_TENSOR_MAP_SWIZZLE_NONE);
     if (rc != ISX_OK) return rc;
-    p.prefetch = 1;
-  }
-  if constexpr (NCTA == 2) {
-    // ISX_PROJECT_MODE = staged (default) | tmem | reg selects the per-cell kernel (A/B measurements,
-    // tests): staged = bf16 operand tiles in shared memory, tmem = A operand in tensor memory,
-    // reg = register-path loads without raw staging.  Read per call (a getenv, not on any hot loop).
-    const char* mode_env = getenv("ISX_PROJECT_MODE");
-    // default: the staged kernel where the map's shape allows TMA boxes, else K3d (any shape)
-    const int mode = (mode_env && mode_env[0] == 't') ? 0 : (mode_env && mode_env[0] == 'r') ? 2
-                     : (mode_env && mode_env[0] == 'd') ? 3 : (mode_env && mode_env[0] == 's') ? 1 : (p.prefetch ? 1 : 3);
-    if (p.prefetch && fast) {
-      p.fast = 1;
-      return launch_project_kernel<-1, 2>(twf, twl, tx, p, grid, stream);
-    }
-    // K3d: any map shape (the loads are per-thread); the TMA-store epilogue needs 16-byte output rows
-    if (mode == 3 && k % 4 == 0 && E % 16 == 0 && (reinterpret_cast<uintptr_t>(out) & 15u) == 0 && m_total < (1ll << 31)) {
-      CUtensorMap tout;
-      rc = encode_tmap_2d(&tout, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, out, static_cast<uint64_t>(m_total),
-                          static_cast<uint64_t>(k), static_cast<uint64_t>(k) * 4, PM, 32, CU_TENSOR_MAP_SWIZZLE_128B);
+    if (fast) {
+      // single fp16 pass: tmap_whi describes the fp16 copy of the weights
+      rc = encode_tmap_2d(&twh, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, pk + l.h_off, static_cast<uint64_t>(l.k_pad),
+                          static_cast<uint64_t>(l.f_pad), static_cast<uint64_t>(l.f_pad) * 2,
+                          static_cast<uint32_t>(l.k_pad / 2), PK, CU_TENSOR_MAP_SWIZZLE_128B);
       if (rc != ISX_OK) return rc;
-      auto kern = l2norm_project_direct_kernel;
-      const int smem = static_cast<int>(ProjDSmem::kDynamicBytes);
-      ISX_CHECK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-      cudaLaunchConfig_t cfg = {};
-      cfg.gridDim = dim3(static_cast<unsigned>(grid));
-      cfg.blockDim = dim3(kProjTThreads);
-      cfg.dynamicSmemBytes = static_cast<size_t>(smem);
-      cfg.stream = stream;
-      cudaLaunchAttribute attr[1];
-      attr[0].id = cudaLaunchAttributeClusterDimension;
-      attr[0].val.clusterDim.x = 2;
-      attr[0].val.clusterDim.y = 1;
-      attr[0].val.clusterDim.z = 1;
-      cfg.attrs = attr;
-      cfg.numAttrs = 1;
-      ISX_CHECK_CUDA(cudaLaunchKernelEx(&cfg, kern, twh, twl, tx, tout, p));
-      return ISX_OK;
     }
-    if (p.prefetch && mode == 0) {
-      auto kern = l2norm_project_tmem_kernel;
-      const int smem = static_cast<int>(ProjTSmem::kDynamicBytes);
-      ISX_CHECK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-      cudaLaunchConfig_t cfg = {};
-      cfg.gridDim = dim3(static_cast<unsigned>(grid));
-      cfg.blockDim = dim3(kProjTThreads);
-      cfg.dynamicSmemBytes = static_cast<size_t>(smem);
-      cfg.stream = stream;
-      cudaLaunchAttribute attr[1];
-      attr[0].id = cudaLaunchAttributeClusterDimension;
-      attr[0].val.clusterDim.x = 2;
-      attr[0].val.clusterDim.y = 1;
-      attr[0].val.clusterDim.z = 1;
-      cfg.attrs = attr;
-      cfg.numAttrs = 1;
-      ISX_CHECK_CUDA(cudaLaunchKernelEx(&cfg, kern, twh, twl, tx, p));
-      return ISX_OK;
-    }
-    if (p.prefetch && (mode == 1 || mode == 3)) return launch_project_kernel<-1, 2>(twh, twl, tx, p, grid, stream);
+    p.rowmajor = rowmajor;
+    p.fast = fast;
+    return launch_pair(l2norm_project_kernel<true>, proj_threads(true), ProjSmem<true>::kDynamicBytes, grid, stream,
+                       twh, twl, tx, p);
   }
-  if (E % PK == 0 && hw == 256) return launch_project_kernel<256, NCTA>(twh, twl, tx, p, grid, stream);
-  if (E % PK == 0 && hw == 64) return launch_project_kernel<64, NCTA>(twh, twl, tx, p, grid, stream);
-  return launch_project_kernel<0, NCTA>(twh, twl, tx, p, grid, stream);
-}
-
-int launch_project(const float* fmap, long long m_total, int E, int hw, int k, int normalize,
-                   const void* packed, float* out, cudaStream_t stream, const char* fn, int fast = 0) {
-  (void)fn;
-  int sms = 148;
-  int rc = device_sm_count(&sms);
-  if (rc != ISX_OK) return rc;
-  // shapes the staged pair kernel cannot take run the exact three-pass kernels even when the fast
-  // mode was asked for (more accurate, never less)
-  if (sms >= 2 && project_ncta() == 2) return launch_project_n<2>(fmap, m_total, E, hw, k, normalize, fast, packed, out, stream);
-  return launch_project_n<1>(fmap, m_total, E, hw, k, normalize, 0, packed, out, stream);
+  // 3. The map's shape or alignment gives no TMA boxes for the staged kernel.  K3d loads any shape from
+  //    global memory; its TMA-store epilogue needs 16-byte output rows and its transform whole
+  //    16-feature groups.  Only the staged kernel has the fp16 pass, so these shapes run the exact
+  //    three-pass split even when the fp16 pass was asked for (more accurate, never less).
+  if (k % 4 == 0 && E % 16 == 0 && (reinterpret_cast<uintptr_t>(out) & 15u) == 0 && m_total < (1ll << 31)) {
+    CUtensorMap tout;
+    rc = encode_tmap_2d(&tout, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, out, static_cast<uint64_t>(m_total),
+                        static_cast<uint64_t>(k), static_cast<uint64_t>(k) * 4, PM, 32, CU_TENSOR_MAP_SWIZZLE_128B);
+    if (rc != ISX_OK) return rc;
+    return launch_pair(l2norm_project_direct_kernel, kProjDThreads, ProjDSmem::kDynamicBytes, grid, stream, twh, twl,
+                       tout, p);
+  }
+  // 4. K3d cannot write this output (or E % 16 != 0): the register path loads any shape and stores
+  //    rows of k floats.  It reads no map descriptor; twh only fills the slot.
+  return launch_pair(l2norm_project_kernel<false>, proj_threads(false), ProjSmem<false>::kDynamicBytes, grid, stream,
+                     twh, twl, twh, p);
 }
 
 }  // namespace
@@ -1612,8 +1208,8 @@ static int l2norm_project_impl(const char* fn, int fast, const float* fmap, int 
   const long long hw = static_cast<long long>(h) * w;
   ISX_REQUIRE(hw < (1ll << 24) && static_cast<long long>(B) * hw < (1ll << 40), "%s: feature map too large", fn);
   if (!pool) {
-    return launch_project(fmap, static_cast<long long>(B) * hw, E, static_cast<int>(hw), k, normalize, packed, out,
-                          stream, fn, fast);
+    return launch_project(fmap, static_cast<long long>(B) * hw, E, static_cast<int>(hw), k, normalize, fast, packed, out,
+                          stream);
   }
   ISX_REQUIRE(normalize, "%s: pool == 1 requires normalize == 1", fn);
   ISX_REQUIRE(E <= 64 * kPoolMaxAcc, "%s: pooled mode supports at most %d channels (E=%d)", fn, 64 * kPoolMaxAcc, E);
@@ -1646,7 +1242,7 @@ static int l2norm_project_impl(const char* fn, int fast, const float* fmap, int 
     ISX_CHECK_CUDA(cudaGetLastError());
   }
   // project the pooled rows: an n x F matrix is a feature "map" with one cell per image
-  return launch_project(pooled, B, E, 1, k, /*normalize=*/0, packed, out, stream, fn, fast);
+  return launch_project(pooled, B, E, 1, k, /*normalize=*/0, fast, packed, out, stream);
 }
 
 int isx_l2norm_project(const float* fmap, int B, int E, int h, int w, int pool, int normalize,

@@ -100,10 +100,17 @@ def test_l2norm_cells_stays_in_bounds(B, E, h, w):
     assert torch.allclose(norms, torch.ones_like(norms), atol=1e-5)
 
 
-@pytest.mark.parametrize("mode", ["staged", "direct", "tmem", "reg"])
-@pytest.mark.parametrize("B,E,h,w,k", [(3, 320, 16, 16, 96), (5, 128, 8, 8, 24), (2, 192, 7, 10, 100), (9, 64, 4, 4, 256)])
-def test_project_stays_in_bounds(mode, B, E, h, w, k, monkeypatch):
-    monkeypatch.setenv("ISX_PROJECT_MODE", mode)
+@pytest.mark.parametrize("aligned", [True, False])
+@pytest.mark.parametrize("B,E,h,w,k", [(3, 320, 16, 16, 96), (3, 320, 16, 16, 95), (5, 128, 8, 8, 24), (5, 128, 8, 8, 23),
+                                       (2, 192, 7, 10, 100), (2, 192, 7, 10, 99), (9, 64, 4, 4, 256), (9, 64, 4, 4, 255),
+                                       (2, 200, 7, 10, 100)])
+def test_project_stays_in_bounds(B, E, h, w, k, aligned):
+    """Each per-cell kernel, reached by shape and alignment (launch_project in project.cu): an aligned
+    16 x 16, 8 x 8 or 4 x 4 map takes the staged kernel (rule 2) for any k; otherwise k % 4 == 0 takes
+    K3d (rule 3) and k % 4 != 0 the register path (rule 4), which writes rows of k floats without TMA
+    stores.  E = 200 (E % 16 != 0) takes the register path with k % 4 == 0 (rule 4 through E % 16), so
+    its float4 stores and their scalar tail are checked too.  An unaligned map starts 4 bytes into its
+    allocation."""
     lib = _lib.load()
     rng = np.random.default_rng(k)
     comps = torch.from_numpy(np.linalg.qr(rng.standard_normal((E, k)))[0].astype(np.float32) if k <= E else
@@ -112,10 +119,13 @@ def test_project_stays_in_bounds(mode, B, E, h, w, k, monkeypatch):
     packed = torch.empty(lib.isx_project_packed_bytes(E, k), dtype=torch.uint8, device="cuda")
     _lib.check(lib.isx_project_pack(means.data_ptr(), comps.data_ptr(), E, k, comps.stride(0), comps.stride(1), packed.data_ptr(),
                                     packed.numel(), stream()), "pack")
-    fmap = torch.randn((B, E, h, w), device="cuda").abs_()
+    off = 0 if aligned else 1
+    fmap = torch.empty(B * E * h * w + off, device="cuda")[off:].view(B, E, h, w)
+    fmap.copy_(torch.randn((B, E, h, w), device="cuda").abs_())
+    assert (fmap.data_ptr() % 16 == 0) == aligned
     out = Guarded(B * h * w * k * 4)
     _lib.check(lib.isx_l2norm_project(fmap.data_ptr(), B, E, h, w, 0, 1, packed.data_ptr(), k, out.ptr, None, 0, stream()), "project")
-    out.check(f"l2norm_project {mode} {(B, E, h, w, k)}")
+    out.check(f"l2norm_project {(B, E, h, w, k)} aligned={aligned}")
     got = out.as_tensor(torch.float32, (B * h * w, k))
     ref = torch.nn.functional.normalize(fmap, dim=1).permute(0, 2, 3, 1).reshape(-1, E) @ comps
     assert (got - ref).abs().max() <= 1e-4 * max(1.0, float(ref.abs().max()))

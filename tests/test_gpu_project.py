@@ -223,18 +223,36 @@ def test_pca_fit_gpu_moments_and_components(golden):
     assert out.shape == (64, 8) and torch.isfinite(out).all()
 
 
-@pytest.mark.parametrize("mode", ["direct", "staged", "tmem", "reg"])
-def test_per_cell_kernel_variants_agree(mode, monkeypatch):
-    """The per-cell kernels (direct global loads + A operand in tensor memory + TMA-store epilogue, the
-    default / operand tiles in shared memory / A operand in tensor memory with a raw ring /
-    register-path loads) are selected by ISX_PROJECT_MODE; each must meet the oracle."""
+@pytest.mark.parametrize(
+    "E,h,w,k,aligned",
+    [
+        (320, 16, 16, 96, True),   # rule 2: staged kernel; hw = 256, a 128-cell tile is half an image
+        (320, 8, 8, 96, True),     # rule 2: staged kernel; hw = 64, a tile spans two images
+        (320, 16, 16, 96, False),  # rule 3: K3d
+        (320, 8, 8, 96, False),    # rule 3: K3d
+        (320, 16, 16, 95, False),  # rule 4: register path through k % 4 != 0
+        (320, 8, 8, 95, False),    # rule 4: register path through k % 4 != 0
+        (320, 7, 10, 96, True),    # rule 3: K3d; 70 cells per image fit no TMA box
+        (320, 7, 10, 95, True),    # rule 4: register path through k % 4 != 0
+        (200, 7, 10, 100, True),   # rule 4: register path through E % 16 != 0; float4 stores, scalar tail
+        (200, 16, 16, 96, False),  # rule 4: register path through E % 16 != 0; float4 stores only
+    ],
+)
+def test_per_cell_kernel_variants_agree(E, h, w, k, aligned):
+    """Every per-cell kernel meets the oracle.  The launch picks the kernel from the input alone, by
+    the first rule that fits (launch_project in project.cu):
+      rule 2, l2norm_project_kernel<true> (staged): 16-byte aligned map, 4 | hw, hw = 128 n or 128 = hw n;
+      rule 3, l2norm_project_direct_kernel (K3d): otherwise, if k % 4 == 0 and E % 16 == 0;
+      rule 4, l2norm_project_kernel<false> (register path): otherwise.  With k % 4 == 0 its epilogue
+      writes float4 pieces, else single floats.
+    An unaligned map is a view 4 bytes into its allocation, so 16 x 16 and 8 x 8 maps reach all three.
+    B = 9 leaves the last CTA pair ragged."""
     import torch
 
     from imagescry_b200.models.decomposition import PCA
 
-    monkeypatch.setenv("ISX_PROJECT_MODE", mode)
     rng = np.random.default_rng(3)
-    B, E, h, w, k = 9, 320, 16, 16, 96  # hw = 256: 128-cell tiles are half images; ragged last pair
+    B = 9
     fmap = np.abs(rng.standard_normal((B, E, h, w))).astype(np.float32)
     comps = np.linalg.qr(rng.standard_normal((E, k)))[0].astype(np.float32)
     means = (rng.standard_normal(E) * 0.01).astype(np.float32)
@@ -245,14 +263,14 @@ def test_per_cell_kernel_variants_agree(mode, monkeypatch):
     pca._num_features.data = torch.tensor(E)
     pca._num_components.data = torch.tensor(k)
     pca = pca.cuda()
-    out = pca.project_feature_map(torch.from_numpy(fmap).cuda()).cpu().numpy()
+    off = 0 if aligned else 1  # one float into the allocation: 4 bytes off a 16-byte boundary
+    x = torch.empty(fmap.size + off, device="cuda")[off:].view(fmap.shape)
+    x.copy_(torch.from_numpy(fmap))
+    assert (x.data_ptr() % 16 == 0) == aligned
+    out = pca.project_feature_map(x).cpu().numpy()
     ref = O.pipeline_project(fmap, means, comps)
     scale = np.linalg.norm(ref, axis=1, keepdims=True)
     assert (np.abs(out - ref) / scale).max() < 2e-5
-    fm8 = fmap[:, :, :8, :8].copy()  # hw = 64: a tile spans two images
-    out8 = pca.project_feature_map(torch.from_numpy(fm8).cuda()).cpu().numpy()
-    ref8 = O.pipeline_project(fm8, means, comps)
-    assert (np.abs(out8 - ref8) / np.linalg.norm(ref8, axis=1, keepdims=True)).max() < 2e-5
 
 
 @pytest.mark.parametrize("pool", [None, "mean"])

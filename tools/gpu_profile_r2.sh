@@ -14,7 +14,6 @@ run knn_d256 knn_search_kernel 2 python tools/run_case.py knn --k 10 --d 256 --i
 run l2norm l2norm_cells 2 python tools/run_case.py l2norm --batch 2048 --iters 1 --warm 2
 run syrk cov_syrk_kernel 2 python tools/run_case.py pcafit --n 65536 --d 1280 --iters 1 --warm 1
 run project_staged l2norm_project_kernel 2 python tools/run_case.py project --batch 2048 --iters 1 --warm 2
-ISX_PROJECT_MODE=direct run project_direct l2norm_project_direct 2 python tools/run_case.py project --batch 2048 --iters 1 --warm 2
 # launch list of the bench command (cold-cache, serialised: compare shares)
 python bench.py --steps 2 --warmup 3 --no-extra --no-verify --preheat 0.2 > gpurun_out/launch_plain.log 2>&1 &&
 ncu --metrics gpu__time_duration.sum --clock-control none -c 400 --csv --log-file gpurun_out/r2_launches.csv python bench.py --steps 2 --warmup 3 --no-extra --no-verify --preheat 0.2 > gpurun_out/launch_ncu.log 2>&1

@@ -3,7 +3,7 @@
 
     python tools/run_case.py knn --n 1000000 --q 10000 --k 100 [--iters 3]
     python tools/run_case.py preprocess --case resize256|nhwc_f32|nhwc_bf16|nchw_f32 [--batch 1024]
-    python tools/run_case.py project --pool none|mean [--batch 1024]
+    python tools/run_case.py project --pool none|mean [--batch 1024] [--side 16]
 Prints the CUDA-event time per iteration and the roofline fraction."""
 from __future__ import annotations
 
@@ -49,7 +49,7 @@ def main():
     ap.add_argument("--pool", default="none")
     ap.add_argument("--batch", type=int, default=1024)
     ap.add_argument("--precision", default="exact")
-    ap.add_argument("--side", type=int, default=16, help="feature-map side for the l2norm case")
+    ap.add_argument("--side", type=int, default=16, help="feature-map side for the l2norm and project cases")
     a = ap.parse_args()
     peaks = json.load(open(os.path.join(REPO, "MEASURED_PEAKS.json"))) if os.path.exists(os.path.join(REPO, "MEASURED_PEAKS.json")) else {"hbm_gbs": 6650.0, "bf16_tflops": 1590.0, "bf16_tflops_sustained": 1400.0}
     dev = torch.device("cuda", 0)
@@ -120,7 +120,7 @@ def main():
     else:
         from imagescry_b200.models.decomposition import PCA
 
-        B, E, h, w, k = a.batch, 1280, 16, 16, 256
+        B, E, h, w, k = a.batch, 1280, a.side, a.side, 256
         fmap = torch.empty((B, E, h, w), dtype=torch.float32, device=dev)
         for s in range(0, B, 256):
             e = min(B, s + 256)

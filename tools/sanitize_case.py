@@ -36,11 +36,16 @@ l2_normalize_cells(torch.randn((2, 96, 7, 10), generator=g, device="cuda"))
 x = torch.randn((3000, 320), generator=g, device="cuda") * torch.linspace(2, 0.1, 320, device="cuda") + 0.3
 pca = PCA(min_num_components=32, max_num_components=32).cuda().fit(x)
 pca.transform(x[:500])
-for mode in ("staged", "direct", "tmem", "reg"):
-    os.environ["ISX_PROJECT_MODE"] = mode
-    pca.project_feature_map(fmap)
-os.environ.pop("ISX_PROJECT_MODE")
-pca.project_feature_map(torch.randn((2, 320, 7, 10), generator=g, device="cuda"))  # odd shape: K3d
+pca31 = PCA(min_num_components=31, max_num_components=31).cuda().fit(x)
+unaligned = torch.empty(fmap.numel() + 1, device="cuda")[1:].view(fmap.shape).copy_(fmap)  # 4 bytes off 16
+odd = torch.randn((2, 320, 7, 10), generator=g, device="cuda")
+pca.project_feature_map(fmap)          # staged kernel
+pca.project_feature_map(unaligned)     # K3d: no TMA boxes for an unaligned map
+pca31.project_feature_map(unaligned)   # register path: k % 4 != 0
+pca.project_feature_map(odd)           # odd shape: K3d
+pca31.project_feature_map(odd)         # odd shape, k % 4 != 0: register path
+pca200 = PCA(min_num_components=32, max_num_components=32).cuda().fit(x[:, :200].contiguous())
+pca200.project_feature_map(torch.randn((2, 200, 7, 10), generator=g, device="cuda"))  # E % 16 != 0: register path, float4 stores
 pca.project_feature_map(fmap, pool="mean")
 print("stage 2 ok", flush=True)
 
