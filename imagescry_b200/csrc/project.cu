@@ -317,8 +317,13 @@ l2norm_project_kernel(const __grid_constant__ CUtensorMap tmap_whi, const __grid
 #pragma unroll
           for (int i = 0; i < 16; ++i) x[i] = raw[i * cb];
         }
+        // The next fill of this stage is a TMA write (async proxy) issued as soon as every warp has
+        // arrived.  A bare arrive does not wait for the loads above to return (the compiler issues it
+        // right behind them), so a late load could read the next fill: the proxy fence completes this
+        // thread's reads of the stage before the warp releases it.
+        fence_proxy_async_smem();
         __syncwarp();
-        if (lane == 0) mbar_arrive(&raw_empty[rs]);  // release: this warp's reads of the stage are done
+        if (lane == 0) mbar_arrive(&raw_empty[rs]);
         if (++rs == static_cast<uint32_t>(RAW_STAGES)) { rs = 0; rph ^= 1; }
         uint32_t hi[8], lo[8];
         if (p.fast) {
@@ -1053,6 +1058,9 @@ l2norm_pool_tma_kernel(const __grid_constant__ CUtensorMap tmap, int B, int E, i
         acc[j] = 0.f;
       }
     }
+    // The refill of `cur` is a TMA write (async proxy); as in the staged projection kernel's raw ring,
+    // the proxy fence completes this thread's generic reads of the buffer before the barrier releases it.
+    fence_proxy_async_smem();
     __syncthreads();  // everyone is done with `cur` (and part/rn_s) before the buffer is refilled
   }
 }

@@ -137,9 +137,11 @@ def test_pipeline_predict_step_end_to_end(golden):
 
 
 def test_full_size_feature_map_properties():
-    """BASELINE.json config 3b at full size (4096 x 1280 x 16 x 16 fp32 -> 256-d): sampled images
-    against an fp64 torch evaluation of the reference's formula (embedding.py:74, data.py:118,
-    decomposition.py:91), layout of pipelines.py:82-84, and pooled == mean of normalised cells."""
+    """BASELINE.json config 3b at full size (4096 x 1280 x 16 x 16 fp32 -> 256-d): one image from every
+    round of pair tiles (an image is one 256-cell pair tile; pair p runs tiles p, p + P, ...) against
+    an fp64 torch evaluation of the reference's formula (embedding.py:74, data.py:118,
+    decomposition.py:91), layout of pipelines.py:82-84, pooled == mean of normalised cells, and two
+    calls give bit-identical outputs."""
     import torch
 
     from imagescry_b200.models.decomposition import PCA
@@ -158,9 +160,14 @@ def test_full_size_feature_map_properties():
     pca._num_components.data = torch.tensor(k, device="cuda")
     out = pca.project_feature_map(fmap)
     assert out.shape == (B, k, h, w) and out.stride() == (h * w * k, 1, w * k, k)  # NHWC memory
+    assert torch.equal(pca.project_feature_map(fmap), out)
     pooled = pca.project_feature_map(fmap, pool="mean")
     assert pooled.shape == (B, k)
-    for b in (0, 777, B - 1):
+    P = min(torch.cuda.get_device_properties(0).multi_processor_count // 2, B)  # CTA pairs launched
+    rounds = -(-B // P)
+    images = [min(r * P + (r * 29) % P, B - 1) for r in range(rounds)]  # a different pair in every round
+    assert len(images) >= 3 and images[-1] >= B - P
+    for b in images:
         x = fmap[b].double()
         e = x / x.norm(dim=0, keepdim=True).clamp_min(1e-12)
         flat = e.permute(1, 2, 0).reshape(-1, E)
