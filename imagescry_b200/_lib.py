@@ -29,6 +29,7 @@ KNN_CONTINUE = 1
 KNN_NO_FINALIZE = 2
 KNN_EXCLUDE_SELF = 4
 KNN_PACKED = 8
+KNN_RANGE_WORKSPACE_BYTES = 2048  # ISX_KNN_RANGE_WORKSPACE_BYTES
 
 # name -> (restype, argtypes); mirrors include/imagescry_b200.h one to one
 SIGNATURES: dict[str, tuple] = {
@@ -98,6 +99,15 @@ SIGNATURES: dict[str, tuple] = {
          c_void_p, c_void_p, c_size_t, c_void_p],
     ),
     "isx_topk_merge_grouped": (c_int, [c_void_p, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "isx_knn_range": (
+        c_int,
+        [c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_int, c_int, c_float, c_int64, c_int64, c_int, c_void_p,
+         c_int64, c_void_p, c_void_p, c_size_t, c_void_p],
+    ),
+    "isx_knn_range_sort_workspace_bytes": (c_size_t, [c_int64, c_int]),
+    "isx_knn_range_sort": (
+        c_int, [c_void_p, c_int64, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]
+    ),
     "isx_roi_rasterize": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int64, c_void_p, c_void_p]),
     "isx_masked_pool": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_int, c_int64, c_void_p, c_void_p]),
 }

@@ -35,6 +35,7 @@
 
 #include <algorithm>
 #include <cfloat>
+#include <cmath>
 #include <climits>
 #include <cstdlib>
 
@@ -211,6 +212,12 @@ struct KnnParams {
   uint32_t throttle_window, throttle_every;
   uint32_t* progress;    // [units] tiles loaded so far by every scheduling unit (lockstep throttle)
   const int32_t* row_group;  // [n] group id of every store row (grouped search only)
+  // range search only: every column with fl(raw * query_rnorm) >= range_tau is appended to
+  // range_rec as {query, global row, fp32 score bits}; range_count counts past range_cap
+  float range_tau;
+  int32_t* range_rec;
+  long long range_cap;
+  unsigned long long* range_count;
 #ifdef ISX_KNN_PROFILE
   unsigned long long* prof;  // [16] wait-cycle counters (diagnostic build only: -DISX_KNN_PROFILE)
   int debug_skip_select;     // ISX_KNN_SKIP_SELECT=1: the epilogue only loads and releases (floor of the MMA pipeline)
@@ -243,8 +250,9 @@ struct KnnParams {
 
 // Shared-memory plan.  k <= kSmallK: 32-entry per-row candidate buffers live in shared memory next to
 // a 4-stage operand ring (the buffers are XOR-swizzled by row so that 32 rows appending at the same
-// depth hit different banks).  Larger k: 256-entry buffers in the global workspace.
-template <int CAP, int NCTA, bool RES_ = false, bool GROUPED = false>
+// depth hit different banks).  Larger k: 256-entry buffers in the global workspace.  Range search
+// (RANGE) has no candidate buffers: it is the CAP = 32 plan without them.
+template <int CAP, int NCTA, bool RES_ = false, bool GROUPED = false, bool RANGE = false>
 struct KnnSmem {
   // RES: the query tile (all k-blocks, at most kResKb = 4, i.e. d <= 256) stays resident in shared
   // memory for a whole item and the ring holds store tiles only: half the operand traffic per tile.
@@ -255,7 +263,7 @@ struct KnnSmem {
   static constexpr int STAGES = RES ? 6 : (NCTA == 2) ? (CAP <= 32 ? 5 : 6) : (CAP <= 32 ? 3 : 4);
   static constexpr bool kSmemCand = (CAP <= 32);
   static constexpr int CHUNK = kSmemCand ? 16 : 32;  // accumulator columns per selection window
-  static constexpr uint32_t kCandBytes = kSmemCand ? G * BM * CAP * 8 : 0;
+  static constexpr uint32_t kCandBytes = (kSmemCand && !RANGE) ? G * BM * CAP * 8 : 0;
   static constexpr uint32_t kAOff = 0;
   static constexpr uint32_t kBOff = kAOff + (RES ? kResKb : STAGES) * A_STAGE_BYTES;
   static constexpr uint32_t kCandOff = kBOff + STAGES * B_STAGE_BYTES;
@@ -559,14 +567,86 @@ __device__ __forceinline__ void prune_row_grouped(uint2* row_buf, int swz, int c
   }
 }
 
+// ---- range search ------------------------------------------------------------------------------
+// A store row e is a hit of query row q when score = fl(raw · rnorm_q) >= tau, raw = fl(dot · rnorm_e)
+// being what the epilogue holds after scaling: the product K5 forms for search(), so a hit's score is
+// bit for bit the one search() reports.
+
+// Raw-score bound of one query row: every raw r of a hit satisfies r > bound, so the fast path's
+// `vmax > thr` never drops a hit.  Argument (round-to-nearest, rq = rnorm_q finite and > 0): let
+// t = pred(tau), the float just below tau.  fl is monotone, so r · rq <= t would give fl(r · rq) <= t
+// < tau: a hit has r · rq > t, i.e. r > t / rq in exact arithmetic.  The quotient is formed in double
+// (t and rq are floats, so it is within 2^-53 relative of t / rq and never overflows or underflows),
+// rounded down to float, and stepped down one more float: a double rounding error of 2^-53 relative
+// can move it across at most one float, so the result is <= t / rq < r.  Rows with rq = 0 or +inf
+// (an overflowing norm) get no bound: every column takes the exact test.
+__device__ __forceinline__ float range_raw_bound(float tau, float rq) {
+  if (!(rq > 0.f) || isinf(rq)) return -INFINITY;
+  const float t = nextafterf(tau, -INFINITY);
+  const float b = __double2float_rd(static_cast<double>(t) / static_cast<double>(rq));
+  return nextafterf(b, -INFINITY);
+}
+
+// Rare path of one 32-column chunk: the exact test of every column of the rows whose chunk maximum
+// passed the bound, then one append per warp.  Lanes' hit counts are prefix-summed, one 64-bit
+// atomicAdd reserves the warp's slots, and a record is written only when its slot is below the
+// capacity; the counter keeps counting past it, so the caller learns the exact total.  Columns past
+// the store's end (ncols) and the query's own row (self_row, -1 when off) are never hits.
+__device__ __forceinline__ void range_append(const uint32_t (&r)[32], bool pass, float rq, int qrow, int cbase,
+                                             int ncols, int gcol0, int self_row, const KnnParams& p) {
+  const int lane = static_cast<int>(lane_id());
+  uint32_t hits = 0;
+  if (pass) {
+#pragma unroll
+    for (int j = 0; j < 32; ++j) {
+      const float s = __fmul_rn(__uint_as_float(r[j]), rq);
+      const bool take = s >= p.range_tau && cbase + j < ncols && gcol0 + cbase + j != self_row;
+      hits |= take ? (1u << j) : 0u;
+    }
+  }
+  const int mine = __popc(hits);
+  int incl = mine;
+#pragma unroll
+  for (int o = 1; o < 32; o <<= 1) {
+    const int t = __shfl_up_sync(kFullMask, incl, o);
+    if (lane >= o) incl += t;
+  }
+  const int total = __shfl_sync(kFullMask, incl, 31);
+  if (total == 0) return;
+  unsigned long long base = 0;
+  if (lane == 31) base = atomicAdd(p.range_count, static_cast<unsigned long long>(total));
+  base = __shfl_sync(kFullMask, base, 31);
+  unsigned long long slot = base + static_cast<unsigned long long>(incl - mine);
+  if (!hits) return;
+  // unrolled over the columns: an index taken from the hit mask would move the accumulator registers
+  // to local memory for the whole epilogue
+#pragma unroll
+  for (int j = 0; j < 32; ++j) {
+    if ((hits >> j) & 1u) {
+      if (slot < static_cast<unsigned long long>(p.range_cap)) {
+        int32_t* rec = p.range_rec + 3 * slot;
+        rec[0] = qrow;
+        rec[1] = gcol0 + cbase + j;
+        rec[2] = static_cast<int32_t>(__float_as_uint(__fmul_rn(__uint_as_float(r[j]), rq)));
+      }
+      ++slot;
+    }
+  }
+}
+
 // GROUPED: image-level search (knn_search_grouped_kernel).  The k-th best DISTINCT-GROUP score of
 // any subset of the store is a lower bound of the global one, so the fast path, the shared bound and
 // the item-end skip stay as they are; only where a threshold is derived — the buffer prune, the
 // item-end merge into the running list and the finalising merge — entries are de-duplicated by group
 // before k are counted.
-template <int CAP, int NCTA, bool RES, bool GROUPED>
+//
+// RANGE: range search (knn_range_kernel, CAP = 32 variants only).  The threshold is fixed and known
+// before the first tile, so the epilogue keeps the fast path and replaces the rest: no candidate
+// buffers, prunes, shared bound or item end; the rare path tests every column of the chunk exactly
+// and appends the hits to a global record buffer (range_append).
+template <int CAP, int NCTA, bool RES, bool GROUPED, bool RANGE = false>
 __device__ __forceinline__ void knn_search_body(const CUtensorMap& tmap_q, const CUtensorMap& tmap_e, const KnnParams& p) {
-  using L = KnnSmem<CAP, NCTA, RES, GROUPED>;
+  using L = KnnSmem<CAP, NCTA, RES, GROUPED, RANGE>;
   constexpr int STAGES = L::STAGES;
   constexpr int kEpiGroups = L::G;
   constexpr int kGroupCols = BN / kEpiGroups;
@@ -792,6 +872,13 @@ __device__ __forceinline__ void knn_search_body(const CUtensorMap& tmap_q, const
       // best of ANY subset of the store cannot be in the global top-k, so other splits' progress
       // prunes this one (the partial list may then hold fewer than k entries; the merge pads).
       float thr = row_valid ? -INFINITY : INFINITY;
+      float range_rq = 0.f;  // range search: the query's inverse norm
+      if constexpr (RANGE) {
+        if (row_valid) {
+          range_rq = __ldg(p.query_rnorm + qrow);
+          thr = range_raw_bound(p.range_tau, range_rq);
+        }
+      }
       int cnt = 0;
       float row_best = -INFINITY;  // best score this item has appended for the row
 
@@ -810,7 +897,9 @@ __device__ __forceinline__ void knn_search_body(const CUtensorMap& tmap_q, const
           pre_g = (n0_ + et < p.n) ? __ldg(p.row_group + n0_ + et) : -1;
           if (kEpiGroups == 1) pre_g2 = (n0_ + et + 128 < p.n) ? __ldg(p.row_group + n0_ + et + 128) : -1;
         }
-        if (row_valid) pre_thr = *reinterpret_cast<const volatile uint32_t*>(p.thr_shared + qrow);
+        if constexpr (!RANGE) {
+          if (row_valid) pre_thr = *reinterpret_cast<const volatile uint32_t*>(p.thr_shared + qrow);
+        }
       };
       prefetch_tile(nb0);
 
@@ -835,7 +924,9 @@ __device__ __forceinline__ void knn_search_body(const CUtensorMap& tmap_q, const
             if (lane == 0) chunk_uni[(et + 128) >> 5] = uni1 ? 1 : 0;
           }
         }
-        if (row_valid) thr = fmaxf(thr, thr_decode_below(pre_thr));
+        if constexpr (!RANGE) {
+          if (row_valid) thr = fmaxf(thr, thr_decode_below(pre_thr));
+        }
         if (nb + 1 < nb1) prefetch_tile(nb + 1);
         ISX_PROF_BEGIN();
         epilogue_bar_sync(eg);
@@ -916,6 +1007,10 @@ __device__ __forceinline__ void knn_search_body(const CUtensorMap& tmap_q, const
         auto collect_chunk = [&](uint32_t (&r)[32], int cbase, const float (&g)[8], float vmax) {
           if (!__any_sync(kFullMask, vmax > thr)) return;
           ISX_PROF_COUNT(10, 1);
+          if constexpr (RANGE) {
+            range_append(r, vmax > thr, range_rq, qrow, cbase, ncols, gcol0, self_row, p);
+            return;
+          }
           ISX_PROF_BEGIN1();
           const bool hit = vmax > thr;
           if constexpr (GROUPED) {
@@ -1064,10 +1159,12 @@ __device__ __forceinline__ void knn_search_body(const CUtensorMap& tmap_q, const
         // Off the hand-off path (the accumulator stage is already released): prune the rows whose
         // buffers are more than half-way from k to full, so that a prune inside the next tiles' chunk
         // loops — where it delays the release every other warp of the pair waits for — stays an exception.
-        prune_rows(__ballot_sync(kFullMask, 2 * cnt > CAP + p.k));
+        if constexpr (!RANGE) prune_rows(__ballot_sync(kFullMask, 2 * cnt > CAP + p.k));
         ISX_PROF_END(6);
         if (++acc == ACC_STAGES) { acc = 0; acc_phase ^= 1; }
       }
+      // range search: the hits are in the record buffer already; there is no list to merge
+      if constexpr (RANGE) continue;
 
       // item done: sort every row's candidates and merge the best k into the query's RUNNING list in
       // global memory (under a per-query lock; lists of different items never share a store row, so
@@ -1408,6 +1505,13 @@ knn_search_grouped_kernel(const __grid_constant__ CUtensorMap tmap_q, const __gr
   knn_search_body<CAP, NCTA, RES, true>(tmap_q, tmap_e, p);
 }
 
+template <int NCTA, bool RES>
+__global__ void __launch_bounds__(knn_threads(32), 1)
+knn_range_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_constant__ CUtensorMap tmap_e,
+                 const KnnParams p) {
+  knn_search_body<32, NCTA, RES, false, true>(tmap_q, tmap_e, p);
+}
+
 // ------------------------------------------------------------------------------------------
 // K5: merge g sorted-or-not partial lists per query into the final top-k.  One warp per query.
 // ------------------------------------------------------------------------------------------
@@ -1603,10 +1707,12 @@ KnnWorkspace knn_workspace(int max_grid, int q, int k) {
   return w;
 }
 
-template <int CAP, int NCTA, bool RES = false, bool GROUPED = false>
+template <int CAP, int NCTA, bool RES = false, bool GROUPED = false, bool RANGE = false>
 int launch_search(const CUtensorMap& tq, const CUtensorMap& te, const KnnParams& p, int grid, cudaStream_t stream) {
-  auto kern = GROUPED ? knn_search_grouped_kernel<CAP, NCTA, RES> : knn_search_kernel<CAP, NCTA, RES>;
-  const int smem = static_cast<int>(KnnSmem<CAP, NCTA, RES, GROUPED>::kDynamicBytes);
+  static_assert(!RANGE || (CAP == 32 && !GROUPED), "range search has the CAP = 32 plan only");
+  auto kern = RANGE ? knn_range_kernel<NCTA, RES>
+                    : GROUPED ? knn_search_grouped_kernel<CAP, NCTA, RES> : knn_search_kernel<CAP, NCTA, RES>;
+  const int smem = static_cast<int>(KnnSmem<CAP, NCTA, RES, GROUPED, RANGE>::kDynamicBytes);
   ISX_CHECK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = dim3(static_cast<unsigned>(grid));
@@ -1623,6 +1729,31 @@ int launch_search(const CUtensorMap& tq, const CUtensorMap& te, const KnnParams&
   ISX_CHECK_CUDA(cudaLaunchKernelEx(&cfg, kern, tq, te, p));
   return ISX_OK;
 }
+
+// Lockstep window in tiles: measured best 16-32 at d = 1280 (640 KB of store rows per tile); it is a
+// footprint in L2, so it scales with 1/d, and the poll interval (a third of it, rounded down to a
+// power of two) with it: one poll reads every unit's counter, ~1 us, against 0.6 us per tile at d = 256.
+void set_throttle(KnnParams& p, int d) {
+  const uint32_t base = getenv("ISX_KNN_WINDOW") ? static_cast<uint32_t>(atoi(getenv("ISX_KNN_WINDOW"))) : 24u;
+  const uint64_t scaled = static_cast<uint64_t>(base) * 1280u / static_cast<uint32_t>(std::max(d, 64));
+  p.throttle_window = static_cast<uint32_t>(std::min<uint64_t>(std::max<uint64_t>(scaled, base), 1u << 30));
+  uint32_t every = 8;
+  while (every * 2 <= p.throttle_window / 3 && every < 1024) every *= 2;
+  p.throttle_every = every;
+}
+
+#ifdef ISX_KNN_PROFILE
+// Diagnostic build: every launch of the shared K4 body (search, grouped and range) flushes its wait
+// counters into p.prof, so every entry point sets it.
+int set_profile(KnnParams& p, cudaStream_t stream) {
+  static unsigned long long* d_prof = nullptr;
+  if (!d_prof) ISX_CHECK_CUDA(cudaMalloc(&d_prof, 24 * sizeof(unsigned long long)));
+  ISX_CHECK_CUDA(cudaMemsetAsync(d_prof, 0, 24 * sizeof(unsigned long long), stream));
+  p.prof = d_prof;
+  p.debug_skip_select = getenv("ISX_KNN_SKIP_SELECT") ? atoi(getenv("ISX_KNN_SKIP_SELECT")) : 0;
+  return ISX_OK;
+}
+#endif
 
 // CTA pairs halve the shared-memory fill and operand-read traffic per SM (each CTA stages half of
 // every store tile).  They need at least two 128-query blocks to pay off; ISX_KNN_CTA_PAIR=0/1
@@ -1766,24 +1897,11 @@ static int knn_search_impl(const char* fn, const void* store, const float* store
   p.row_group = row_group;
   // a continued search keeps the lists and the bounds they imply; only the lockstep counters restart
   if (cont) ISX_CHECK_CUDA(cudaMemsetAsync(p.progress, 0, 256 * sizeof(uint32_t), stream));
-  // Lockstep window in tiles: measured best 16-32 at d = 1280 (640 KB of store rows per tile); it is a
-  // footprint in L2, so it scales with 1/d, and the poll interval (a third of it, rounded down to a
-  // power of two) with it: one poll reads every unit's counter, ~1 us, against 0.6 us per tile at d = 256.
-  {
-    const uint32_t base = getenv("ISX_KNN_WINDOW") ? static_cast<uint32_t>(atoi(getenv("ISX_KNN_WINDOW"))) : 24u;
-    const uint64_t scaled = static_cast<uint64_t>(base) * 1280u / static_cast<uint32_t>(std::max(d, 64));
-    p.throttle_window = static_cast<uint32_t>(std::min<uint64_t>(std::max<uint64_t>(scaled, base), 1u << 30));
-    uint32_t every = 8;
-    while (every * 2 <= p.throttle_window / 3 && every < 1024) every *= 2;
-    p.throttle_every = every;
-  }
+  set_throttle(p, d);
 
 #ifdef ISX_KNN_PROFILE
-  static unsigned long long* d_prof = nullptr;
-  if (!d_prof) ISX_CHECK_CUDA(cudaMalloc(&d_prof, 24 * sizeof(unsigned long long)));
-  ISX_CHECK_CUDA(cudaMemsetAsync(d_prof, 0, 24 * sizeof(unsigned long long), stream));
-  p.prof = d_prof;
-  p.debug_skip_select = getenv("ISX_KNN_SKIP_SELECT") ? atoi(getenv("ISX_KNN_SKIP_SELECT")) : 0;
+  rc = set_profile(p, stream);
+  if (rc != ISX_OK) return rc;
 #endif
   // the grouped search picks the same (CAP, NCTA, RES) variant as the plain one for the same (q, d, k):
   // same MMA shapes, same scaling, bit-identical scores
@@ -1811,7 +1929,7 @@ static int knn_search_impl(const char* fn, const void* store, const float* store
   {
     unsigned long long h[24];
     ISX_CHECK_CUDA(cudaStreamSynchronize(stream));
-    ISX_CHECK_CUDA(cudaMemcpy(h, d_prof, sizeof(h), cudaMemcpyDeviceToHost));
+    ISX_CHECK_CUDA(cudaMemcpy(h, p.prof, sizeof(h), cudaMemcpyDeviceToHost));
     const double units = static_cast<double>(plan.grid / ncta);
     const double tiles = static_cast<double>(plan.nb) * plan.mb / units;  // per unit
     fprintf(stderr,
@@ -1915,6 +2033,71 @@ int isx_topk_merge_packed(const void* records, int g, int q, int k, float* out_s
   ISX_REQUIRE((reinterpret_cast<uintptr_t>(records) & 7u) == 0, "%s: records must be 8-byte aligned", fn);
   if (g == 0) return launch_merge(out_scores, out_idx, 0, q, k, nullptr, out_scores, out_idx, stream);
   return launch_merge(static_cast<const float*>(records), nullptr, g, q, k, nullptr, out_scores, out_idx, stream);
+}
+
+int isx_knn_range(const void* store, const float* store_rnorm, int64_t n, const void* queries,
+                  const float* query_rnorm, int q, int d, float threshold, int64_t index_base,
+                  int64_t query_index_base, int flags, int32_t* records, int64_t capacity,
+                  unsigned long long* count, void* workspace, size_t workspace_bytes, isx_stream_t stream_) {
+  const char* fn = "isx_knn_range";
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  const bool cont = (flags & ISX_KNN_CONTINUE) != 0, no_self = (flags & ISX_KNN_EXCLUDE_SELF) != 0;
+  ISX_REQUIRE((flags & ~(ISX_KNN_CONTINUE | ISX_KNN_EXCLUDE_SELF)) == 0, "%s: unknown flag bits 0x%x", fn, flags);
+  ISX_REQUIRE(std::isfinite(threshold), "%s: the threshold must be finite (got %g)", fn, static_cast<double>(threshold));
+  ISX_REQUIRE(q > 0 && d > 0 && n >= 0, "%s: need q, d > 0 and n >= 0 (q=%d d=%d n=%lld)", fn, q, d, (long long)n);
+  ISX_REQUIRE(d % 8 == 0, "%s: d = %d must be a multiple of 8 (16-byte rows for TMA)", fn, d);
+  ISX_REQUIRE(n < (1ll << 31) - BN, "%s: at most 2^31 store rows per call (n=%lld); shard the store", fn, (long long)n);
+  ISX_REQUIRE(index_base >= 0 && index_base + n < (1ll << 31), "%s: index_base + n must fit in int32", fn);
+  ISX_REQUIRE(!no_self || (query_index_base >= 0 && query_index_base + q < (1ll << 31)),
+              "%s: query_index_base + q must fit in int32 (got %lld)", fn, (long long)query_index_base);
+  ISX_REQUIRE(capacity >= 0 && capacity < (1ll << 60), "%s: capacity out of range (%lld)", fn, (long long)capacity);
+  ISX_REQUIRE(queries && query_rnorm && count && (capacity == 0 || records), "%s: null pointer", fn);
+  ISX_REQUIRE((reinterpret_cast<uintptr_t>(records) & 3u) == 0 && (reinterpret_cast<uintptr_t>(count) & 7u) == 0,
+              "%s: records must be 4-byte and count 8-byte aligned", fn);
+  ISX_REQUIRE((reinterpret_cast<uintptr_t>(queries) & 15u) == 0 && (reinterpret_cast<uintptr_t>(store) & 15u) == 0,
+              "%s: store and queries must be 16-byte aligned", fn);
+  ISX_REQUIRE(workspace != nullptr && workspace_bytes >= ISX_KNN_RANGE_WORKSPACE_BYTES,
+              "%s: workspace too small (%zu < %d)", fn, workspace_bytes, ISX_KNN_RANGE_WORKSPACE_BYTES);
+  if (!cont) ISX_CHECK_CUDA(cudaMemsetAsync(count, 0, sizeof(unsigned long long), stream));
+  if (n == 0) return ISX_OK;
+  ISX_REQUIRE(store && store_rnorm, "%s: null store pointer", fn);
+  int sms = 148;
+  int rc = device_sm_count(&sms);
+  if (rc != ISX_OK) return rc;
+  // the variant search() runs for k <= kSmallK at the same (q, d): same MMAs, same scaling, so a hit's
+  // score is bit for bit the one search() reports
+  const int ncta = (sms >= 2) ? knn_ncta(q) : 1;
+  const KnnPlan plan = plan_knn(n, q, kSmallK, sms, ncta);
+  CUtensorMap tq, te;
+  rc = encode_tmap_2d(&tq, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, queries, static_cast<uint64_t>(q),
+                      static_cast<uint64_t>(d), static_cast<uint64_t>(d) * 2, BM, BK, CU_TENSOR_MAP_SWIZZLE_128B);
+  if (rc != ISX_OK) return rc;
+  rc = encode_tmap_2d(&te, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, store, static_cast<uint64_t>(n),
+                      static_cast<uint64_t>(d), static_cast<uint64_t>(d) * 2, BN / ncta, BK, CU_TENSOR_MAP_SWIZZLE_128B);
+  if (rc != ISX_OK) return rc;
+
+  KnnParams p = {};
+  p.q = q; p.d = d; p.k = kSmallK; p.n = n;
+  p.mb = plan.mb; p.splits = plan.splits; p.nb = plan.nb; p.items = plan.items;
+  p.index_base = static_cast<int>(index_base);
+  p.self_base = no_self ? static_cast<int>(query_index_base) : -1;
+  p.store_rnorm = store_rnorm;
+  p.query_rnorm = query_rnorm;
+  p.progress = reinterpret_cast<uint32_t*>((reinterpret_cast<uintptr_t>(workspace) + 255) & ~uintptr_t(255));
+  p.range_tau = threshold;
+  p.range_rec = records;
+  p.range_cap = capacity;
+  p.range_count = count;
+  ISX_CHECK_CUDA(cudaMemsetAsync(p.progress, 0, 256 * sizeof(uint32_t), stream));
+#ifdef ISX_KNN_PROFILE
+  rc = set_profile(p, stream);
+  if (rc != ISX_OK) return rc;
+#endif
+  set_throttle(p, d);
+  static const bool no_res = [] { const char* e = getenv("ISX_KNN_RESIDENT"); return e && e[0] == '0'; }();
+  if (ncta == 2 && d <= 256 && !no_res) return launch_search<32, 2, true, false, true>(tq, te, p, plan.grid, stream);
+  if (ncta == 2) return launch_search<32, 2, false, false, true>(tq, te, p, plan.grid, stream);
+  return launch_search<32, 1, false, false, true>(tq, te, p, plan.grid, stream);
 }
 
 }  // extern "C"

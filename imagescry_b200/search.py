@@ -18,12 +18,22 @@ Several GPUs: ShardedEmbeddingStore — rows are split contiguously over the ran
 
 from __future__ import annotations
 
+import math
+import numbers
+
 import torch
 from torch import Tensor
 
 from imagescry_b200 import _lib
 
 MAX_K = 128
+# range search: a store's first call sizes its record buffer for RANGE_HITS_PER_QUERY hits per query,
+# later calls for the hits per query of the store's previous call of the same kind (search or graph)
+# plus RANGE_HEADROOM, never below RANGE_MIN_CAPACITY records; a call that overflows reruns once at its
+# exact count
+RANGE_HITS_PER_QUERY = 16
+RANGE_HEADROOM = 1.25
+RANGE_MIN_CAPACITY = 4096
 
 
 def shard_range(num_rows: int, world_size: int, rank: int) -> tuple[int, int]:
@@ -180,6 +190,79 @@ def gather_group_records(records: Tensor, group=None) -> Tensor:
     out = torch.empty((world * q, k, three), dtype=records.dtype, device=records.device)
     dist.all_gather_into_tensor(out, records.contiguous(), group=group)
     return out.view(world, q, k, three)
+
+
+def range_threshold(threshold) -> float:
+    """The range search's threshold as the fp32 value the kernel compares against (a finite float)."""
+    if isinstance(threshold, Tensor):
+        ok = threshold.numel() == 1 and threshold.dtype.is_floating_point
+    else:  # Python and numpy numbers; bool is a number to Python, not a threshold
+        ok = isinstance(threshold, numbers.Real) and not isinstance(threshold, bool)
+    if not ok:
+        raise ValueError(f"threshold must be a real number, got {threshold!r}")
+    t = float(torch.tensor(float(threshold), dtype=torch.float32))
+    if not math.isfinite(t):
+        raise ValueError(f"threshold must be finite in float32, got {threshold!r}")
+    return t
+
+
+def range_capacity(hits_per_query: float, num_queries: int) -> int:
+    """Record capacity of a range search's first run, from the expected hits per query."""
+    return max(RANGE_MIN_CAPACITY, math.ceil(hits_per_query * RANGE_HEADROOM * num_queries))
+
+
+def range_retry_capacity(count: int, capacity: int) -> int | None:
+    """The capacity of the one rerun a range search needs, or None: the hit set is deterministic, so a
+    rerun at exactly `count` records holds every hit."""
+    return count if count > capacity else None
+
+
+def range_empty(num_queries: int, device) -> tuple[Tensor, Tensor, Tensor]:
+    """CSR of a range search without hits: (offsets int64 Q + 1, indices int64 [0], scores fp32 [0])."""
+    return (torch.zeros(num_queries + 1, dtype=torch.int64, device=device), torch.empty(0, dtype=torch.int64, device=device),
+            torch.empty(0, dtype=torch.float32, device=device))
+
+
+def range_sort(records: Tensor, num_queries: int, hits: int) -> tuple[Tensor, Tensor, Tensor]:
+    """Ordering pass of a range search (`isx_knn_range_sort`): N×3 int32 records {query, row, score
+    bits} (row < 0 = padding) holding `hits` real records → CSR (offsets int64 Q + 1, indices int64,
+    scores fp32), each query's hits ordered by (score desc, row asc)."""
+    if records.ndim != 2 or records.shape[1] != 3 or records.dtype != torch.int32:
+        raise ValueError("records must be an N×3 int32 tensor")
+    _lib.require_cuda(records, "records")
+    dev = records.device
+    if num_queries == 0:
+        return range_empty(0, dev)
+    r = records.contiguous()
+    offsets = torch.empty(num_queries + 1, dtype=torch.int64, device=dev)
+    rows = torch.empty(hits, dtype=torch.int32, device=dev)
+    scores = torch.empty(hits, dtype=torch.float32, device=dev)
+    lib = _lib.load()
+    with torch.cuda.device(dev):
+        ws = torch.empty(max(int(lib.isx_knn_range_sort_workspace_bytes(r.shape[0], num_queries)), 256),
+                         dtype=torch.uint8, device=dev)
+    with _lib.on_device(r, offsets, ws) as stream:
+        rc = lib.isx_knn_range_sort(r.data_ptr(), r.shape[0], num_queries, offsets.data_ptr(), rows.data_ptr(),
+                                    scores.data_ptr(), ws.data_ptr(), ws.numel(), stream)
+    _lib.check(rc, "isx_knn_range_sort")
+    return offsets, rows.to(torch.int64), scores
+
+
+def gather_range_records(records: Tensor, count: int, group=None) -> tuple[Tensor, int]:
+    """All-gather every rank's first `count` range records (N×3 int32): one all-gather of the counts,
+    one of the records padded to the largest count with row = -1.  Returns (world·max×3, total hits)."""
+    import torch.distributed as dist
+
+    world = dist.get_world_size(group)
+    counts = torch.empty(world, dtype=torch.int64, device=records.device)
+    dist.all_gather_into_tensor(counts, torch.tensor([count], dtype=torch.int64, device=records.device), group=group)
+    counts = counts.tolist()
+    width = max(counts)
+    padded = torch.full((width, 3), -1, dtype=torch.int32, device=records.device)
+    padded[:count] = records[:count]
+    out = torch.empty((world * width, 3), dtype=torch.int32, device=records.device)
+    dist.all_gather_into_tensor(out, padded, group=group)
+    return out, sum(counts)
 
 
 def _as_bf16_matrix(x: Tensor, name: str) -> Tensor:
@@ -351,6 +434,68 @@ class EmbeddingStore:
         scores, rows, images = self.search_images_raw(queries, k)
         return scores, images.to(torch.int64), image_cells(rows, images, self.group_first_row)
 
+    def range_records(
+        self, q: Tensor, q_rnorm: Tensor, threshold: float, *, flags: int = 0, query_index_base: int = 0,
+        _capacity: int | None = None,
+    ) -> tuple[Tensor, int]:
+        """Unordered hits of a range search over this store for the prepared queries `q`: (N×3 int32
+        records {query, global row, score bits}, N).  The buffer is sized from the hits per query of
+        the store's previous call with the same flags; if the hits do not fit, the search runs once
+        more with exactly as many records."""
+        lib = _lib.load()
+        nq = q.shape[0]
+        hints = self.__dict__.setdefault("_range_hints", {})
+        cap = range_capacity(hints.get(flags, RANGE_HITS_PER_QUERY), nq) if _capacity is None else _capacity
+        count = torch.zeros(1, dtype=torch.int64, device=self.device)
+        with torch.cuda.device(self.device):
+            ws = self._ws(_lib.KNN_RANGE_WORKSPACE_BYTES)
+        while True:
+            records = torch.empty((cap, 3), dtype=torch.int32, device=self.device)
+            with _lib.on_device(self.embeddings, q, q_rnorm, records, count, ws) as stream:
+                rc = lib.isx_knn_range(
+                    self.embeddings.data_ptr(), self.rnorm.data_ptr(), len(self), q.data_ptr(), q_rnorm.data_ptr(), nq,
+                    q.shape[1], threshold, self.index_base, int(query_index_base), int(flags), records.data_ptr(), cap,
+                    count.data_ptr(), ws.data_ptr(), ws.numel(), stream,
+                )
+            _lib.check(rc, "isx_knn_range")
+            hits = int(count.item())
+            retry = range_retry_capacity(hits, cap)
+            if retry is None:
+                break
+            cap = retry
+        if nq:
+            hints[flags] = hits / nq
+        if cap > 2 * hits + RANGE_MIN_CAPACITY:
+            # a buffer sized for many more hits would stay allocated through the ordering pass
+            return records[:hits].clone(), hits
+        return records[:hits], hits
+
+    def search_range(self, queries: Tensor, threshold: float) -> tuple[Tensor, Tensor, Tensor]:
+        """Every store row whose cosine score with a query is >= `threshold` (rounded to float32), as CSR:
+        (offsets int64 Q + 1, indices int64 M, scores fp32 M).  Query i's hits are
+        indices[offsets[i]:offsets[i + 1]], ordered by (score desc, index asc); a score is bit for bit
+        what `search` reports for the pair, so the hits are the prefix of a long enough `search`
+        result whose scores are >= threshold."""
+        t = range_threshold(threshold)
+        q = self._queries(queries)
+        nq = q.shape[0]
+        if nq == 0 or len(self) == 0:
+            return range_empty(nq, self.device)
+        records, hits = self.range_records(q, row_rnorm(q), t)
+        return range_sort(records, nq, hits)
+
+    def range_graph(self, threshold: float) -> tuple[Tensor, Tensor, Tensor]:
+        """ε-graph of the store: every OTHER row whose cosine score with a row is >= `threshold`, as the
+        CSR of `search_range` with the store's own rows as queries (a row is never its own hit).  The
+        counterpart of `knn_graph` for a fixed similarity instead of a fixed count."""
+        t = range_threshold(threshold)
+        n = len(self)
+        if n == 0:
+            return range_empty(0, self.device)
+        records, hits = self.range_records(self.embeddings, self.rnorm, t, flags=_lib.KNN_EXCLUDE_SELF,
+                                           query_index_base=self.index_base)
+        return range_sort(records, n, hits)
+
     def knn_graph(self, k: int) -> tuple[Tensor, Tensor]:
         """All-pairs similarity graph (BASELINE.json config 5): the k nearest OTHER rows of every row,
         (scores N×k fp32, indices N×k int64).  One fused search with the store's own rows as queries;
@@ -456,6 +601,22 @@ class ShardedEmbeddingStore:
         s, r, g = self.local.search_images_raw(queries, k)
         merged_s, merged_r, merged_g = merge_topk_groups(gather_group_records(pack_group_records(s, r, g), self.group), k)
         return merged_s, merged_g.to(torch.int64), image_cells(merged_r, merged_g, self.local.group_first_row)
+
+    def search_range(self, queries: Tensor, threshold: float) -> tuple[Tensor, Tensor, Tensor]:
+        """`EmbeddingStore.search_range` over the sharded store: local range search with global rows, one
+        all-gather of the per-rank hit counts, one of the records padded to the largest count, one
+        ordering pass.  Every rank returns the same CSR."""
+        t = range_threshold(threshold)
+        q = self.local._queries(queries)
+        nq = q.shape[0]
+        if nq == 0:
+            return range_empty(0, self.local.device)
+        if len(self.local):
+            records, hits = self.local.range_records(q, row_rnorm(q), t)
+        else:
+            records, hits = torch.empty((0, 3), dtype=torch.int32, device=self.local.device), 0
+        gathered, total = gather_range_records(records, hits, self.group)
+        return range_sort(gathered, nq, total)
 
     # ------------------------------------------------------------------ gather over peer memory
     def _peer_buffers(self, nq: int, k: int):

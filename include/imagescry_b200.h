@@ -236,6 +236,32 @@ int isx_knn_search_grouped(const void* store, const float* store_rnorm, const in
 int isx_topk_merge_grouped(const int32_t* records, int g, int q, int k, float* out_scores,
                            int32_t* out_rows, int32_t* out_groups, isx_stream_t stream);
 
+/* Range search: every store row whose cosine score with a query is >= threshold (a finite float),
+ * the score being bit for bit the fp32 value isx_knn_search reports for that pair.  The selection is
+ * fused into the search kernel; hits are appended in no particular order to `records` as int32
+ * {query row (0..q-1), index_base + local row, fp32 score bits}, at most `capacity` of them, and
+ * `count` (device memory) receives the number of hits, also when it exceeds the capacity: a caller
+ * whose buffer was too small learns the exact size and runs again.  flags:
+ *   ISX_KNN_CONTINUE      do not zero `count`: this call appends the hits of another store block to
+ *                         the same buffer (same queries, same threshold);
+ *   ISX_KNN_EXCLUDE_SELF  as for the k-NN search: query row r is store row query_index_base + r and
+ *                         never its own hit.
+ * workspace: at least ISX_KNN_RANGE_WORKSPACE_BYTES of device memory. */
+#define ISX_KNN_RANGE_WORKSPACE_BYTES 2048
+int isx_knn_range(const void* store, const float* store_rnorm, int64_t n, const void* queries,
+                  const float* query_rnorm, int q, int d, float threshold, int64_t index_base,
+                  int64_t query_index_base, int flags, int32_t* records, int64_t capacity,
+                  unsigned long long* count, void* workspace, size_t workspace_bytes, isx_stream_t stream);
+/* Ordering pass of a range search: `total` records as above (rows < 0 are padding and are skipped,
+ * so the padded all-gather of several shards' records can be passed as it is) become CSR: offsets
+ * int64 q + 1, then the rows (int32) and scores (fp32) of query i at [offsets[i], offsets[i + 1]),
+ * ordered by (score desc, row asc).  rows and scores hold one entry per non-padding record.
+ * total < 2^31.  The workspace size depends on (total, q) only. */
+size_t isx_knn_range_sort_workspace_bytes(int64_t total, int q);
+int isx_knn_range_sort(const int32_t* records, int64_t total, int q, int64_t* offsets,
+                       int32_t* rows, float* scores, void* workspace, size_t workspace_bytes,
+                       isx_stream_t stream);
+
 /* ---- ROI masks on the feature-map grid (SURVEY.md 8f-4) ---------------------------------------
  * geometry.py:14-65 `create_roi_mask`: rasterio.features.rasterize(shapes, out_shape=(hf, wf),
  * transform=Affine.scale(w / wf, h / hf), fill=0, all_touched=True) * class_index.  rasterio / GDAL
