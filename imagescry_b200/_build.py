@@ -44,8 +44,14 @@ def sources() -> list[str]:
     return sorted(os.path.join(CSRC, f) for f in os.listdir(CSRC) if f.endswith(".cu"))
 
 
+def _extra_flags() -> list[str]:
+    # diagnostic builds only, e.g. ISX_NVCC_EXTRA="-DISX_KNN_PROFILE" python -m imagescry_b200._build --force
+    return os.environ.get("ISX_NVCC_EXTRA", "").split()
+
+
 def _digest() -> str:
-    h = hashlib.sha256()
+    # the flags are part of the digest: a library built with them is never taken for a plain build
+    h = hashlib.sha256(repr(_extra_flags()).encode())
     files = sources() + sorted(
         os.path.join(CSRC, f) for f in os.listdir(CSRC) if f.endswith((".cuh", ".h"))
     ) + [os.path.join(REPO, "include", "imagescry_b200.h"), os.path.abspath(__file__)]
@@ -70,8 +76,7 @@ def build(force: bool = False, verbose: bool = False) -> str:
     os.makedirs(OBJ_DIR, exist_ok=True)
     nvcc = _nvcc()
     extra = ["-Xptxas", "-v"] if verbose else []
-    # diagnostic builds only, e.g. ISX_NVCC_EXTRA="-DISX_KNN_PROFILE" python -m imagescry_b200._build --force
-    extra += os.environ.get("ISX_NVCC_EXTRA", "").split()
+    extra += _extra_flags()
 
     def compile_one(src: str) -> str:
         obj = os.path.join(OBJ_DIR, os.path.basename(src)[:-3] + ".o")

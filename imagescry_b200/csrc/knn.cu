@@ -53,12 +53,9 @@ constexpr int kEpilogueWarp0 = 4;
 // own partial list.  Two warps per scheduler halve the epilogue time per tile and hide each other's
 // TMEM / shared-memory latencies (d = 256: the epilogue, not the MMA, was the limiter with one group).
 // Large k (256-entry candidate buffers in global memory, long sorts) keeps one group: there the
-// second set of per-row lists costs more than the shorter fast path saves.
-#ifdef ISX_KNN_ONE_GROUP  // diagnostic A/B only (with the pipelined loads: d = 256 4.83 ms against 4.38, d = 64 4.57 against 3.64)
-__host__ __device__ constexpr int epi_groups(int) { return 1; }
-#else
+// second set of per-row lists costs more than the shorter fast path saves.  One group at small k
+// measured slower (with the pipelined loads: d = 256 4.83 ms against 4.38, d = 64 4.57 against 3.64).
 __host__ __device__ constexpr int epi_groups(int cap) { return cap <= 32 ? 2 : 1; }
-#endif
 __host__ __device__ constexpr int knn_threads(int cap) { return kEpilogueWarp0 * 32 + 128 * epi_groups(cap); }
 constexpr int kMaxK = 128;
 constexpr int kSmallK = 16;  // k <= kSmallK keeps candidate buffers in shared memory
@@ -74,7 +71,7 @@ struct KnnPlan {
 };
 
 // ncta = 2: CTA pairs (cta_group::2) — an M block is 256 queries and the schedulable units are SM pairs.
-KnnPlan plan_knn(long long n, int q, int k, int sms_total, int ncta) {
+KnnPlan plan_knn(long long n, int q, int sms_total, int ncta) {
   KnnPlan p;
   const int sms = std::max(1, sms_total / ncta);
   p.mb = (q + BM * ncta - 1) / (BM * ncta);
@@ -86,7 +83,6 @@ KnnPlan plan_knn(long long n, int q, int k, int sms_total, int ncta) {
   // (with the running lists) short items no longer buy better thresholds.
   int best_s = 1;
   double best_eff = -1.0;
-  (void)k;
   for (long long s = 1; s <= max_s; ++s) {
     const long long items = static_cast<long long>(p.mb) * s;
     const long long waves = (items + sms - 1) / sms;
@@ -97,9 +93,6 @@ KnnPlan plan_knn(long long n, int q, int k, int sms_total, int ncta) {
     if (eff > best_eff + 1e-9) { best_eff = eff; best_s = static_cast<int>(s); }
     if (eff >= 0.97) break;
   }
-  // ISX_KNN_SPLITS forces the split count (tuning / A-B measurements)
-  static const int forced = [] { const char* e = getenv("ISX_KNN_SPLITS"); return e ? atoi(e) : 0; }();
-  if (forced > 0) best_s = static_cast<int>(std::min<long long>(forced, max_s));
   p.splits = best_s;
   p.items = static_cast<long long>(p.mb) * p.splits;
   p.grid = static_cast<int>(std::min<long long>(sms, p.items)) * ncta;
@@ -714,7 +707,7 @@ __device__ __forceinline__ void knn_search_body(const CUtensorMap& tmap_q, const
       // every tile is then fetched from HBM once per query block.  Every kThrottleEvery tiles a unit
       // publishes how many tiles it has loaded and waits until the slowest unit is within
       // kThrottleWindow tiles (all units are co-resident: grid <= #SMs, one CTA per SM).  k = 100:
-      // DRAM reads 37.8 GB -> ~5 GB per pass, 23.5 -> 21 ms.  ISX_KNN_WINDOW overrides the window.
+      // DRAM reads 37.8 GB -> ~5 GB per pass, 23.5 -> 21 ms.
       // Units are normally co-resident (grid <= #SMs, one CTA per SM); the wait gives up after 2 ms.
       const uint32_t kThrottleEvery = p.throttle_every;  // a power of two
       const uint32_t kThrottleWindow = p.throttle_window;
@@ -1734,7 +1727,7 @@ int launch_search(const CUtensorMap& tq, const CUtensorMap& te, const KnnParams&
 // footprint in L2, so it scales with 1/d, and the poll interval (a third of it, rounded down to a
 // power of two) with it: one poll reads every unit's counter, ~1 us, against 0.6 us per tile at d = 256.
 void set_throttle(KnnParams& p, int d) {
-  const uint32_t base = getenv("ISX_KNN_WINDOW") ? static_cast<uint32_t>(atoi(getenv("ISX_KNN_WINDOW"))) : 24u;
+  constexpr uint32_t base = 24;
   const uint64_t scaled = static_cast<uint64_t>(base) * 1280u / static_cast<uint32_t>(std::max(d, 64));
   p.throttle_window = static_cast<uint32_t>(std::min<uint64_t>(std::max<uint64_t>(scaled, base), 1u << 30));
   uint32_t every = 8;
@@ -1756,15 +1749,77 @@ int set_profile(KnnParams& p, cudaStream_t stream) {
 #endif
 
 // CTA pairs halve the shared-memory fill and operand-read traffic per SM (each CTA stages half of
-// every store tile).  They need at least two 128-query blocks to pay off; ISX_KNN_CTA_PAIR=0/1
-// overrides the choice (for A/B measurements).
-int knn_ncta(int q) {
-  static const int forced = [] {
-    const char* e = getenv("ISX_KNN_CTA_PAIR");
-    return (e && (e[0] == '0' || e[0] == '1')) ? (e[0] - '0') : -1;
-  }();
-  if (forced >= 0) return forced ? 2 : 1;
-  return q > BM ? 2 : 1;
+// every store tile).  They need at least two 128-query blocks to pay off.
+int knn_ncta(int q) { return q > BM ? 2 : 1; }
+
+// Argument checks every search entry point (plain, grouped, range) makes.
+int check_search_args(const char* fn, const void* store, int64_t n, const void* queries, int q, int d,
+                      int64_t index_base, int64_t query_index_base, bool no_self) {
+  ISX_REQUIRE(d % 8 == 0, "%s: d = %d must be a multiple of 8 (16-byte rows for TMA)", fn, d);
+  ISX_REQUIRE(n < (1ll << 31) - BN, "%s: at most 2^31 store rows per call (n=%lld); shard the store", fn, (long long)n);
+  ISX_REQUIRE(index_base >= 0 && index_base + n < (1ll << 31), "%s: index_base + n must fit in int32", fn);
+  ISX_REQUIRE(!no_self || (query_index_base >= 0 && query_index_base + q < (1ll << 31)),
+              "%s: query_index_base + q must fit in int32 (got %lld)", fn, (long long)query_index_base);
+  ISX_REQUIRE((reinterpret_cast<uintptr_t>(queries) & 15u) == 0 && (reinterpret_cast<uintptr_t>(store) & 15u) == 0,
+              "%s: store and queries must be 16-byte aligned", fn);
+  return ISX_OK;
+}
+
+// What a search launch needs beyond its workspace: the variant's CTA count, the plan, the two tensor
+// maps and the parameters every entry point sets alike.
+struct KnnLaunch {
+  int ncta;
+  KnnPlan plan;
+  CUtensorMap tq, te;
+  KnnParams p;
+};
+
+// k is the length of the running lists (kSmallK for range search, which runs the k <= kSmallK variant).
+int prepare_search(KnnLaunch& L, const void* store, const float* store_rnorm, int64_t n, const void* queries,
+                   const float* query_rnorm, int q, int d, int k, int64_t index_base, int64_t query_index_base,
+                   bool no_self, int sms, cudaStream_t stream) {
+  L.ncta = (sms >= 2) ? knn_ncta(q) : 1;
+  L.plan = plan_knn(n, q, sms, L.ncta);
+  int rc = encode_tmap_2d(&L.tq, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, queries, static_cast<uint64_t>(q),
+                          static_cast<uint64_t>(d), static_cast<uint64_t>(d) * 2, BM, BK, CU_TENSOR_MAP_SWIZZLE_128B);
+  if (rc != ISX_OK) return rc;
+  rc = encode_tmap_2d(&L.te, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, store, static_cast<uint64_t>(n),
+                      static_cast<uint64_t>(d), static_cast<uint64_t>(d) * 2, BN / L.ncta, BK, CU_TENSOR_MAP_SWIZZLE_128B);
+  if (rc != ISX_OK) return rc;
+  KnnParams& p = L.p;
+  p = {};
+  p.q = q; p.d = d; p.k = k; p.n = n;
+  p.mb = L.plan.mb; p.splits = L.plan.splits; p.nb = L.plan.nb; p.items = L.plan.items;
+  p.index_base = static_cast<int>(index_base);
+  p.self_base = no_self ? static_cast<int>(query_index_base) : -1;
+  p.store_rnorm = store_rnorm;
+  p.query_rnorm = query_rnorm;
+  set_throttle(p, d);
+#ifdef ISX_KNN_PROFILE
+  rc = set_profile(p, stream);
+  if (rc != ISX_OK) return rc;
+#else
+  (void)stream;
+#endif
+  return ISX_OK;
+}
+
+// The one choice of kernel variant (CAP, NCTA, RES).  Plain, grouped and range search pick the same
+// variant for the same (q, d, k <= kSmallK): same MMA shapes, same scaling, so their scores are bit
+// for bit equal.
+template <bool GROUPED, bool RANGE>
+int launch_variant(const KnnLaunch& L, cudaStream_t stream) {
+  const KnnParams& p = L.p;
+  const int grid = L.plan.grid;
+  if constexpr (!RANGE) {
+    if (p.k > kSmallK)
+      return L.ncta == 2 ? launch_search<256, 2, false, GROUPED>(L.tq, L.te, p, grid, stream)
+                         : launch_search<256, 1, false, GROUPED>(L.tq, L.te, p, grid, stream);
+  }
+  if (L.ncta == 1) return launch_search<32, 1, false, GROUPED, RANGE>(L.tq, L.te, p, grid, stream);
+  // short rows, small k: the query tile stays resident
+  if (p.d <= 256) return launch_search<32, 2, true, GROUPED, RANGE>(L.tq, L.te, p, grid, stream);
+  return launch_search<32, 2, false, GROUPED, RANGE>(L.tq, L.te, p, grid, stream);
 }
 
 }  // namespace
@@ -1835,19 +1890,14 @@ static int knn_search_impl(const char* fn, const void* store, const float* store
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
   ISX_REQUIRE(q > 0 && d > 0 && k > 0 && n >= 0, "%s: need q, d, k > 0 and n >= 0 (q=%d d=%d k=%d n=%lld)", fn, q, d, k, (long long)n);
   ISX_REQUIRE(k <= kMaxK, "%s: k = %d exceeds the supported maximum of %d", fn, k, kMaxK);
-  ISX_REQUIRE(d % 8 == 0, "%s: d = %d must be a multiple of 8 (16-byte rows for TMA)", fn, d);
-  ISX_REQUIRE(n < (1ll << 31) - BN, "%s: at most 2^31 store rows per call (n=%lld); shard the store", fn, (long long)n);
-  ISX_REQUIRE(index_base >= 0 && index_base + n < (1ll << 31), "%s: index_base + n must fit in int32", fn);
+  int rc = check_search_args(fn, store, n, queries, q, d, index_base, query_index_base, no_self);
+  if (rc != ISX_OK) return rc;
   ISX_REQUIRE(queries && query_rnorm, "%s: null pointer", fn);
   ISX_REQUIRE(!finalize || peers || (out_scores && (packed || out_idx)), "%s: null output pointer", fn);
   ISX_REQUIRE(!grouped || (out_groups && flags == 0 && !peers), "%s: null output pointer", fn);
   ISX_REQUIRE(!grouped || n == 0 || row_group, "%s: null row_group pointer", fn);
-  ISX_REQUIRE(!no_self || (query_index_base >= 0 && query_index_base + q < (1ll << 31)),
-              "%s: query_index_base + q must fit in int32 (got %lld)", fn, (long long)query_index_base);
-  ISX_REQUIRE((reinterpret_cast<uintptr_t>(queries) & 15u) == 0 && (reinterpret_cast<uintptr_t>(store) & 15u) == 0,
-              "%s: store and queries must be 16-byte aligned", fn);
   int sms = 148;
-  int rc = device_sm_count(&sms);
+  rc = device_sm_count(&sms);
   if (rc != ISX_OK) return rc;
   const KnnWorkspace ws = knn_workspace(sms, q, k);
   ISX_REQUIRE(workspace != nullptr && workspace_bytes >= ws.total, "%s: workspace too small (%zu < %zu)", fn,
@@ -1870,24 +1920,11 @@ static int knn_search_impl(const char* fn, const void* store, const float* store
     return launch_merge(run_scores, run_idx, 1, q, k, query_rnorm, out_scores, packed ? nullptr : out_idx, stream, peers);
   }
   ISX_REQUIRE(store && store_rnorm, "%s: null store pointer", fn);
-  const int ncta = (sms >= 2) ? knn_ncta(q) : 1;
-  const KnnPlan plan = plan_knn(n, q, k, sms, ncta);
-
-  CUtensorMap tq, te;
-  rc = encode_tmap_2d(&tq, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, queries, static_cast<uint64_t>(q),
-                      static_cast<uint64_t>(d), static_cast<uint64_t>(d) * 2, BM, BK, CU_TENSOR_MAP_SWIZZLE_128B);
+  KnnLaunch L;
+  rc = prepare_search(L, store, store_rnorm, n, queries, query_rnorm, q, d, k, index_base, query_index_base, no_self,
+                      sms, stream);
   if (rc != ISX_OK) return rc;
-  rc = encode_tmap_2d(&te, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, store, static_cast<uint64_t>(n),
-                      static_cast<uint64_t>(d), static_cast<uint64_t>(d) * 2, BN / ncta, BK, CU_TENSOR_MAP_SWIZZLE_128B);
-  if (rc != ISX_OK) return rc;
-
-  KnnParams p;
-  p.q = q; p.d = d; p.k = k; p.n = n;
-  p.mb = plan.mb; p.splits = plan.splits; p.nb = plan.nb; p.items = plan.items;
-  p.index_base = static_cast<int>(index_base);
-  p.self_base = no_self ? static_cast<int>(query_index_base) : -1;
-  p.store_rnorm = store_rnorm;
-  p.query_rnorm = query_rnorm;
+  KnnParams& p = L.p;
   p.run_scores = run_scores;
   p.run_idx = run_idx;
   p.cand_global = reinterpret_cast<uint2*>(wbase + ws.cand_off);
@@ -1897,36 +1934,12 @@ static int knn_search_impl(const char* fn, const void* store, const float* store
   p.row_group = row_group;
   // a continued search keeps the lists and the bounds they imply; only the lockstep counters restart
   if (cont) ISX_CHECK_CUDA(cudaMemsetAsync(p.progress, 0, 256 * sizeof(uint32_t), stream));
-  set_throttle(p, d);
-
-#ifdef ISX_KNN_PROFILE
-  rc = set_profile(p, stream);
-  if (rc != ISX_OK) return rc;
-#endif
-  // the grouped search picks the same (CAP, NCTA, RES) variant as the plain one for the same (q, d, k):
-  // same MMA shapes, same scaling, bit-identical scores
-  static const bool no_res = [] { const char* e = getenv("ISX_KNN_RESIDENT"); return e && e[0] == '0'; }();
-  if (grouped) {
-    if (ncta == 2) {
-      if (k <= kSmallK && d <= 256 && !no_res) rc = launch_search<32, 2, true, true>(tq, te, p, plan.grid, stream);
-      else if (k <= kSmallK) rc = launch_search<32, 2, false, true>(tq, te, p, plan.grid, stream);
-      else rc = launch_search<256, 2, false, true>(tq, te, p, plan.grid, stream);
-    } else {
-      if (k <= kSmallK) rc = launch_search<32, 1, false, true>(tq, te, p, plan.grid, stream);
-      else rc = launch_search<256, 1, false, true>(tq, te, p, plan.grid, stream);
-    }
-  } else if (ncta == 2) {
-    // short rows, small k: the query tile stays resident (ISX_KNN_RESIDENT=0 switches it off)
-    if (k <= kSmallK && d <= 256 && !no_res) rc = launch_search<32, 2, true>(tq, te, p, plan.grid, stream);
-    else if (k <= kSmallK) rc = launch_search<32, 2>(tq, te, p, plan.grid, stream);
-    else rc = launch_search<256, 2>(tq, te, p, plan.grid, stream);
-  } else {
-    if (k <= kSmallK) rc = launch_search<32, 1>(tq, te, p, plan.grid, stream);
-    else rc = launch_search<256, 1>(tq, te, p, plan.grid, stream);
-  }
+  rc = grouped ? launch_variant<true, false>(L, stream) : launch_variant<false, false>(L, stream);
   if (rc != ISX_OK) return rc;
 #ifdef ISX_KNN_PROFILE
   {
+    const KnnPlan& plan = L.plan;
+    const int ncta = L.ncta;
     unsigned long long h[24];
     ISX_CHECK_CUDA(cudaStreamSynchronize(stream));
     ISX_CHECK_CUDA(cudaMemcpy(h, p.prof, sizeof(h), cudaMemcpyDeviceToHost));
@@ -2045,59 +2058,32 @@ int isx_knn_range(const void* store, const float* store_rnorm, int64_t n, const 
   ISX_REQUIRE((flags & ~(ISX_KNN_CONTINUE | ISX_KNN_EXCLUDE_SELF)) == 0, "%s: unknown flag bits 0x%x", fn, flags);
   ISX_REQUIRE(std::isfinite(threshold), "%s: the threshold must be finite (got %g)", fn, static_cast<double>(threshold));
   ISX_REQUIRE(q > 0 && d > 0 && n >= 0, "%s: need q, d > 0 and n >= 0 (q=%d d=%d n=%lld)", fn, q, d, (long long)n);
-  ISX_REQUIRE(d % 8 == 0, "%s: d = %d must be a multiple of 8 (16-byte rows for TMA)", fn, d);
-  ISX_REQUIRE(n < (1ll << 31) - BN, "%s: at most 2^31 store rows per call (n=%lld); shard the store", fn, (long long)n);
-  ISX_REQUIRE(index_base >= 0 && index_base + n < (1ll << 31), "%s: index_base + n must fit in int32", fn);
-  ISX_REQUIRE(!no_self || (query_index_base >= 0 && query_index_base + q < (1ll << 31)),
-              "%s: query_index_base + q must fit in int32 (got %lld)", fn, (long long)query_index_base);
+  int rc = check_search_args(fn, store, n, queries, q, d, index_base, query_index_base, no_self);
+  if (rc != ISX_OK) return rc;
   ISX_REQUIRE(capacity >= 0 && capacity < (1ll << 60), "%s: capacity out of range (%lld)", fn, (long long)capacity);
   ISX_REQUIRE(queries && query_rnorm && count && (capacity == 0 || records), "%s: null pointer", fn);
   ISX_REQUIRE((reinterpret_cast<uintptr_t>(records) & 3u) == 0 && (reinterpret_cast<uintptr_t>(count) & 7u) == 0,
               "%s: records must be 4-byte and count 8-byte aligned", fn);
-  ISX_REQUIRE((reinterpret_cast<uintptr_t>(queries) & 15u) == 0 && (reinterpret_cast<uintptr_t>(store) & 15u) == 0,
-              "%s: store and queries must be 16-byte aligned", fn);
   ISX_REQUIRE(workspace != nullptr && workspace_bytes >= ISX_KNN_RANGE_WORKSPACE_BYTES,
               "%s: workspace too small (%zu < %d)", fn, workspace_bytes, ISX_KNN_RANGE_WORKSPACE_BYTES);
   if (!cont) ISX_CHECK_CUDA(cudaMemsetAsync(count, 0, sizeof(unsigned long long), stream));
   if (n == 0) return ISX_OK;
   ISX_REQUIRE(store && store_rnorm, "%s: null store pointer", fn);
   int sms = 148;
-  int rc = device_sm_count(&sms);
+  rc = device_sm_count(&sms);
   if (rc != ISX_OK) return rc;
-  // the variant search() runs for k <= kSmallK at the same (q, d): same MMAs, same scaling, so a hit's
-  // score is bit for bit the one search() reports
-  const int ncta = (sms >= 2) ? knn_ncta(q) : 1;
-  const KnnPlan plan = plan_knn(n, q, kSmallK, sms, ncta);
-  CUtensorMap tq, te;
-  rc = encode_tmap_2d(&tq, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, queries, static_cast<uint64_t>(q),
-                      static_cast<uint64_t>(d), static_cast<uint64_t>(d) * 2, BM, BK, CU_TENSOR_MAP_SWIZZLE_128B);
+  KnnLaunch L;
+  rc = prepare_search(L, store, store_rnorm, n, queries, query_rnorm, q, d, kSmallK, index_base, query_index_base,
+                      no_self, sms, stream);
   if (rc != ISX_OK) return rc;
-  rc = encode_tmap_2d(&te, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, store, static_cast<uint64_t>(n),
-                      static_cast<uint64_t>(d), static_cast<uint64_t>(d) * 2, BN / ncta, BK, CU_TENSOR_MAP_SWIZZLE_128B);
-  if (rc != ISX_OK) return rc;
-
-  KnnParams p = {};
-  p.q = q; p.d = d; p.k = kSmallK; p.n = n;
-  p.mb = plan.mb; p.splits = plan.splits; p.nb = plan.nb; p.items = plan.items;
-  p.index_base = static_cast<int>(index_base);
-  p.self_base = no_self ? static_cast<int>(query_index_base) : -1;
-  p.store_rnorm = store_rnorm;
-  p.query_rnorm = query_rnorm;
+  KnnParams& p = L.p;
   p.progress = reinterpret_cast<uint32_t*>((reinterpret_cast<uintptr_t>(workspace) + 255) & ~uintptr_t(255));
   p.range_tau = threshold;
   p.range_rec = records;
   p.range_cap = capacity;
   p.range_count = count;
   ISX_CHECK_CUDA(cudaMemsetAsync(p.progress, 0, 256 * sizeof(uint32_t), stream));
-#ifdef ISX_KNN_PROFILE
-  rc = set_profile(p, stream);
-  if (rc != ISX_OK) return rc;
-#endif
-  set_throttle(p, d);
-  static const bool no_res = [] { const char* e = getenv("ISX_KNN_RESIDENT"); return e && e[0] == '0'; }();
-  if (ncta == 2 && d <= 256 && !no_res) return launch_search<32, 2, true, false, true>(tq, te, p, plan.grid, stream);
-  if (ncta == 2) return launch_search<32, 2, false, false, true>(tq, te, p, plan.grid, stream);
-  return launch_search<32, 1, false, false, true>(tq, te, p, plan.grid, stream);
+  return launch_variant<false, true>(L, stream);
 }
 
 }  // extern "C"

@@ -38,6 +38,18 @@ def test_library_exports_every_declared_symbol():
         assert re.search(rf"\bT {name}\b", nm), f"{name} is not an exported text symbol"
 
 
+def test_extra_nvcc_flags_are_part_of_the_build_digest(monkeypatch):
+    # a diagnostic library (e.g. -DISX_KNN_PROFILE) must never pass for the current plain build
+    from imagescry_b200 import _build
+
+    monkeypatch.delenv("ISX_NVCC_EXTRA", raising=False)
+    plain = _build._digest()
+    monkeypatch.setenv("ISX_NVCC_EXTRA", "-DISX_KNN_PROFILE")
+    assert _build._digest() != plain
+    monkeypatch.setenv("ISX_NVCC_EXTRA", "  ")
+    assert _build._digest() == plain
+
+
 def test_no_cpu_fallback():
     from imagescry_b200 import search
     from imagescry_b200.image import transforms as T

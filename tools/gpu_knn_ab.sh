@@ -1,29 +1,23 @@
 #!/bin/bash
-# A/B of a search-kernel variant selected by a macro: the shipped library against a rebuild with $1
-# (nvcc defines, e.g. -DISX_KNN_SMEM_PRUNE=0).  Both libraries are built first and every case
-# alternates shipped / variant / shipped / variant in fresh processes, so that the GPU's thermal
-# state (which moves these timings by several per cent) hits both alike.  The shipped library is
-# restored afterwards.  $2 = "notest" skips the knn tests on the shipped library.  If $1 is a file it
-# is taken as the prebuilt variant library (e.g. one built from an older commit in a git worktree).
+# A/B of the shipped library against prebuilt variant libraries: $1 is the path of a variant library,
+# or several separated by ';' (named variant0, variant1, ...).  The source has no tuning macros, so a
+# variant is a library built from another tree, e.g. the parent commit checked out in a git worktree
+# and built there with `python -m imagescry_b200._build`.  Every case alternates shipped / variant /
+# shipped / variant in fresh processes, so that the GPU's thermal state (which moves these timings by
+# several per cent) hits both alike.  The shipped library is restored afterwards.  $2 = "notest" skips
+# the knn tests on the shipped library.
 mkdir -p gpurun_out
 LIB=imagescry_b200/lib/libimagescry_b200.so
 cases=("knn --d 256 --k 10" "knn --d 64 --k 10" "knn --d 128 --k 16" "knn --d 1280 --k 10" "knn --d 256 --k 100" "graph --n 500000 --d 256 --k 10 --iters 3 --warm 1" "graph --n 131072 --d 256 --k 10")
 # ISX_AB_CASES="preprocess --case nhwc_f32 --batch 4096;preprocess --case nhwc_bf16 --batch 4096" overrides the list
 if [ -n "$ISX_AB_CASES" ]; then IFS=';' read -r -a cases <<< "$ISX_AB_CASES"; fi
+IFS=';' read -r -a variants <<< "$1"
+for v in "${variants[@]}"; do [ -f "$v" ] || { echo "no such library: $v"; exit 1; }; done
 cp $LIB /tmp/lib_shipped.so
 {
   if [ "$2" != "notest" ]; then timeout 900 python -m pytest tests/test_gpu_knn.py tests/test_gpu_guard_bands.py -x -q -m gpu 2>&1 | tail -2; fi
-  # several variants: separate their defines with ';' (e.g. "-DA=1;-DB=2"); names variant0, variant1, ...
   names=(shipped)
-  IFS=';' read -r -a defs <<< "$1"
-  if [ -f "${defs[0]}" ]; then
-    for i in "${!defs[@]}"; do cp "${defs[$i]}" /tmp/lib_variant$i.so; names+=(variant$i); echo "variant$i = ${defs[$i]}"; done
-  else
-    for i in "${!defs[@]}"; do
-      ISX_NVCC_EXTRA="${defs[$i]}" python -m imagescry_b200._build --force > gpurun_out/ab_build.log 2>&1 || { echo "build failed"; tail -20 gpurun_out/ab_build.log; }
-      cp $LIB /tmp/lib_variant$i.so; names+=(variant$i); echo "variant$i = ${defs[$i]}"
-    done
-  fi
+  for i in "${!variants[@]}"; do cp "${variants[$i]}" /tmp/lib_variant$i.so; names+=(variant$i); echo "variant$i = ${variants[$i]}"; done
   for args in "${cases[@]}"; do
     for rep in 1 2; do
       for which in "${names[@]}"; do
