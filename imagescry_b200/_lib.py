@@ -108,7 +108,18 @@ SIGNATURES: dict[str, tuple] = {
     "isx_knn_range_sort": (
         c_int, [c_void_p, c_int64, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]
     ),
-    "isx_roi_rasterize": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int64, c_void_p, c_void_p]),
+    "isx_quantize_rows_e4m3": (c_int, [c_void_p, c_int64, c_int, c_int, c_void_p, c_void_p, c_void_p]),
+    "isx_knn_search_fp8": (
+        c_int,
+        [c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_int, c_int, c_int, c_int64, c_void_p, c_void_p, c_void_p,
+         c_size_t, c_void_p],
+    ),
+    "isx_knn_rescore": (
+        c_int,
+        [c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_int, c_int, c_void_p, c_int, c_int64, c_int, c_void_p,
+         c_void_p, c_void_p],
+    ),
+    "isx_roi_rasterize":(c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int64, c_void_p, c_void_p]),
     "isx_masked_pool": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_int, c_int64, c_void_p, c_void_p]),
 }
 

@@ -339,6 +339,39 @@ __device__ __forceinline__ void tc_mma_f16_pair(uint32_t d_tmem, uint64_t a_desc
       : "memory");
 }
 
+// kind::f8f6f4: 8-bit float operands (K = 32 elements = 32 bytes per instruction), fp32 accumulation.
+// In its instruction descriptor the A / B format 0 is E4M3 (make_idesc(0, m, n)).
+__device__ __forceinline__ void tc_mma_f8(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc,
+                                          uint32_t idesc, uint32_t accumulate) {
+  asm volatile(
+      "{\n\t"
+      ".reg .pred p;\n\t"
+      "setp.ne.b32 p, %4, 0;\n\t"
+      "tcgen05.mma.cta_group::1.kind::f8f6f4 [%0], %1, %2, %3, p;\n\t"
+      "}\n" ::"r"(d_tmem),
+      "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate)
+      : "memory");
+}
+__device__ __forceinline__ void tc_mma_f8_pair(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc,
+                                               uint32_t idesc, uint32_t accumulate) {
+  asm volatile(
+      "{\n\t"
+      ".reg .pred p;\n\t"
+      "setp.ne.b32 p, %4, 0;\n\t"
+      "tcgen05.mma.cta_group::2.kind::f8f6f4 [%0], %1, %2, %3, p;\n\t"
+      "}\n" ::"r"(d_tmem),
+      "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate)
+      : "memory");
+}
+
+// Two fp32 -> two E4M3 bytes (round to nearest even, saturating to +-448): `lo` goes to the lower
+// address of the returned little-endian pair.
+__device__ __forceinline__ uint16_t cvt_e4m3x2(float lo, float hi) {
+  uint16_t r;
+  asm("cvt.rn.satfinite.e4m3x2.f32 %0, %1, %2;" : "=h"(r) : "f"(hi), "f"(lo));
+  return r;
+}
+
 // A operand in tensor memory ("TS" form): D[tmem] (+)= A[tmem] * B[smem].  A is M x K with row m on
 // TMEM lane m and two consecutive 16-bit K elements per 32-bit column (K = 16 -> 8 columns).
 __device__ __forceinline__ void tc_mma_f16_pair_ts(uint32_t d_tmem, uint32_t a_tmem, uint64_t b_desc,
@@ -375,8 +408,9 @@ __device__ __forceinline__ uint64_t make_kmajor_sw128_desc(uint32_t smem_addr) {
   return desc;
 }
 
-// Instruction descriptor for tcgen05.mma kind::f16 / kind::tf32, dense, fp32 accumulate,
-// both operands K-major.  ab_format: 0 = f16, 1 = bf16, 2 = tf32.
+// Instruction descriptor for tcgen05.mma kind::f16 / kind::tf32 / kind::f8f6f4, dense, fp32
+// accumulate, both operands K-major.  ab_format: 0 = f16, 1 = bf16, 2 = tf32; under kind::f8f6f4
+// 0 = e4m3.
 __host__ __device__ constexpr uint32_t make_idesc(uint32_t ab_format, uint32_t m, uint32_t n) {
   return (1u << 4) |                // D format: f32
          (ab_format << 7) |         // A format

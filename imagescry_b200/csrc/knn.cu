@@ -7,6 +7,9 @@
 //   K5  topk_merge_kernel  finalises K4's running lists (scale by the queries' inverse norms, rebase
 //                          the rows — as two arrays, packed records, or packed records stored into every
 //                          peer's gather buffer over NVLink) and merges the partial lists of several GPUs.
+//   fp8 search (isx_knn_search_fp8): K0q quantize_e4m3_kernel writes an E4M3 copy of the rows and its
+//   inverse norms, K4 in its fp8 form (knn_search_fp8_kernel: the same body with kind::f8f6f4 MMAs
+//   over 128-element k-blocks) picks candidates, K5r rescore_kernel re-scores them from the bf16 rows.
 //
 // There is no reference implementation of this stage (SURVEY.md §0.2); semantics follow
 // oracle/oracle.py::cosine_knn: normalize(q) . normalize(e) with F.normalize's eps
@@ -131,6 +134,100 @@ row_rnorm_kernel(const __nv_bfloat16* __restrict__ x, long long n, int d, float 
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) ss += __shfl_xor_sync(kFullMask, ss, o);
     if (lane == 0) rnorm[row] = 1.0f / fmaxf(sqrtf(ss), eps);
+  }
+}
+
+// ------------------------------------------------------------------------------------------
+// K0q: E4M3 copy of bf16 rows for the fp8 scan.  One warp per row:
+//   1. m = max |x|; the row is scaled by the power of two 2^e that puts m in (224, 448] (exact, and a
+//      cosine does not see it), so every row uses the format's full range whatever its norm;
+//   2. round to nearest even into E4M3 (cvt.rn.satfinite), zero-pad to d16 bytes (16-byte TMA rows);
+//   3. rnorm = 1 / max(||q||, eps) of the E4M3 values q themselves.  Their squares are exact and their
+//      sum is exact in fp64 (every q^2 is a multiple of 2^-18 below 2^18), so the norm is the correctly
+//      rounded one, whatever the summation order.
+// The fp8 scan therefore ranks by the exact cosine of the quantized rows, up to the fp32 accumulation
+// of the tensor cores; rows that are power-of-two multiples of each other get identical bytes.  A zero
+// row stays zero (e = 0) and gets 1 / eps, as in row_rnorm_kernel.
+// ------------------------------------------------------------------------------------------
+constexpr float kRnormEps = 1e-12f;  // F.normalize's eps, the value row_rnorm is called with
+
+// exponent e with 224 < m * 2^e <= 448 for finite m > 0 (0 otherwise)
+__device__ __forceinline__ int e4m3_row_exponent(float m) {
+  if (!(m > 0.f) || isinf(m)) return 0;
+  int ex;
+  const float f = frexpf(m, &ex);  // m = f * 2^ex, f in [0.5, 1): 2f is m's significand
+  return (f > 0.875f) ? 8 - ex : 9 - ex;
+}
+
+// value of a finite E4M3 byte (sign, 4 exponent bits with bias 7, 3 mantissa bits)
+__device__ __forceinline__ float e4m3_to_f32(uint32_t b) {
+  const uint32_t ex = (b >> 3) & 15u, man = b & 7u;
+  const float mag = ex ? __uint_as_float(((ex + 120u) << 23) | (man << 20)) : static_cast<float>(man) * 0.001953125f;
+  return (b & 0x80u) ? -mag : mag;
+}
+
+__global__ void __launch_bounds__(256)
+quantize_e4m3_kernel(const __nv_bfloat16* __restrict__ x, long long n, int d, int d16, uint8_t* __restrict__ out,
+                     float* __restrict__ rnorm) {
+  const int lane = threadIdx.x & 31;
+  const long long warps = (static_cast<long long>(gridDim.x) * blockDim.x) >> 5;
+  const bool vec = (d & 7) == 0 && (reinterpret_cast<uintptr_t>(x) & 15u) == 0;
+  for (long long row = (static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x) >> 5; row < n;
+       row += warps) {
+    const __nv_bfloat16* p = x + row * d;
+    uint8_t* o = out + row * d16;
+    float m = 0.f;
+    if (vec) {
+      for (int i = lane * 8; i < d; i += 256) {
+        const uint4 v = ld_nc_v4(p + i);
+        const uint32_t w[4] = {v.x, v.y, v.z, v.w};
+#pragma unroll
+        for (int j = 0; j < 4; ++j) m = fmaxf(m, fmaxf(fabsf(__uint_as_float(w[j] << 16)), fabsf(__uint_as_float(w[j] & 0xFFFF0000u))));
+      }
+    } else {
+      for (int i = lane; i < d; i += 32) m = fmaxf(m, fabsf(__bfloat162float(p[i])));
+    }
+#pragma unroll
+    for (int o2 = 16; o2 > 0; o2 >>= 1) m = fmaxf(m, __shfl_xor_sync(kFullMask, m, o2));
+    // 2^e in two factors (e reaches 157 for the smallest bf16 subnormals): each product is exact for
+    // every element that does not end far below E4M3's smallest subnormal
+    const int e = e4m3_row_exponent(m);
+    const int e1 = e / 2;
+    const float s1 = __int_as_float((127 + e1) << 23), s2 = __int_as_float((127 + e - e1) << 23);
+    double ss = 0.0;
+    auto quant2 = [&](float a, float b) -> uint16_t {
+      const uint16_t r = cvt_e4m3x2(__fmul_rn(__fmul_rn(a, s1), s2), __fmul_rn(__fmul_rn(b, s1), s2));
+      const double qa = e4m3_to_f32(r & 0xFFu), qb = e4m3_to_f32(r >> 8);
+      ss = fma(qa, qa, ss);
+      ss = fma(qb, qb, ss);
+      return r;
+    };
+    if (vec) {
+      // 8 elements (one 16-byte load, one 8-byte store) per lane and step; d % 8 == 0 and d16 % 16 == 0,
+      // so a step is either all data or all padding
+      for (int i = lane * 8; i < d16; i += 256) {
+        uint4 v = make_uint4(0u, 0u, 0u, 0u);
+        if (i < d) v = ld_nc_v4(p + i);
+        const uint32_t w[4] = {v.x, v.y, v.z, v.w};
+        uint32_t b[2];
+#pragma unroll
+        for (int j = 0; j < 2; ++j) {
+          const uint16_t lo = quant2(__uint_as_float(w[2 * j] << 16), __uint_as_float(w[2 * j] & 0xFFFF0000u));
+          const uint16_t hi = quant2(__uint_as_float(w[2 * j + 1] << 16), __uint_as_float(w[2 * j + 1] & 0xFFFF0000u));
+          b[j] = static_cast<uint32_t>(lo) | (static_cast<uint32_t>(hi) << 16);
+        }
+        *reinterpret_cast<uint2*>(o + i) = make_uint2(b[0], b[1]);
+      }
+    } else {
+      for (int i = lane * 2; i < d16; i += 64) {
+        const float a = i < d ? __bfloat162float(p[i]) : 0.f;
+        const float b = i + 1 < d ? __bfloat162float(p[i + 1]) : 0.f;
+        *reinterpret_cast<uint16_t*>(o + i) = quant2(a, b);
+      }
+    }
+#pragma unroll
+    for (int o2 = 16; o2 > 0; o2 >>= 1) ss += __shfl_xor_sync(kFullMask, ss, o2);
+    if (lane == 0) rnorm[row] = 1.0f / fmaxf(__double2float_rn(sqrt(ss)), kRnormEps);
   }
 }
 
@@ -637,8 +734,14 @@ __device__ __forceinline__ void range_append(const uint32_t (&r)[32], bool pass,
 // before the first tile, so the epilogue keeps the fast path and replaces the rest: no candidate
 // buffers, prunes, shared bound or item end; the rare path tests every column of the chunk exactly
 // and appends the hits to a global record buffer (range_append).
-template <int CAP, int NCTA, bool RES, bool GROUPED, bool RANGE = false>
+//
+// F8: the operands are E4M3 rows (knn_search_fp8_kernel).  The producer moves them as 16-bit pairs
+// (p.d = d16 / 2, tensor maps of UINT16), so a k-block is still one 128-byte swizzle row of BK units,
+// now 128 elements: the ring, the TMA boxes, the descriptors and their 32-byte step per MMA (K = 32
+// under kind::f8f6f4) and the whole epilogue are those of the bf16 kernel; only the MMA kind changes.
+template <int CAP, int NCTA, bool RES, bool GROUPED, bool RANGE = false, bool F8 = false>
 __device__ __forceinline__ void knn_search_body(const CUtensorMap& tmap_q, const CUtensorMap& tmap_e, const KnnParams& p) {
+  static_assert(!F8 || (!GROUPED && !RANGE), "the fp8 scan is a plain search");
   using L = KnnSmem<CAP, NCTA, RES, GROUPED, RANGE>;
   constexpr int STAGES = L::STAGES;
   constexpr int kEpiGroups = L::G;
@@ -784,7 +887,7 @@ __device__ __forceinline__ void knn_search_body(const CUtensorMap& tmap_q, const
   } else if (warp == 1) {
     // ===================== MMA issuer =====================
     if (lane == 0 && rank == 0) {
-      constexpr uint32_t idesc = make_idesc(/*bf16*/ 1, BM * NCTA, BN);
+      constexpr uint32_t idesc = make_idesc(F8 ? 0 /*e4m3*/ : 1 /*bf16*/, BM * NCTA, BN);
       uint32_t stage = 0, phase = 0, acc = 0, acc_phase = 0, item_no = 0;
       for (long long item = unit; item < p.items; item += num_units) {
         const int split = static_cast<int>(item / p.mb);
@@ -811,8 +914,13 @@ __device__ __forceinline__ void knn_search_body(const CUtensorMap& tmap_q, const
             for (int k = 0; k < BK / UMMA_K; ++k) {
               const uint64_t a_desc = make_kmajor_sw128_desc(a_addr + k * UMMA_K * 2);
               const uint64_t b_desc = make_kmajor_sw128_desc(b_addr + k * UMMA_K * 2);
-              if (NCTA == 2) tc_mma_f16_pair(d_tmem, a_desc, b_desc, idesc, (kb | k) != 0);
-              else tc_mma_f16(d_tmem, a_desc, b_desc, idesc, (kb | k) != 0);
+              if constexpr (F8) {
+                if (NCTA == 2) tc_mma_f8_pair(d_tmem, a_desc, b_desc, idesc, (kb | k) != 0);
+                else tc_mma_f8(d_tmem, a_desc, b_desc, idesc, (kb | k) != 0);
+              } else {
+                if (NCTA == 2) tc_mma_f16_pair(d_tmem, a_desc, b_desc, idesc, (kb | k) != 0);
+                else tc_mma_f16(d_tmem, a_desc, b_desc, idesc, (kb | k) != 0);
+              }
             }
             // frees the smem slot (in both CTAs of a pair) once these MMAs have read it
             if (NCTA == 2) tc_commit_pair(&empty_bar[stage]); else tc_commit(&empty_bar[stage]);
@@ -1505,6 +1613,13 @@ knn_range_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_consta
   knn_search_body<32, NCTA, RES, false, true>(tmap_q, tmap_e, p);
 }
 
+template <int CAP, int NCTA, bool RES>
+__global__ void __launch_bounds__(knn_threads(CAP), 1)
+knn_search_fp8_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_constant__ CUtensorMap tmap_e,
+                      const KnnParams p) {
+  knn_search_body<CAP, NCTA, RES, false, false, true>(tmap_q, tmap_e, p);
+}
+
 // ------------------------------------------------------------------------------------------
 // K5: merge g sorted-or-not partial lists per query into the final top-k.  One warp per query.
 // ------------------------------------------------------------------------------------------
@@ -1676,6 +1791,94 @@ int launch_merge_grouped(const int32_t* records, const float* scores, const int3
   return ISX_OK;
 }
 
+// ------------------------------------------------------------------------------------------
+// K5r: exact re-score of candidate lists (the second stage of the fp8 search).  One warp per query:
+// every candidate row (global; -1 and rows outside the store are skipped) gets the bf16 dot product
+// in fp32 — each lane sums its 8-element slices in a fixed order, then a butterfly, so every lane
+// holds the same bits — and score = fl(fl(dot * rnorm_e) * rnorm_q), the epilogue's and K5's product
+// order.  The best k by (score desc, row asc) are written, padded with (-inf, -1); a row listed twice
+// comes out once.  Nothing depends on timing: repeated calls give identical bits.
+// ------------------------------------------------------------------------------------------
+template <int E>
+__global__ void __launch_bounds__(128)
+rescore_kernel(const __nv_bfloat16* __restrict__ store, const float* __restrict__ rnorm, long long n,
+               const __nv_bfloat16* __restrict__ queries, const float* __restrict__ qrnorm, int q, int d,
+               const int32_t* __restrict__ cand, int kc, int index_base, int k, float* __restrict__ out_scores,
+               int32_t* __restrict__ out_idx) {
+  const int lane = threadIdx.x & 31;
+  const int query = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  if (query >= q) return;
+  const __nv_bfloat16* qp = queries + static_cast<size_t>(query) * d;
+  const float rq = qrnorm[query];
+  float s[E];
+  int id[E];
+#pragma unroll
+  for (int e = 0; e < E; ++e) {
+    s[e] = -INFINITY;
+    id[e] = INT_MAX;
+    const int j0 = e * 32;
+    const int mine = (j0 + lane < kc) ? cand[static_cast<size_t>(query) * kc + j0 + lane] : -1;
+    const int cnt = min(32, kc - j0);
+#pragma unroll 1
+    for (int l = 0; l < cnt; ++l) {
+      const int r = __shfl_sync(kFullMask, mine, l);
+      const long long local = static_cast<long long>(r) - index_base;
+      if (r < 0 || local < 0 || local >= n) continue;  // warp-uniform
+      const __nv_bfloat16* ep = store + local * d;
+      float acc = 0.f;
+#pragma unroll 4
+      for (int i = lane * 8; i < d; i += 256) {
+        const uint4 a = ld_nc_v4(ep + i), b = ld_nc_v4(qp + i);
+        const uint32_t wa[4] = {a.x, a.y, a.z, a.w}, wb[4] = {b.x, b.y, b.z, b.w};
+#pragma unroll
+        for (int j = 0; j < 4; ++j) {
+          acc = fmaf(__uint_as_float(wa[j] << 16), __uint_as_float(wb[j] << 16), acc);
+          acc = fmaf(__uint_as_float(wa[j] & 0xFFFF0000u), __uint_as_float(wb[j] & 0xFFFF0000u), acc);
+        }
+      }
+#pragma unroll
+      for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(kFullMask, acc, o);
+      if (lane == l) {
+        s[e] = __fmul_rn(__fmul_rn(acc, __ldg(rnorm + local)), rq);
+        id[e] = r;
+      }
+    }
+  }
+  warp_sort_desc<E>(s, id);
+  // a row listed twice sorts next to its copy: drop the later one and sort again (rare)
+  bool dup[E];
+  bool any = false;
+  int carry = INT_MAX;  // row of element e * 32 - 1
+#pragma unroll
+  for (int e = 0; e < E; ++e) {
+    const int up = __shfl_up_sync(kFullMask, id[e], 1);
+    const int prev = lane ? up : carry;
+    carry = __shfl_sync(kFullMask, id[e], 31);
+    dup[e] = id[e] != INT_MAX && id[e] == prev;
+    any |= dup[e];
+  }
+  if (__any_sync(kFullMask, any)) {
+#pragma unroll
+    for (int e = 0; e < E; ++e) {
+      if (dup[e]) { s[e] = -INFINITY; id[e] = INT_MAX; }
+    }
+    warp_sort_desc<E>(s, id);
+  }
+#pragma unroll
+  for (int e = 0; e < E; ++e) {
+    const int pos = e * 32 + lane;
+    if (pos < k) {
+      const bool have = id[e] != INT_MAX;
+      out_scores[static_cast<size_t>(query) * k + pos] = have ? s[e] : -INFINITY;
+      out_idx[static_cast<size_t>(query) * k + pos] = have ? id[e] : -1;
+    }
+  }
+  for (int pos = 32 * E + lane; pos < k; pos += 32) {
+    out_scores[static_cast<size_t>(query) * k + pos] = -INFINITY;
+    out_idx[static_cast<size_t>(query) * k + pos] = -1;
+  }
+}
+
 size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
 struct KnnWorkspace {
@@ -1700,11 +1903,13 @@ KnnWorkspace knn_workspace(int max_grid, int q, int k) {
   return w;
 }
 
-template <int CAP, int NCTA, bool RES = false, bool GROUPED = false, bool RANGE = false>
+template <int CAP, int NCTA, bool RES = false, bool GROUPED = false, bool RANGE = false, bool F8 = false>
 int launch_search(const CUtensorMap& tq, const CUtensorMap& te, const KnnParams& p, int grid, cudaStream_t stream) {
   static_assert(!RANGE || (CAP == 32 && !GROUPED), "range search has the CAP = 32 plan only");
-  auto kern = RANGE ? knn_range_kernel<NCTA, RES>
-                    : GROUPED ? knn_search_grouped_kernel<CAP, NCTA, RES> : knn_search_kernel<CAP, NCTA, RES>;
+  static_assert(!F8 || (!GROUPED && !RANGE), "the fp8 scan is a plain search");
+  auto kern = F8 ? knn_search_fp8_kernel<CAP, NCTA, RES>
+                 : RANGE ? knn_range_kernel<NCTA, RES>
+                         : GROUPED ? knn_search_grouped_kernel<CAP, NCTA, RES> : knn_search_kernel<CAP, NCTA, RES>;
   const int smem = static_cast<int>(KnnSmem<CAP, NCTA, RES, GROUPED, RANGE>::kDynamicBytes);
   ISX_CHECK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
   cudaLaunchConfig_t cfg = {};
@@ -1723,12 +1928,13 @@ int launch_search(const CUtensorMap& tq, const CUtensorMap& te, const KnnParams&
   return ISX_OK;
 }
 
-// Lockstep window in tiles: measured best 16-32 at d = 1280 (640 KB of store rows per tile); it is a
-// footprint in L2, so it scales with 1/d, and the poll interval (a third of it, rounded down to a
-// power of two) with it: one poll reads every unit's counter, ~1 us, against 0.6 us per tile at d = 256.
-void set_throttle(KnnParams& p, int d) {
+// Lockstep window in tiles: measured best 16-32 at bf16 d = 1280 (640 KB of store rows per tile); it is
+// a footprint in L2, so it scales with 1 / row bytes, and the poll interval (a third of it, rounded down
+// to a power of two) with it: one poll reads every unit's counter, ~1 us, against 0.6 us per tile at
+// bf16 d = 256.
+void set_throttle(KnnParams& p, int row_bytes) {
   constexpr uint32_t base = 24;
-  const uint64_t scaled = static_cast<uint64_t>(base) * 1280u / static_cast<uint32_t>(std::max(d, 64));
+  const uint64_t scaled = static_cast<uint64_t>(base) * 2560u / static_cast<uint32_t>(std::max(row_bytes, 128));
   p.throttle_window = static_cast<uint32_t>(std::min<uint64_t>(std::max<uint64_t>(scaled, base), 1u << 30));
   uint32_t every = 8;
   while (every * 2 <= p.throttle_window / 3 && every < 1024) every *= 2;
@@ -1775,15 +1981,18 @@ struct KnnLaunch {
 };
 
 // k is the length of the running lists (kSmallK for range search, which runs the k <= kSmallK variant).
+// dtype: BFLOAT16 for bf16 rows; UINT16 for the fp8 scan, whose E4M3 rows are moved as 16-bit pairs
+// (d = d16 / 2) so that a box row is 128 bytes in both.
 int prepare_search(KnnLaunch& L, const void* store, const float* store_rnorm, int64_t n, const void* queries,
                    const float* query_rnorm, int q, int d, int k, int64_t index_base, int64_t query_index_base,
-                   bool no_self, int sms, cudaStream_t stream) {
+                   bool no_self, int sms, cudaStream_t stream,
+                   CUtensorMapDataType dtype = CU_TENSOR_MAP_DATA_TYPE_BFLOAT16) {
   L.ncta = (sms >= 2) ? knn_ncta(q) : 1;
   L.plan = plan_knn(n, q, sms, L.ncta);
-  int rc = encode_tmap_2d(&L.tq, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, queries, static_cast<uint64_t>(q),
+  int rc = encode_tmap_2d(&L.tq, dtype, 2, queries, static_cast<uint64_t>(q),
                           static_cast<uint64_t>(d), static_cast<uint64_t>(d) * 2, BM, BK, CU_TENSOR_MAP_SWIZZLE_128B);
   if (rc != ISX_OK) return rc;
-  rc = encode_tmap_2d(&L.te, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, store, static_cast<uint64_t>(n),
+  rc = encode_tmap_2d(&L.te, dtype, 2, store, static_cast<uint64_t>(n),
                       static_cast<uint64_t>(d), static_cast<uint64_t>(d) * 2, BN / L.ncta, BK, CU_TENSOR_MAP_SWIZZLE_128B);
   if (rc != ISX_OK) return rc;
   KnnParams& p = L.p;
@@ -1794,7 +2003,7 @@ int prepare_search(KnnLaunch& L, const void* store, const float* store_rnorm, in
   p.self_base = no_self ? static_cast<int>(query_index_base) : -1;
   p.store_rnorm = store_rnorm;
   p.query_rnorm = query_rnorm;
-  set_throttle(p, d);
+  set_throttle(p, 2 * d);
 #ifdef ISX_KNN_PROFILE
   rc = set_profile(p, stream);
   if (rc != ISX_OK) return rc;
@@ -1806,20 +2015,20 @@ int prepare_search(KnnLaunch& L, const void* store, const float* store_rnorm, in
 
 // The one choice of kernel variant (CAP, NCTA, RES).  Plain, grouped and range search pick the same
 // variant for the same (q, d, k <= kSmallK): same MMA shapes, same scaling, so their scores are bit
-// for bit equal.
-template <bool GROUPED, bool RANGE>
+// for bit equal.  F8 (the E4M3 scan, p.d in 16-bit pairs) follows the same rules.
+template <bool GROUPED, bool RANGE, bool F8 = false>
 int launch_variant(const KnnLaunch& L, cudaStream_t stream) {
   const KnnParams& p = L.p;
   const int grid = L.plan.grid;
   if constexpr (!RANGE) {
     if (p.k > kSmallK)
-      return L.ncta == 2 ? launch_search<256, 2, false, GROUPED>(L.tq, L.te, p, grid, stream)
-                         : launch_search<256, 1, false, GROUPED>(L.tq, L.te, p, grid, stream);
+      return L.ncta == 2 ? launch_search<256, 2, false, GROUPED, false, F8>(L.tq, L.te, p, grid, stream)
+                         : launch_search<256, 1, false, GROUPED, false, F8>(L.tq, L.te, p, grid, stream);
   }
-  if (L.ncta == 1) return launch_search<32, 1, false, GROUPED, RANGE>(L.tq, L.te, p, grid, stream);
-  // short rows, small k: the query tile stays resident
-  if (p.d <= 256) return launch_search<32, 2, true, GROUPED, RANGE>(L.tq, L.te, p, grid, stream);
-  return launch_search<32, 2, false, GROUPED, RANGE>(L.tq, L.te, p, grid, stream);
+  if (L.ncta == 1) return launch_search<32, 1, false, GROUPED, RANGE, F8>(L.tq, L.te, p, grid, stream);
+  // short rows (at most 512 bytes: the resident tile's 4 k-blocks), small k: the query tile stays resident
+  if (p.d <= 256) return launch_search<32, 2, true, GROUPED, RANGE, F8>(L.tq, L.te, p, grid, stream);
+  return launch_search<32, 2, false, GROUPED, RANGE, F8>(L.tq, L.te, p, grid, stream);
 }
 
 }  // namespace
@@ -1880,8 +2089,9 @@ static int knn_search_impl(const char* fn, const void* store, const float* store
                            const float* query_rnorm, int q, int d, int k, int64_t index_base,
                            int64_t query_index_base, int flags, float* out_scores, int32_t* out_idx,
                            void* workspace, size_t workspace_bytes, isx_stream_t stream_, const PeerOut* peers,
-                           const int32_t* row_group = nullptr, int32_t* out_groups = nullptr) {
+                           const int32_t* row_group = nullptr, int32_t* out_groups = nullptr, bool f8 = false) {
   // row_group != nullptr: grouped search (isx_knn_search_grouped), flags 0, outputs (scores, rows, groups)
+  // f8: store and queries are E4M3 rows of d bytes (isx_knn_search_fp8)
   const bool grouped = row_group != nullptr || out_groups != nullptr;
   const bool cont = (flags & ISX_KNN_CONTINUE) != 0, finalize = (flags & ISX_KNN_NO_FINALIZE) == 0;
   const bool packed = (flags & ISX_KNN_PACKED) != 0, no_self = (flags & ISX_KNN_EXCLUDE_SELF) != 0;
@@ -1921,8 +2131,9 @@ static int knn_search_impl(const char* fn, const void* store, const float* store
   }
   ISX_REQUIRE(store && store_rnorm, "%s: null store pointer", fn);
   KnnLaunch L;
-  rc = prepare_search(L, store, store_rnorm, n, queries, query_rnorm, q, d, k, index_base, query_index_base, no_self,
-                      sms, stream);
+  // the fp8 scan moves its E4M3 rows (d bytes) as d / 2 16-bit pairs
+  rc = prepare_search(L, store, store_rnorm, n, queries, query_rnorm, q, f8 ? d / 2 : d, k, index_base, query_index_base,
+                      no_self, sms, stream, f8 ? CU_TENSOR_MAP_DATA_TYPE_UINT16 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16);
   if (rc != ISX_OK) return rc;
   KnnParams& p = L.p;
   p.run_scores = run_scores;
@@ -1934,7 +2145,8 @@ static int knn_search_impl(const char* fn, const void* store, const float* store
   p.row_group = row_group;
   // a continued search keeps the lists and the bounds they imply; only the lockstep counters restart
   if (cont) ISX_CHECK_CUDA(cudaMemsetAsync(p.progress, 0, 256 * sizeof(uint32_t), stream));
-  rc = grouped ? launch_variant<true, false>(L, stream) : launch_variant<false, false>(L, stream);
+  rc = grouped ? launch_variant<true, false>(L, stream)
+               : f8 ? launch_variant<false, false, true>(L, stream) : launch_variant<false, false>(L, stream);
   if (rc != ISX_OK) return rc;
 #ifdef ISX_KNN_PROFILE
   {
@@ -2004,6 +2216,63 @@ int isx_knn_search(const void* store, const float* store_rnorm, int64_t n, const
                    isx_stream_t stream) {
   return isx_knn_search_ex(store, store_rnorm, n, queries, query_rnorm, q, d, k, index_base, 0, 0, out_scores,
                            out_idx, workspace, workspace_bytes, stream);
+}
+
+int isx_quantize_rows_e4m3(const void* x, int64_t n, int d, int d16, void* out, float* rnorm, isx_stream_t stream_) {
+  const char* fn = "isx_quantize_rows_e4m3";
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  ISX_REQUIRE(n >= 0 && d > 0, "%s: need n >= 0 and d > 0 (n=%lld d=%d)", fn, (long long)n, d);
+  ISX_REQUIRE(d16 >= d && d16 % 16 == 0, "%s: d16 = %d must be a multiple of 16 and >= d = %d", fn, d16, d);
+  if (n == 0) return ISX_OK;
+  ISX_REQUIRE(x && out && rnorm, "%s: null pointer", fn);
+  ISX_REQUIRE((reinterpret_cast<uintptr_t>(out) & 15u) == 0, "%s: out must be 16-byte aligned", fn);
+  int sms = 148;
+  int rc = device_sm_count(&sms);
+  if (rc != ISX_OK) return rc;
+  const long long want = (n + 7) / 8;
+  const int blocks = static_cast<int>(std::max<long long>(1, std::min<long long>(want, static_cast<long long>(sms) * 16)));
+  quantize_e4m3_kernel<<<blocks, 256, 0, stream>>>(static_cast<const __nv_bfloat16*>(x), n, d, d16,
+                                                   static_cast<uint8_t*>(out), rnorm);
+  ISX_CHECK_CUDA(cudaGetLastError());
+  return ISX_OK;
+}
+
+int isx_knn_search_fp8(const void* store8, const float* rnorm8, int64_t n, const void* queries8, const float* qrnorm8,
+                       int q, int d16, int k, int64_t index_base, float* out_scores, int32_t* out_idx, void* workspace,
+                       size_t workspace_bytes, isx_stream_t stream) {
+  const char* fn = "isx_knn_search_fp8";
+  ISX_REQUIRE(d16 > 0 && d16 % 16 == 0, "%s: d16 = %d must be a positive multiple of 16 (16-byte rows for TMA)", fn, d16);
+  return knn_search_impl(fn, store8, rnorm8, n, queries8, qrnorm8, q, d16, k, index_base, 0, 0, out_scores, out_idx,
+                         workspace, workspace_bytes, stream, nullptr, nullptr, nullptr, true);
+}
+
+int isx_knn_rescore(const void* store, const float* rnorm, int64_t n, const void* queries, const float* qrnorm, int q,
+                    int d, const int32_t* cand, int kc, int64_t index_base, int k, float* out_scores, int32_t* out_idx,
+                    isx_stream_t stream_) {
+  const char* fn = "isx_knn_rescore";
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  ISX_REQUIRE(q >= 0 && d > 0 && n >= 0, "%s: need q >= 0, d > 0 and n >= 0 (q=%d d=%d n=%lld)", fn, q, d, (long long)n);
+  ISX_REQUIRE(kc >= 1 && kc <= kMaxK && k >= 1 && k <= kMaxK, "%s: need 1 <= kc, k <= %d (kc=%d k=%d)", fn, kMaxK, kc, k);
+  int rc = check_search_args(fn, store, n, queries, q, d, index_base, 0, false);
+  if (rc != ISX_OK) return rc;
+  if (q == 0) return ISX_OK;
+  ISX_REQUIRE(queries && qrnorm && cand && out_scores && out_idx && (n == 0 || (store && rnorm)), "%s: null pointer", fn);
+  const int blocks = (q + 3) / 4;
+  const int base = static_cast<int>(index_base);
+  if (kc <= 32)
+    rescore_kernel<1><<<blocks, 128, 0, stream>>>(static_cast<const __nv_bfloat16*>(store), rnorm, n,
+                                                  static_cast<const __nv_bfloat16*>(queries), qrnorm, q, d, cand, kc, base,
+                                                  k, out_scores, out_idx);
+  else if (kc <= 64)
+    rescore_kernel<2><<<blocks, 128, 0, stream>>>(static_cast<const __nv_bfloat16*>(store), rnorm, n,
+                                                  static_cast<const __nv_bfloat16*>(queries), qrnorm, q, d, cand, kc, base,
+                                                  k, out_scores, out_idx);
+  else
+    rescore_kernel<4><<<blocks, 128, 0, stream>>>(static_cast<const __nv_bfloat16*>(store), rnorm, n,
+                                                  static_cast<const __nv_bfloat16*>(queries), qrnorm, q, d, cand, kc, base,
+                                                  k, out_scores, out_idx);
+  ISX_CHECK_CUDA(cudaGetLastError());
+  return ISX_OK;
 }
 
 int isx_topk_merge(const float* scores, const int32_t* idx, int g, int q, int k, float* out_scores,

@@ -27,6 +27,9 @@ from torch import Tensor
 from imagescry_b200 import _lib
 
 MAX_K = 128
+# fp8 search: candidates the E4M3 scan passes to the exact re-score by default, the most the scan's
+# fast selection (k <= 16) keeps
+FP8_CANDIDATES = 16
 # range search: a store's first call sizes its record buffer for RANGE_HITS_PER_QUERY hits per query,
 # later calls for the hits per query of the store's previous call of the same kind (search or graph)
 # plus RANGE_HEADROOM, never below RANGE_MIN_CAPACITY records; a call that overflows reruns once at its
@@ -57,6 +60,30 @@ def row_rnorm(x: Tensor, eps: float = 1e-12) -> Tensor:
             rc = _lib.load().isx_row_rnorm_bf16(x.data_ptr(), n, d, eps, out.data_ptr(), stream)
         _lib.check(rc, "isx_row_rnorm_bf16")
     return out
+
+
+def fp8_width(d: int) -> int:
+    """Row width in bytes of the E4M3 copy of d-wide rows: d rounded up to 16 (16-byte TMA rows)."""
+    return (d + 15) // 16 * 16
+
+
+def quantize_e4m3(x: Tensor) -> tuple[Tensor, Tensor]:
+    """E4M3 copy of a bf16 matrix for the fp8 scan (`isx_quantize_rows_e4m3`): every row scaled by the
+    power of two that puts its largest |x| in (224, 448], rounded to nearest even and zero-padded to
+    `fp8_width(d)` bytes.  Returns (uint8 N×d16 E4M3 bit patterns, fp32 `1 / max(‖row‖, eps)` of the
+    E4M3 values)."""
+    _lib.require_cuda(x, "x")
+    if x.dtype != torch.bfloat16 or x.ndim != 2 or not x.is_contiguous():
+        raise ValueError("quantize_e4m3 expects a contiguous 2-D bfloat16 tensor")
+    n, d = x.shape
+    d16 = fp8_width(d)
+    out = torch.empty((n, d16), dtype=torch.uint8, device=x.device)
+    rn = torch.empty(n, dtype=torch.float32, device=x.device)
+    if n:
+        with _lib.on_device(x, out, rn) as stream:
+            rc = _lib.load().isx_quantize_rows_e4m3(x.data_ptr(), n, d, d16, out.data_ptr(), rn.data_ptr(), stream)
+        _lib.check(rc, "isx_quantize_rows_e4m3")
+    return out, rn
 
 
 def merge_topk(scores: Tensor, indices: Tensor, k: int | None = None) -> tuple[Tensor, Tensor]:
@@ -294,9 +321,14 @@ class EmbeddingStore:
 
     `groups` describes which rows belong to one image (a per-cell store has one row per feature-map
     cell): an int `c` (rows [i·c, (i+1)·c) are image i) or a 1-D int64 tensor of `row_offsets`
-    (image i owns rows [offsets[i], offsets[i + 1])).  It enables `search_images`."""
+    (image i owns rows [offsets[i], offsets[i + 1])).  It enables `search_images`.
 
-    def __init__(self, embeddings: Tensor, *, index_base: int = 0, groups: int | Tensor | None = None) -> None:
+    `fp8=True` also keeps an E4M3 copy of the rows (`embeddings_e4m3`, N × `fp8_width(dim)` bytes, with
+    its inverse norms `rnorm_e4m3`), built once here: N·d16 + 4N more bytes of device memory.  It
+    enables `search_fp8`."""
+
+    def __init__(self, embeddings: Tensor, *, index_base: int = 0, groups: int | Tensor | None = None,
+                 fp8: bool = False) -> None:
         if embeddings.ndim != 2:
             raise ValueError(f"embeddings must be 2-D (rows × features), got shape {tuple(embeddings.shape)}")
         offsets = None if groups is None else group_offsets(groups, embeddings.shape[0])
@@ -308,6 +340,10 @@ class EmbeddingStore:
         self.row_group: Tensor | None = None
         if offsets is not None:
             self._set_groups(offsets, 0, self.index_base)
+        self.embeddings_e4m3: Tensor | None = None
+        self.rnorm_e4m3: Tensor | None = None
+        if fp8:
+            self.embeddings_e4m3, self.rnorm_e4m3 = quantize_e4m3(self.embeddings)
 
     def _set_groups(self, offsets: Tensor, begin: int, row0: int) -> None:
         """Rows of this store are rows [begin, begin + len) of the layout `offsets`; a hit's row in
@@ -433,6 +469,83 @@ class EmbeddingStore:
         by (score desc, row asc); if the store has fewer than k images the tail is (-inf, -1, -1)."""
         scores, rows, images = self.search_images_raw(queries, k)
         return scores, images.to(torch.int64), image_cells(rows, images, self.group_first_row)
+
+    def scan_fp8(self, queries: Tensor, k: int) -> tuple[Tensor, Tensor]:
+        """The fp8 scan alone (`isx_knn_search_fp8`): the top-k of the E4M3 copies of the queries and
+        the store by their cosine, (scores fp32 Q×k, int32 global indices Q×k), padding (-inf, -1).
+        These are candidates; the scores are those of the quantized rows."""
+        if self.embeddings_e4m3 is None:
+            raise ValueError("search_fp8 needs a store built with fp8=True")
+        q = self._queries(queries)
+        self._check_k(k)
+        nq = q.shape[0]
+        scores = torch.empty((nq, k), dtype=torch.float32, device=self.device)
+        idx = torch.empty((nq, k), dtype=torch.int32, device=self.device)
+        if nq == 0:
+            return scores, idx
+        q8, qr8 = quantize_e4m3(q)
+        lib = _lib.load()
+        d16 = q8.shape[1]
+        with torch.cuda.device(self.device):
+            ws = self._ws(max(int(lib.isx_knn_workspace_bytes(max(len(self), 1), nq, d16, k)), 256))
+        with _lib.on_device(self.embeddings_e4m3, q8, qr8, scores, idx, ws) as stream:
+            rc = lib.isx_knn_search_fp8(
+                self.embeddings_e4m3.data_ptr(), self.rnorm_e4m3.data_ptr(), len(self), q8.data_ptr(), qr8.data_ptr(), nq,
+                d16, k, self.index_base, scores.data_ptr(), idx.data_ptr(), ws.data_ptr(), ws.numel(), stream,
+            )
+        _lib.check(rc, "isx_knn_search_fp8")
+        return scores, idx
+
+    def rescore(self, queries: Tensor, candidates: Tensor, k: int, *, query_rnorm: Tensor | None = None) -> tuple[Tensor, Tensor]:
+        """Exact re-score of candidate lists (`isx_knn_rescore`): `candidates` Q×kc global rows (any order,
+        -1 = none, 1 <= kc <= 128) → the best k by the bf16 cosine `search` computes, (scores fp32 Q×k,
+        int32 global indices Q×k) ordered by (score desc, index asc), padding (-inf, -1)."""
+        q = self._queries(queries)
+        self._check_k(k)
+        if candidates.ndim != 2 or candidates.shape[0] != q.shape[0] or not (1 <= candidates.shape[1] <= MAX_K):
+            raise ValueError(f"candidates must be Q×kc with 1 <= kc <= {MAX_K}, got shape {tuple(candidates.shape)}")
+        if candidates.dtype.is_floating_point or candidates.dtype == torch.bool:
+            raise ValueError("candidates must be an integer tensor of global rows")
+        nq, kc = candidates.shape
+        cand = candidates.to(device=self.device, dtype=torch.int32).contiguous()
+        scores = torch.empty((nq, k), dtype=torch.float32, device=self.device)
+        idx = torch.empty((nq, k), dtype=torch.int32, device=self.device)
+        if nq == 0:
+            return scores, idx
+        qr = row_rnorm(q) if query_rnorm is None else query_rnorm
+        with _lib.on_device(self.embeddings, q, qr, cand, scores, idx) as stream:
+            rc = _lib.load().isx_knn_rescore(
+                self.embeddings.data_ptr(), self.rnorm.data_ptr(), len(self), q.data_ptr(), qr.data_ptr(), nq, q.shape[1],
+                cand.data_ptr(), kc, self.index_base, k, scores.data_ptr(), idx.data_ptr(), stream,
+            )
+        _lib.check(rc, "isx_knn_rescore")
+        return scores, idx
+
+    def search_fp8_raw(self, queries: Tensor, k: int, *, candidates: int = FP8_CANDIDATES) -> tuple[Tensor, Tensor]:
+        """`search_fp8` with int32 global indices."""
+        if self.embeddings_e4m3 is None:
+            raise ValueError("search_fp8 needs a store built with fp8=True")
+        if isinstance(k, bool) or isinstance(candidates, bool) or not (1 <= k <= candidates <= MAX_K):
+            raise ValueError(f"search_fp8 needs 1 <= k <= candidates <= {MAX_K}, got k={k} candidates={candidates}")
+        q = self._queries(queries)
+        nq = q.shape[0]
+        if nq == 0 or len(self) == 0:
+            return (torch.full((nq, k), float("-inf"), dtype=torch.float32, device=self.device),
+                    torch.full((nq, k), -1, dtype=torch.int32, device=self.device))
+        _, cand = self.scan_fp8(q, candidates)
+        return self.rescore(q, cand, k)
+
+    def search_fp8(self, queries: Tensor, k: int, *, candidates: int = FP8_CANDIDATES) -> tuple[Tensor, Tensor]:
+        """Cosine top-k through the fp8 tensor-core path: (scores fp32 Q×k, indices int64 Q×k).
+
+        An E4M3 scan of the store picks the `candidates` best rows of every query by the cosine of the
+        quantized rows; those are re-scored exactly from the bf16 rows and the best k returned, ordered
+        by (score desc, index asc).  Every returned score is the fp32 cosine `search` computes for the
+        pair (up to its fp32 summation order); only recall is approximate: a row of the exact top-k is
+        missed when quantization moves it out of the candidates.  More candidates, more recall; 16 is
+        the most the scan's fast selection keeps.  Needs a store built with `fp8=True`."""
+        scores, idx = self.search_fp8_raw(queries, k, candidates=candidates)
+        return scores, idx.to(torch.int64)
 
     def range_records(
         self, q: Tensor, q_rnorm: Tensor, threshold: float, *, flags: int = 0, query_index_base: int = 0,
@@ -568,7 +681,7 @@ class ShardedEmbeddingStore:
     be cut by a shard boundary."""
 
     def __init__(self, local_embeddings: Tensor, *, total_rows: int | None = None, index_base: int | None = None, group=None,
-                 groups: int | Tensor | None = None) -> None:
+                 groups: int | Tensor | None = None, fp8: bool = False) -> None:
         import torch.distributed as dist
 
         self.group = group
@@ -584,7 +697,7 @@ class ShardedEmbeddingStore:
                 )
             index_base = begin
         self.total_rows = total_rows
-        self.local = EmbeddingStore(local_embeddings, index_base=index_base)
+        self.local = EmbeddingStore(local_embeddings, index_base=index_base, fp8=fp8)
         if groups is not None:
             if isinstance(groups, int) and not isinstance(groups, bool) and total_rows is None:
                 raise ValueError("groups given as rows per image need total_rows")
@@ -601,6 +714,17 @@ class ShardedEmbeddingStore:
         s, r, g = self.local.search_images_raw(queries, k)
         merged_s, merged_r, merged_g = merge_topk_groups(gather_group_records(pack_group_records(s, r, g), self.group), k)
         return merged_s, merged_g.to(torch.int64), image_cells(merged_r, merged_g, self.local.group_first_row)
+
+    def search_fp8(self, queries: Tensor, k: int, *, candidates: int = FP8_CANDIDATES) -> tuple[Tensor, Tensor]:
+        """`EmbeddingStore.search_fp8` over the sharded store (built with `fp8=True`): local fp8 scan and
+        exact re-score, ONE all-gather of the packed records, merge.  The ranks merge exact scores: a
+        returned score is bit for bit the one the unsharded store computes for the pair.  Each rank keeps
+        its own `candidates`, a superset of the unsharded candidates (the scan's scores do not depend on
+        the shard), so the result is the exact top-k of more candidates: never a worse row, sometimes a
+        better one than the unsharded `search_fp8`."""
+        s, i = self.local.search_fp8_raw(queries, k, candidates=candidates)
+        merged_s, merged_i = merge_topk_packed(gather_records(pack_records(s, i), self.group), k)
+        return merged_s, merged_i.to(torch.int64)
 
     def search_range(self, queries: Tensor, threshold: float) -> tuple[Tensor, Tensor, Tensor]:
         """`EmbeddingStore.search_range` over the sharded store: local range search with global rows, one

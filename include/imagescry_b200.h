@@ -262,6 +262,35 @@ int isx_knn_range_sort(const int32_t* records, int64_t total, int q, int64_t* of
                        int32_t* rows, float* scores, void* workspace, size_t workspace_bytes,
                        isx_stream_t stream);
 
+/* fp8 search, stage 1 of 3: an E4M3 copy of bf16 rows (n x d) for isx_knn_search_fp8.  Every row is
+ * scaled by the power of two that puts its largest |x| in (224, 448] (exact; a cosine does not change),
+ * rounded to nearest even into E4M3 and zero-padded to d16 bytes (d16 % 16 == 0, d16 >= d): out is
+ * uint8 n x d16, 16-byte aligned.  rnorm[i] = 1 / max(||row_i||_2, 1e-12) of the E4M3 values as
+ * written (the correctly rounded norm).  A zero row stays zero and gets 1 / 1e-12, so it scores 0.
+ * Rows that are power-of-two multiples of each other get identical bytes. */
+int isx_quantize_rows_e4m3(const void* x, int64_t n, int d, int d16, void* out, float* rnorm, isx_stream_t stream);
+
+/* fp8 search, stage 2: the k-NN search of isx_knn_search over E4M3 rows from isx_quantize_rows_e4m3
+ * (store8 n x d16, queries8 q x d16, with their rnorm), on the tensor cores' fp8 path.  out_scores fp32
+ * q x k are the cosines of the quantized rows, out_idx int32 q x k = index_base + local row, ordered
+ * and padded as by isx_knn_search.  These are CANDIDATES: the scores are not within the search's
+ * tolerance of the bf16 cosine; isx_knn_rescore makes them exact.  k <= 128; the workspace is sized by
+ * isx_knn_workspace_bytes(n, q, d16, k). */
+int isx_knn_search_fp8(const void* store8, const float* rnorm8, int64_t n, const void* queries8,
+                       const float* qrnorm8, int q, int d16, int k, int64_t index_base, float* out_scores,
+                       int32_t* out_idx, void* workspace, size_t workspace_bytes, isx_stream_t stream);
+
+/* fp8 search, stage 3: exact re-score of candidate lists.  cand: int32 q x kc global rows (any order;
+ * -1 and rows outside [index_base, index_base + n) are skipped, a row listed twice counts once), 1 <= kc
+ * <= 128.  Each candidate is scored from the bf16 rows (store n x d, queries q x d, d % 8 == 0, 16-byte
+ * aligned) with the inverse norms of isx_row_rnorm_bf16: fp32 dot product in a fixed order, then
+ * fl(fl(dot * rnorm) * qrnorm), the product order of isx_knn_search.  out_scores fp32 q x k and out_idx
+ * int32 q x k receive the best k by (score desc, index asc), padded with (-inf, -1) (also when kc < k).
+ * Deterministic: the same inputs give the same bits. */
+int isx_knn_rescore(const void* store, const float* rnorm, int64_t n, const void* queries, const float* qrnorm,
+                    int q, int d, const int32_t* cand, int kc, int64_t index_base, int k, float* out_scores,
+                    int32_t* out_idx, isx_stream_t stream);
+
 /* ---- ROI masks on the feature-map grid (SURVEY.md 8f-4) ---------------------------------------
  * geometry.py:14-65 `create_roi_mask`: rasterio.features.rasterize(shapes, out_shape=(hf, wf),
  * transform=Affine.scale(w / wf, h / hf), fill=0, all_touched=True) * class_index.  rasterio / GDAL
