@@ -119,6 +119,15 @@ SIGNATURES: dict[str, tuple] = {
         [c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_int, c_int, c_void_p, c_int, c_int64, c_int, c_void_p,
          c_void_p, c_void_p],
     ),
+    "isx_knn_maxsim": (
+        c_int,
+        [c_void_p, c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_int, c_int, c_int64, c_int64, c_void_p, c_void_p,
+         c_size_t, c_void_p],
+    ),
+    "isx_maxsim_sets_topk": (
+        c_int,
+        [c_void_p, c_void_p, c_int, c_int64, c_int64, c_int64, c_void_p, c_int, c_int, c_int64, c_void_p, c_void_p],
+    ),
     "isx_roi_rasterize":(c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int64, c_void_p, c_void_p]),
     "isx_masked_pool": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_int, c_int64, c_void_p, c_void_p]),
 }

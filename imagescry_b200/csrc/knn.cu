@@ -308,6 +308,10 @@ struct KnnParams {
   int32_t* range_rec;
   long long range_cap;
   unsigned long long* range_count;
+  // maxsim only: cell_max[q][num_groups] (row-major, 64-bit index) receives, for every query row and
+  // group g in [group_base, group_base + num_groups), the largest raw score of g's rows (atomic max)
+  float* cell_max;
+  int group_base, num_groups;
 #ifdef ISX_KNN_PROFILE
   unsigned long long* prof;  // [16] wait-cycle counters (diagnostic build only: -DISX_KNN_PROFILE)
   int debug_skip_select;     // ISX_KNN_SKIP_SELECT=1: the epilogue only loads and releases (floor of the MMA pipeline)
@@ -341,8 +345,9 @@ struct KnnParams {
 // Shared-memory plan.  k <= kSmallK: 32-entry per-row candidate buffers live in shared memory next to
 // a 4-stage operand ring (the buffers are XOR-swizzled by row so that 32 rows appending at the same
 // depth hit different banks).  Larger k: 256-entry buffers in the global workspace.  Range search
-// (RANGE) has no candidate buffers: it is the CAP = 32 plan without them.
-template <int CAP, int NCTA, bool RES_ = false, bool GROUPED = false, bool RANGE = false>
+// (RANGE) has no candidate buffers: it is the CAP = 32 plan without them; MAXSIM likewise, plus the
+// tile's group ids.
+template <int CAP, int NCTA, bool RES_ = false, bool GROUPED = false, bool RANGE = false, bool MAXSIM = false>
 struct KnnSmem {
   // RES: the query tile (all k-blocks, at most kResKb = 4, i.e. d <= 256) stays resident in shared
   // memory for a whole item and the ring holds store tiles only: half the operand traffic per tile.
@@ -353,7 +358,7 @@ struct KnnSmem {
   static constexpr int STAGES = RES ? 6 : (NCTA == 2) ? (CAP <= 32 ? 5 : 6) : (CAP <= 32 ? 3 : 4);
   static constexpr bool kSmemCand = (CAP <= 32);
   static constexpr int CHUNK = kSmemCand ? 16 : 32;  // accumulator columns per selection window
-  static constexpr uint32_t kCandBytes = (kSmemCand && !RANGE) ? G * BM * CAP * 8 : 0;
+  static constexpr uint32_t kCandBytes = (kSmemCand && !RANGE && !MAXSIM) ? G * BM * CAP * 8 : 0;
   static constexpr uint32_t kAOff = 0;
   static constexpr uint32_t kBOff = kAOff + (RES ? kResKb : STAGES) * A_STAGE_BYTES;
   static constexpr uint32_t kCandOff = kBOff + STAGES * B_STAGE_BYTES;
@@ -361,9 +366,11 @@ struct KnnSmem {
   static constexpr uint32_t kBarOff = kRnormOff + ACC_STAGES * BN * 4;    // mbarriers
   static constexpr uint32_t kNumBars = 2 * STAGES + 2 * ACC_STAGES + 2;  // + resident-query full / empty
   static constexpr uint32_t kTmemPtrOff = kBarOff + kNumBars * 8;
-  // grouped search: [ACC_STAGES][BN / 32] flags, 1 where all 32 store rows of a chunk are one group
+  // grouped search and maxsim: [ACC_STAGES][BN / 32] flags, 1 where all 32 store rows of a chunk are one group
   static constexpr uint32_t kChunkUniOff = kTmemPtrOff + 16;
-  static constexpr uint32_t kTotal = kChunkUniOff + (GROUPED ? ACC_STAGES * (BN / 32) * 4 : 0);
+  // maxsim: [ACC_STAGES][BN] group ids of the tile's store rows (-1 past the store's end)
+  static constexpr uint32_t kGroupIdOff = kChunkUniOff + ((GROUPED || MAXSIM) ? ACC_STAGES * (BN / 32) * 4 : 0);
+  static constexpr uint32_t kTotal = kGroupIdOff + (MAXSIM ? ACC_STAGES * BN * 4 : 0);
   // the operand tiles need 1024-byte alignment; the dynamic window normally starts aligned, so only
   // as much slack as the 227 KB limit leaves is requested and the kernel checks that it suffices
   static constexpr uint32_t kMaxDynamic = 232448;
@@ -724,6 +731,17 @@ __device__ __forceinline__ void range_append(const uint32_t (&r)[32], bool pass,
   }
 }
 
+// ---- maxsim ------------------------------------------------------------------------------------
+// atomic max of an fp32 value: a non-negative float orders like its bits as a signed int, a negative
+// one inversely to its bits as an unsigned int, so the pair signed max / unsigned min updates the
+// value in place (the slot starts at -inf).  -0 is turned into +0 first, so that the two never race
+// through different updates.
+__device__ __forceinline__ void atomic_max_f32(float* addr, float v) {
+  v = (v == 0.f) ? 0.f : v;
+  if (__float_as_int(v) >= 0) atomicMax(reinterpret_cast<int*>(addr), __float_as_int(v));
+  else atomicMin(reinterpret_cast<unsigned int*>(addr), __float_as_uint(v));
+}
+
 // GROUPED: image-level search (knn_search_grouped_kernel).  The k-th best DISTINCT-GROUP score of
 // any subset of the store is a lower bound of the global one, so the fast path, the shared bound and
 // the item-end skip stay as they are; only where a threshold is derived — the buffer prune, the
@@ -739,10 +757,18 @@ __device__ __forceinline__ void range_append(const uint32_t (&r)[32], bool pass,
 // (p.d = d16 / 2, tensor maps of UINT16), so a k-block is still one 128-byte swizzle row of BK units,
 // now 128 elements: the ring, the TMA boxes, the descriptors and their 32-byte step per MMA (K = 32
 // under kind::f8f6f4) and the whole epilogue are those of the bf16 kernel; only the MMA kind changes.
-template <int CAP, int NCTA, bool RES, bool GROUPED, bool RANGE = false, bool F8 = false>
+//
+// MAXSIM: the per-(query row, group) maxima of multi-vector search (knn_maxsim_kernel, CAP = 32
+// variants only).  The epilogue keeps the fast path's scaling and chunk maximum and drops everything
+// else (thresholds, buffers, prunes, shared bound, item end): a chunk of one group folds its maximum
+// into the row's running (group, max) pair, a mixed chunk walks its columns by the staged group ids,
+// and a pair is flushed into p.cell_max by atomic max when the group changes and at the item end.
+// Atomics, because a group can be cut by an N-split or between the two epilogue groups' halves.
+template <int CAP, int NCTA, bool RES, bool GROUPED, bool RANGE = false, bool F8 = false, bool MAXSIM = false>
 __device__ __forceinline__ void knn_search_body(const CUtensorMap& tmap_q, const CUtensorMap& tmap_e, const KnnParams& p) {
   static_assert(!F8 || (!GROUPED && !RANGE), "the fp8 scan is a plain search");
-  using L = KnnSmem<CAP, NCTA, RES, GROUPED, RANGE>;
+  static_assert(!MAXSIM || (!GROUPED && !RANGE && !F8 && CAP == 32), "maxsim is its own mode of the CAP = 32 plan");
+  using L = KnnSmem<CAP, NCTA, RES, GROUPED, RANGE, MAXSIM>;
   constexpr int STAGES = L::STAGES;
   constexpr int kEpiGroups = L::G;
   constexpr int kGroupCols = BN / kEpiGroups;
@@ -994,13 +1020,21 @@ __device__ __forceinline__ void knn_search_body(const CUtensorMap& tmap_q, const
         const long long n0_ = nb_ * BN;
         pre_rn = (n0_ + et < p.n) ? __ldg(p.store_rnorm + n0_ + et) : 0.f;
         if (kEpiGroups == 1) pre_rn2 = (n0_ + et + 128 < p.n) ? __ldg(p.store_rnorm + n0_ + et + 128) : 0.f;
-        if constexpr (GROUPED) {
+        if constexpr (GROUPED || MAXSIM) {
           pre_g = (n0_ + et < p.n) ? __ldg(p.row_group + n0_ + et) : -1;
           if (kEpiGroups == 1) pre_g2 = (n0_ + et + 128 < p.n) ? __ldg(p.row_group + n0_ + et + 128) : -1;
         }
-        if constexpr (!RANGE) {
+        if constexpr (!RANGE && !MAXSIM) {
           if (row_valid) pre_thr = *reinterpret_cast<const volatile uint32_t*>(p.thr_shared + qrow);
         }
+      };
+      // maxsim: the row's running (group, maximum) pair and its flush into cell_max
+      int ms_g = -1;
+      float ms_max = -INFINITY;
+      auto maxsim_flush = [&]() {
+        const long long gi = static_cast<long long>(ms_g) - p.group_base;
+        if (row_valid && gi >= 0 && gi < p.num_groups)
+          atomic_max_f32(p.cell_max + static_cast<size_t>(qrow) * static_cast<size_t>(p.num_groups) + gi, ms_max);
       };
       prefetch_tile(nb0);
 
@@ -1014,7 +1048,12 @@ __device__ __forceinline__ void knn_search_body(const CUtensorMap& tmap_q, const
         rn[et] = pre_rn;
         if (kEpiGroups == 1) rn[et + 128] = pre_rn2;
         int* chunk_uni = reinterpret_cast<int*>(smem + L::kChunkUniOff) + acc * (BN / 32);
-        if constexpr (GROUPED) {
+        int* gid_s = reinterpret_cast<int*>(smem + L::kGroupIdOff) + acc * BN;
+        if constexpr (MAXSIM) {
+          gid_s[et] = pre_g;
+          if (kEpiGroups == 1) gid_s[et + 128] = pre_g2;
+        }
+        if constexpr (GROUPED || MAXSIM) {
           // the 32 rows this warp stages are one selection chunk: flag it when they are all one group
           const int g0 = __shfl_sync(kFullMask, pre_g, 0);
           const bool uni = __all_sync(kFullMask, pre_g == g0 && pre_g >= 0);
@@ -1025,7 +1064,7 @@ __device__ __forceinline__ void knn_search_body(const CUtensorMap& tmap_q, const
             if (lane == 0) chunk_uni[(et + 128) >> 5] = uni1 ? 1 : 0;
           }
         }
-        if constexpr (!RANGE) {
+        if constexpr (!RANGE && !MAXSIM) {
           if (row_valid) thr = fmaxf(thr, thr_decode_below(pre_thr));
         }
         if (nb + 1 < nb1) prefetch_tile(nb + 1);
@@ -1104,8 +1143,28 @@ __device__ __forceinline__ void knn_search_body(const CUtensorMap& tmap_q, const
           }
           return vmax;
         };
+        // maxsim: fold one chunk into the running pair (group ids are warp-uniform: one column at a time)
+        auto maxsim_chunk = [&](const uint32_t (&r)[32], int cbase, float vmax) {
+          if (chunk_uni[cbase >> 5]) {
+            const int g = gid_s[cbase];
+            if (g != ms_g) { maxsim_flush(); ms_g = g; ms_max = vmax; }
+            else ms_max = fmaxf(ms_max, vmax);
+            return;
+          }
+#pragma unroll
+          for (int j = 0; j < 32; ++j) {
+            const int g = gid_s[cbase + j];
+            const float v = __uint_as_float(r[j]);
+            if (g != ms_g) { maxsim_flush(); ms_g = g; ms_max = v; }
+            else ms_max = fmaxf(ms_max, v);
+          }
+        };
         // rare path of one chunk
         auto collect_chunk = [&](uint32_t (&r)[32], int cbase, const float (&g)[8], float vmax) {
+          if constexpr (MAXSIM) {
+            maxsim_chunk(r, cbase, vmax);
+            return;
+          }
           if (!__any_sync(kFullMask, vmax > thr)) return;
           ISX_PROF_COUNT(10, 1);
           if constexpr (RANGE) {
@@ -1260,12 +1319,17 @@ __device__ __forceinline__ void knn_search_body(const CUtensorMap& tmap_q, const
         // Off the hand-off path (the accumulator stage is already released): prune the rows whose
         // buffers are more than half-way from k to full, so that a prune inside the next tiles' chunk
         // loops — where it delays the release every other warp of the pair waits for — stays an exception.
-        if constexpr (!RANGE) prune_rows(__ballot_sync(kFullMask, 2 * cnt > CAP + p.k));
+        if constexpr (!RANGE && !MAXSIM) prune_rows(__ballot_sync(kFullMask, 2 * cnt > CAP + p.k));
         ISX_PROF_END(6);
         if (++acc == ACC_STAGES) { acc = 0; acc_phase ^= 1; }
       }
       // range search: the hits are in the record buffer already; there is no list to merge
       if constexpr (RANGE) continue;
+      // maxsim: the row's last pair of the item; there is no list to merge either
+      if constexpr (MAXSIM) {
+        maxsim_flush();
+        continue;
+      }
 
       // item done: sort every row's candidates and merge the best k into the query's RUNNING list in
       // global memory (under a per-query lock; lists of different items never share a store row, so
@@ -1620,6 +1684,13 @@ knn_search_fp8_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_c
   knn_search_body<CAP, NCTA, RES, false, false, true>(tmap_q, tmap_e, p);
 }
 
+template <int NCTA, bool RES>
+__global__ void __launch_bounds__(knn_threads(32), 1)
+knn_maxsim_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_constant__ CUtensorMap tmap_e,
+                  const KnnParams p) {
+  knn_search_body<32, NCTA, RES, false, false, false, true>(tmap_q, tmap_e, p);
+}
+
 // ------------------------------------------------------------------------------------------
 // K5: merge g sorted-or-not partial lists per query into the final top-k.  One warp per query.
 // ------------------------------------------------------------------------------------------
@@ -1879,6 +1950,83 @@ rescore_kernel(const __nv_bfloat16* __restrict__ store, const float* __restrict_
   }
 }
 
+// ------------------------------------------------------------------------------------------
+// K6: set scores and top-k of multi-vector (maxsim) search.  One CTA per query set S = rows [s0, s1):
+// a thread owns the columns col0 + tid, col0 + tid + 256, ... (consecutive threads read consecutive
+// columns of a cell_max row) and scores each as
+//   score = fl(sum over c = s0 .. s1-1, in that order, of fl(cell_max[c][col] * rnorm_q[c])) / |S|
+// (fp32 adds and a correctly rounded divide: no contraction, no reordering).  A column whose score is
+// -inf (a group without rows) is not a result.  The CTA keeps its best k in shared memory, sorted by
+// (score desc, group asc); a round of 256 columns with any column that sorts before the k-th appends
+// those to the list and re-sorts the 512 slots (bitonic).  Output: k packed records {score bits,
+// group_base + col} per set, padded with (-inf, -1): the format isx_topk_merge_packed merges.
+// ------------------------------------------------------------------------------------------
+constexpr int kSetThreads = 256;
+constexpr int kSetSlots = 512;  // k <= 128 kept + 256 fresh, rounded up to a power of two
+
+__global__ void __launch_bounds__(kSetThreads)
+maxsim_sets_topk_kernel(const float* __restrict__ cell_max, const float* __restrict__ qrnorm, int q, long long ld,
+                        int col0, int col1, const int64_t* __restrict__ set_off, int k, int group_base,
+                        uint2* __restrict__ records) {
+  __shared__ float ls[kSetSlots];
+  __shared__ int li[kSetSlots];
+  const int tid = threadIdx.x;
+  const int set = blockIdx.x;
+  // offsets come from the caller: clamp them to the matrix so that a malformed set reads nothing outside it
+  const long long lo = set_off[set], hi = set_off[set + 1];
+  const long long s0 = min(max(lo, 0ll), static_cast<long long>(q));
+  const long long s1 = min(max(hi, s0), static_cast<long long>(q));
+  for (int i = tid; i < kSetSlots; i += kSetThreads) { ls[i] = -INFINITY; li[i] = INT_MAX; }
+  __syncthreads();
+  const float set_size = static_cast<float>(s1 - s0);  // exact below 2^24
+  if (s1 > s0) {
+    for (int base = col0; base < col1; base += kSetThreads) {
+      const int c = base + tid;
+      float sc = -INFINITY;
+      const int id = group_base + c;
+      if (c < col1) {
+        const float* col = cell_max + c;
+        float sum = 0.f;
+#pragma unroll 8
+        for (long long r = s0; r < s1; ++r) sum = __fadd_rn(sum, __fmul_rn(__ldg(col + r * ld), __ldg(qrnorm + r)));
+        sc = __fdiv_rn(sum, set_size);
+      }
+      const bool cand = sc > -INFINITY && pair_before(sc, id, ls[k - 1], li[k - 1]);
+      if (__syncthreads_or(cand)) {
+        ls[k + tid] = cand ? sc : -INFINITY;
+        li[k + tid] = cand ? id : INT_MAX;
+        __syncthreads();
+        for (int size = 2; size <= kSetSlots; size <<= 1) {
+          for (int stride = size >> 1; stride > 0; stride >>= 1) {
+            const int i = 2 * tid - (tid & (stride - 1));
+            const int j = i + stride;
+            const bool desc = (i & size) == 0;
+            const float si = ls[i], sj = ls[j];
+            const int ii = li[i], ij = li[j];
+            if (desc ? pair_before(sj, ij, si, ii) : pair_before(si, ii, sj, ij)) {
+              ls[i] = sj; ls[j] = si; li[i] = ij; li[j] = ii;
+            }
+            __syncthreads();
+          }
+        }
+        for (int i = k + tid; i < kSetSlots; i += kSetThreads) { ls[i] = -INFINITY; li[i] = INT_MAX; }
+        __syncthreads();
+      }
+    }
+  }
+  for (int j = tid; j < k; j += kSetThreads) {
+    const bool have = li[j] != INT_MAX;
+    records[static_cast<size_t>(set) * k + j] =
+        make_uint2(__float_as_uint(have ? ls[j] : -INFINITY), static_cast<uint32_t>(have ? li[j] : -1));
+  }
+}
+
+__global__ void __launch_bounds__(256) fill_f32_kernel(float* __restrict__ x, long long n, float v) {
+  for (long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x; i < n;
+       i += static_cast<long long>(gridDim.x) * blockDim.x)
+    x[i] = v;
+}
+
 size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
 struct KnnWorkspace {
@@ -1903,14 +2051,17 @@ KnnWorkspace knn_workspace(int max_grid, int q, int k) {
   return w;
 }
 
-template <int CAP, int NCTA, bool RES = false, bool GROUPED = false, bool RANGE = false, bool F8 = false>
+template <int CAP, int NCTA, bool RES = false, bool GROUPED = false, bool RANGE = false, bool F8 = false,
+          bool MAXSIM = false>
 int launch_search(const CUtensorMap& tq, const CUtensorMap& te, const KnnParams& p, int grid, cudaStream_t stream) {
   static_assert(!RANGE || (CAP == 32 && !GROUPED), "range search has the CAP = 32 plan only");
   static_assert(!F8 || (!GROUPED && !RANGE), "the fp8 scan is a plain search");
-  auto kern = F8 ? knn_search_fp8_kernel<CAP, NCTA, RES>
-                 : RANGE ? knn_range_kernel<NCTA, RES>
-                         : GROUPED ? knn_search_grouped_kernel<CAP, NCTA, RES> : knn_search_kernel<CAP, NCTA, RES>;
-  const int smem = static_cast<int>(KnnSmem<CAP, NCTA, RES, GROUPED, RANGE>::kDynamicBytes);
+  static_assert(!MAXSIM || (CAP == 32 && !GROUPED && !RANGE && !F8), "maxsim has the CAP = 32 plan only");
+  auto kern = MAXSIM ? knn_maxsim_kernel<NCTA, RES>
+              : F8   ? knn_search_fp8_kernel<CAP, NCTA, RES>
+              : RANGE ? knn_range_kernel<NCTA, RES>
+                      : GROUPED ? knn_search_grouped_kernel<CAP, NCTA, RES> : knn_search_kernel<CAP, NCTA, RES>;
+  const int smem = static_cast<int>(KnnSmem<CAP, NCTA, RES, GROUPED, RANGE, MAXSIM>::kDynamicBytes);
   ISX_CHECK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = dim3(static_cast<unsigned>(grid));
@@ -2015,20 +2166,22 @@ int prepare_search(KnnLaunch& L, const void* store, const float* store_rnorm, in
 
 // The one choice of kernel variant (CAP, NCTA, RES).  Plain, grouped and range search pick the same
 // variant for the same (q, d, k <= kSmallK): same MMA shapes, same scaling, so their scores are bit
-// for bit equal.  F8 (the E4M3 scan, p.d in 16-bit pairs) follows the same rules.
-template <bool GROUPED, bool RANGE, bool F8 = false>
+// for bit equal.  F8 (the E4M3 scan, p.d in 16-bit pairs) follows the same rules, and so does MAXSIM
+// (run with p.k = kSmallK, like range search), whose maxima are therefore maxima of search()'s values.
+template <bool GROUPED, bool RANGE, bool F8 = false, bool MAXSIM = false>
 int launch_variant(const KnnLaunch& L, cudaStream_t stream) {
+  static_assert(!MAXSIM || (!GROUPED && !RANGE && !F8), "maxsim excludes the grouped, range and fp8 modes");
   const KnnParams& p = L.p;
   const int grid = L.plan.grid;
-  if constexpr (!RANGE) {
+  if constexpr (!RANGE && !MAXSIM) {
     if (p.k > kSmallK)
       return L.ncta == 2 ? launch_search<256, 2, false, GROUPED, false, F8>(L.tq, L.te, p, grid, stream)
                          : launch_search<256, 1, false, GROUPED, false, F8>(L.tq, L.te, p, grid, stream);
   }
-  if (L.ncta == 1) return launch_search<32, 1, false, GROUPED, RANGE, F8>(L.tq, L.te, p, grid, stream);
+  if (L.ncta == 1) return launch_search<32, 1, false, GROUPED, RANGE, F8, MAXSIM>(L.tq, L.te, p, grid, stream);
   // short rows (at most 512 bytes: the resident tile's 4 k-blocks), small k: the query tile stays resident
-  if (p.d <= 256) return launch_search<32, 2, true, GROUPED, RANGE, F8>(L.tq, L.te, p, grid, stream);
-  return launch_search<32, 2, false, GROUPED, RANGE, F8>(L.tq, L.te, p, grid, stream);
+  if (p.d <= 256) return launch_search<32, 2, true, GROUPED, RANGE, F8, MAXSIM>(L.tq, L.te, p, grid, stream);
+  return launch_search<32, 2, false, GROUPED, RANGE, F8, MAXSIM>(L.tq, L.te, p, grid, stream);
 }
 
 }  // namespace
@@ -2353,6 +2506,65 @@ int isx_knn_range(const void* store, const float* store_rnorm, int64_t n, const 
   p.range_count = count;
   ISX_CHECK_CUDA(cudaMemsetAsync(p.progress, 0, 256 * sizeof(uint32_t), stream));
   return launch_variant<false, true>(L, stream);
+}
+
+int isx_knn_maxsim(const void* store, const float* store_rnorm, const int32_t* row_group, int64_t n, const void* queries,
+                   const float* query_rnorm, int q, int d, int64_t group_base, int64_t num_groups, float* cell_max,
+                   void* workspace, size_t workspace_bytes, isx_stream_t stream_) {
+  const char* fn = "isx_knn_maxsim";
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  ISX_REQUIRE(q > 0 && d > 0 && n >= 0, "%s: need q, d > 0 and n >= 0 (q=%d d=%d n=%lld)", fn, q, d, (long long)n);
+  ISX_REQUIRE(num_groups >= 1 && group_base >= 0 && group_base + num_groups <= (1ll << 31),
+              "%s: need num_groups >= 1 and 0 <= group_base, group_base + num_groups <= 2^31 (got %lld, %lld)", fn,
+              (long long)group_base, (long long)num_groups);
+  int rc = check_search_args(fn, store, n, queries, q, d, 0, 0, false);
+  if (rc != ISX_OK) return rc;
+  ISX_REQUIRE(queries && query_rnorm && cell_max, "%s: null pointer", fn);
+  ISX_REQUIRE((reinterpret_cast<uintptr_t>(cell_max) & 3u) == 0, "%s: cell_max must be 4-byte aligned", fn);
+  ISX_REQUIRE(workspace != nullptr && workspace_bytes >= ISX_KNN_RANGE_WORKSPACE_BYTES,
+              "%s: workspace too small (%zu < %d)", fn, workspace_bytes, ISX_KNN_RANGE_WORKSPACE_BYTES);
+  int sms = 148;
+  rc = device_sm_count(&sms);
+  if (rc != ISX_OK) return rc;
+  const long long cells = static_cast<long long>(q) * num_groups;
+  const int fill_blocks = static_cast<int>(std::max<long long>(1, std::min<long long>((cells + 255) / 256, static_cast<long long>(sms) * 16)));
+  fill_f32_kernel<<<fill_blocks, 256, 0, stream>>>(cell_max, cells, -INFINITY);
+  ISX_CHECK_CUDA(cudaGetLastError());
+  if (n == 0) return ISX_OK;
+  ISX_REQUIRE(store && store_rnorm && row_group, "%s: null store pointer", fn);
+  KnnLaunch L;
+  rc = prepare_search(L, store, store_rnorm, n, queries, query_rnorm, q, d, kSmallK, 0, 0, false, sms, stream);
+  if (rc != ISX_OK) return rc;
+  KnnParams& p = L.p;
+  p.progress = reinterpret_cast<uint32_t*>((reinterpret_cast<uintptr_t>(workspace) + 255) & ~uintptr_t(255));
+  p.row_group = row_group;
+  p.cell_max = cell_max;
+  p.group_base = static_cast<int>(group_base);
+  p.num_groups = static_cast<int>(std::min<int64_t>(num_groups, INT_MAX));
+  ISX_CHECK_CUDA(cudaMemsetAsync(p.progress, 0, 256 * sizeof(uint32_t), stream));
+  return launch_variant<false, false, false, true>(L, stream);
+}
+
+int isx_maxsim_sets_topk(const float* cell_max, const float* query_rnorm, int q, int64_t num_groups, int64_t col_begin,
+                         int64_t col_end, const int64_t* set_offsets, int num_sets, int k, int64_t group_base,
+                         void* records, isx_stream_t stream_) {
+  const char* fn = "isx_maxsim_sets_topk";
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  ISX_REQUIRE(q >= 0 && num_sets >= 0 && num_groups >= 1, "%s: need q, num_sets >= 0 and num_groups >= 1", fn);
+  ISX_REQUIRE(k >= 1 && k <= kMaxK, "%s: need 1 <= k <= %d (k=%d)", fn, kMaxK, k);
+  ISX_REQUIRE(0 <= col_begin && col_begin <= col_end && col_end <= num_groups,
+              "%s: need 0 <= col_begin <= col_end <= num_groups (got %lld, %lld, %lld)", fn, (long long)col_begin,
+              (long long)col_end, (long long)num_groups);
+  ISX_REQUIRE(group_base >= 0 && group_base + num_groups <= (1ll << 31), "%s: group ids must fit in int32", fn);
+  if (num_sets == 0) return ISX_OK;
+  ISX_REQUIRE(set_offsets && records && (q == 0 || (cell_max && query_rnorm)), "%s: null pointer", fn);
+  ISX_REQUIRE((reinterpret_cast<uintptr_t>(records) & 7u) == 0, "%s: records must be 8-byte aligned", fn);
+  maxsim_sets_topk_kernel<<<num_sets, kSetThreads, 0, stream>>>(cell_max, query_rnorm, q, num_groups,
+                                                                static_cast<int>(col_begin), static_cast<int>(col_end),
+                                                                set_offsets, k, static_cast<int>(group_base),
+                                                                static_cast<uint2*>(records));
+  ISX_CHECK_CUDA(cudaGetLastError());
+  return ISX_OK;
 }
 
 }  // extern "C"

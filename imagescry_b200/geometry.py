@@ -140,4 +140,31 @@ def roi_query(embeddings: Tensor, mask: Tensor, class_index: int = 1) -> Tensor:
     return out[0] if squeeze else out
 
 
-__all__: Sequence[str] = ("create_roi_mask", "polygon_edges", "roi_query")
+def roi_cells(embeddings: Tensor, mask: Tensor, class_index: int = 1) -> tuple[Tensor, Tensor]:
+    """The ROI's cells as a multi-vector query: the multi-vector counterpart of `roi_query`.
+
+    embeddings: float32 `B x E x h x w` (or `E x h x w`); mask: int64 `h x w` (one ROI for every image)
+    or `B x h x w`.  Returns (cells bf16 `M x E`, sets int64 `B + 1`): the rows of `maps_to_rows` whose
+    cell's mask value is `class_index`, image by image in row-major cell order, and the offsets of each
+    image's rows (an image without such a cell gives an empty set).  Pass them as `queries, sets` to
+    `EmbeddingStore.search_images_maxsim`."""
+    from imagescry_b200.store_format import maps_to_rows
+
+    _lib.require_cuda(embeddings, "embeddings")
+    _lib.require_cuda(mask, "mask")
+    emb = embeddings.unsqueeze(0) if embeddings.ndim == 3 else embeddings
+    if emb.ndim != 4 or emb.dtype != torch.float32:
+        raise ValueError(f"embeddings must be float32 B x E x h x w, got {embeddings.dtype} {tuple(embeddings.shape)}")
+    b, e, h, w = emb.shape
+    if mask.dtype != torch.int64 or tuple(mask.shape) not in ((h, w), (b, h, w)):
+        raise ValueError(f"mask must be int64 {h}x{w} or {b}x{h}x{w}, got {mask.dtype} {tuple(mask.shape)}")
+    if mask.device != emb.device:
+        raise ValueError(f"embeddings and mask are on different devices ({emb.device}, {mask.device})")
+    covered = (mask == class_index).expand(b, h, w).reshape(b, h * w)
+    cells = maps_to_rows(emb)[covered.reshape(-1)]
+    sets = torch.zeros(b + 1, dtype=torch.int64, device=emb.device)
+    sets[1:] = covered.sum(dim=1).cumsum(0)
+    return cells, sets
+
+
+__all__: Sequence[str] = ("create_roi_mask", "polygon_edges", "roi_cells", "roi_query")

@@ -219,6 +219,30 @@ def gather_group_records(records: Tensor, group=None) -> Tensor:
     return out.view(world, q, k, three)
 
 
+def maxsim_block_plan(offsets: Tensor, num_queries: int, budget_bytes: int) -> list[tuple[int, int]]:
+    """Image-aligned blocks of a multi-vector search (`search_images_maxsim`): `offsets` (images + 1
+    row offsets) → [(first image, end image)) in order, covering every image, each block's Q × images
+    fp32 cell-max matrix within `budget_bytes` and at least one image per block (an image whose column
+    alone exceeds the budget gets a block of its own)."""
+    if isinstance(budget_bytes, bool) or not isinstance(budget_bytes, int) or budget_bytes < 1:
+        raise ValueError(f"budget_bytes must be a positive int, got {budget_bytes!r}")
+    images = len(offsets) - 1
+    per = max(1, budget_bytes // max(1, 4 * num_queries))
+    return [(i, min(images, i + per)) for i in range(0, images, per)]
+
+
+def combine_cut_columns(ids: Tensor, columns: Tensor, image: int) -> Tensor:
+    """Cell-max column of an image cut by shard boundaries: the element-wise max of every gathered
+    column (`columns` R×Q fp32) whose id (`ids` R) is `image`.  A max of maxima is exact, so the result
+    is the column the unsharded store computes."""
+    if ids.ndim != 1 or columns.ndim != 2 or columns.shape[0] != ids.shape[0]:
+        raise ValueError("ids must be R and columns R×Q")
+    pick = ids == image
+    if not bool(pick.any()):
+        raise ValueError(f"no column of image {image}")
+    return columns[pick].amax(dim=0)
+
+
 def range_threshold(threshold) -> float:
     """The range search's threshold as the fp32 value the kernel compares against (a finite float)."""
     if isinstance(threshold, Tensor):
@@ -350,6 +374,7 @@ class EmbeddingStore:
         the results is row0 + its layout row."""
         self.row_group = row_groups(offsets, begin, begin + len(self)).to(self.device)
         self.group_first_row = (offsets[:-1] + row0).to(self.device)
+        self._layout = (offsets, begin)
 
     def __len__(self) -> int:
         return self.embeddings.shape[0]
@@ -469,6 +494,97 @@ class EmbeddingStore:
         by (score desc, row asc); if the store has fewer than k images the tail is (-inf, -1, -1)."""
         scores, rows, images = self.search_images_raw(queries, k)
         return scores, images.to(torch.int64), image_cells(rows, images, self.group_first_row)
+
+    def _maxsim_prepare(self, queries: Tensor, sets, k: int):
+        """Checks of a multi-vector search: (prepared queries, set offsets int64 CPU)."""
+        if self.row_group is None:
+            raise ValueError("search_images_maxsim needs a store built with groups= (rows per image or row offsets)")
+        self._check_k(k)
+        q = self._queries(queries)
+        return q, group_offsets(sets, q.shape[0])
+
+    def _maxsim_records(self, q: Tensor, qr: Tensor, set_off: Tensor, k: int, budget_bytes: int, *,
+                        shard: bool = False) -> tuple[list[Tensor], list[tuple[int, Tensor]]]:
+        """Per image-aligned block of this store's rows: one `isx_knn_maxsim` and one
+        `isx_maxsim_sets_topk`.  Returns the blocks' S×k packed records and, with `shard`, the
+        (image, cell-max column) of the store's first and last image when a shard boundary cuts them;
+        those images are left out of the records."""
+        offsets, begin = self._layout
+        n, nq, num_sets = len(self), q.shape[0], len(set_off) - 1
+        if n == 0:
+            return [], []
+        end = begin + n
+        lo = int(torch.searchsorted(offsets, torch.tensor([begin]), right=True)[0]) - 1
+        hi = int(torch.searchsorted(offsets, torch.tensor([end - 1]), right=True)[0])  # one past the last image
+        local = offsets[lo:hi + 1].clamp(begin, end) - begin
+        cut_first = shard and int(offsets[lo]) < begin
+        cut_last = shard and int(offsets[hi]) > end
+        plan = maxsim_block_plan(local, nq, budget_bytes)
+        lib = _lib.load()
+        with torch.cuda.device(self.device):
+            ws = self._ws(_lib.KNN_RANGE_WORKSPACE_BYTES)
+        cell = torch.empty(nq * max(b - a for a, b in plan), dtype=torch.float32, device=self.device)
+        sets_dev = set_off.to(self.device)
+        records, edges = [], []
+        for a, b in plan:
+            r0, r1, ng = int(local[a]), int(local[b]), b - a
+            cm = cell[: nq * ng].view(nq, ng)
+            rows = self.embeddings[r0:r1]
+            with _lib.on_device(rows, q, qr, cm, ws, self.row_group) as stream:
+                rc = lib.isx_knn_maxsim(
+                    rows.data_ptr(), self.rnorm[r0:].data_ptr(), self.row_group[r0:].data_ptr(), r1 - r0, q.data_ptr(),
+                    qr.data_ptr(), nq, q.shape[1], lo + a, ng, cm.data_ptr(), ws.data_ptr(), ws.numel(), stream,
+                )
+            _lib.check(rc, "isx_knn_maxsim")
+            first, last = cut_first and a == 0, cut_last and b == len(local) - 1
+            c0 = 1 if first else 0
+            c1 = max(c0, ng - 1 if last else ng)
+            if first:
+                edges.append((lo, cm[:, 0].clone()))
+            if last:
+                edges.append((hi - 1, cm[:, ng - 1].clone()))
+            records.append(self._maxsim_sets_topk(cm, qr, c0, c1, lo + a, sets_dev, num_sets, k))
+        return records, edges
+
+    def _maxsim_sets_topk(self, cm: Tensor, qr: Tensor, c0: int, c1: int, group_base: int, sets_dev: Tensor,
+                          num_sets: int, k: int) -> Tensor:
+        """One `isx_maxsim_sets_topk` over columns [c0, c1) of the cell-max matrix `cm`: S×k records."""
+        rec = torch.empty((num_sets, k), dtype=torch.int64, device=self.device)
+        nq, ng = cm.shape
+        with _lib.on_device(cm, qr, sets_dev, rec) as stream:
+            rc = _lib.load().isx_maxsim_sets_topk(cm.data_ptr(), qr.data_ptr(), nq, ng, c0, c1, sets_dev.data_ptr(), num_sets,
+                                                  k, group_base, rec.data_ptr(), stream)
+        _lib.check(rc, "isx_maxsim_sets_topk")
+        return rec
+
+    def search_images_maxsim(self, queries: Tensor, sets, k: int, *, budget_bytes: int = 1 << 30) -> tuple[Tensor, Tensor]:
+        """Multi-vector image search (late interaction, "MaxSim"): the k best images for every query SET.
+
+        `sets` says which query rows form one set: an int m (consecutive sets of m rows; Q % m == 0) or a
+        1-D offsets tensor from 0 to Q (set s = rows [offsets[s], offsets[s + 1]); sets may be empty).
+        Image I scores, for the set S,
+
+            score(S, I) = (1 / |S|) · Σ_{c ∈ S} max_{r ∈ I} cos(q_c, e_r)
+
+        where the cosine of (c, r) is bit for bit the fp32 score `search` reports, so each term is the
+        `search_images` score of image I for row c.  The terms are summed in fp32 in ascending row order
+        and the sum is divided (correctly rounded) by |S|: the result does not depend on the store's
+        blocks or tiles.  Returns (scores fp32 S×k, images int64 S×k), ordered by (score desc, image
+        asc) and padded with (-inf, -1) when there are fewer than k images; an empty set gets padding
+        only.  Needs a store built with `groups=`.
+
+        The per-(row, image) maxima are formed in the search kernel's epilogue (`isx_knn_maxsim`): the
+        Q × N score matrix never exists, only Q × images fp32 maxima, in image-aligned blocks of at most
+        `budget_bytes` each (at least one image per block)."""
+        q, set_off = self._maxsim_prepare(queries, sets, k)
+        num_sets = len(set_off) - 1
+        nq = q.shape[0]
+        if nq == 0 or len(self) == 0:
+            return (torch.full((num_sets, k), float("-inf"), dtype=torch.float32, device=self.device),
+                    torch.full((num_sets, k), -1, dtype=torch.int64, device=self.device))
+        records, _ = self._maxsim_records(q, row_rnorm(q), set_off, k, budget_bytes)
+        scores, images = merge_topk_packed(torch.stack(records), k)
+        return scores, images.to(torch.int64)
 
     def scan_fp8(self, queries: Tensor, k: int) -> tuple[Tensor, Tensor]:
         """The fp8 scan alone (`isx_knn_search_fp8`): the top-k of the E4M3 copies of the queries and
@@ -714,6 +830,48 @@ class ShardedEmbeddingStore:
         s, r, g = self.local.search_images_raw(queries, k)
         merged_s, merged_r, merged_g = merge_topk_groups(gather_group_records(pack_group_records(s, r, g), self.group), k)
         return merged_s, merged_g.to(torch.int64), image_cells(merged_r, merged_g, self.local.group_first_row)
+
+    def search_images_maxsim(self, queries: Tensor, sets, k: int, *, budget_bytes: int = 1 << 30) -> tuple[Tensor, Tensor]:
+        """`EmbeddingStore.search_images_maxsim` over the sharded store, bit for bit the unsharded result.
+
+        Every rank scores the images whose rows it holds entirely.  An image cut by a shard boundary is
+        scored by the rank that holds its first row: every rank keeps the cell-max columns (Q floats)
+        of its first and last image when a boundary cuts them, one all-gather moves those columns and
+        their image ids, and the owner combines them by max (`combine_cut_columns`, exact) and scores
+        the image with the same set-reduce kernel.  Then one all-gather of the S×k packed records and
+        one merge."""
+        import torch.distributed as dist
+
+        st = self.local
+        q, set_off = st._maxsim_prepare(queries, sets, k)
+        num_sets, nq, dev = len(set_off) - 1, q.shape[0], st.device
+        if nq == 0 or num_sets == 0:
+            return (torch.full((num_sets, k), float("-inf"), dtype=torch.float32, device=dev),
+                    torch.full((num_sets, k), -1, dtype=torch.int64, device=dev))
+        qr = row_rnorm(q)
+        records, edges = st._maxsim_records(q, qr, set_off, k, budget_bytes, shard=True)
+        # rows of the edge exchange: int32 [image id or -1, Q fp32 bit patterns], first and last image
+        send = torch.zeros((2, nq + 1), dtype=torch.int32, device=dev)
+        send[:, 0] = -1
+        for j, (image, col) in enumerate(edges[:2]):
+            send[j, 0] = image
+            send[j, 1:] = col.view(torch.int32)
+        got = torch.empty((self.world_size * 2, nq + 1), dtype=torch.int32, device=dev)
+        dist.all_gather_into_tensor(got, send, group=self.group)
+        offsets, begin = st._layout
+        for image, _ in edges:
+            # the last image of this shard, cut at its end and starting here: this rank owns it
+            if int(offsets[image]) >= begin and int(offsets[image + 1]) > begin + len(st):
+                col = combine_cut_columns(got[:, 0], got[:, 1:].contiguous().view(torch.float32), image)
+                records.append(st._maxsim_sets_topk(col.view(nq, 1), qr, 0, 1, image, set_off.to(dev), num_sets, k))
+        if records:
+            s, i = merge_topk_packed(torch.stack(records), k)
+            mine = pack_records(s, i)
+        else:
+            mine = pack_records(torch.full((num_sets, k), float("-inf"), device=dev),
+                                torch.full((num_sets, k), -1, dtype=torch.int32, device=dev))
+        scores, images = merge_topk_packed(gather_records(mine, self.group), k)
+        return scores, images.to(torch.int64)
 
     def search_fp8(self, queries: Tensor, k: int, *, candidates: int = FP8_CANDIDATES) -> tuple[Tensor, Tensor]:
         """`EmbeddingStore.search_fp8` over the sharded store (built with `fp8=True`): local fp8 scan and

@@ -291,6 +291,33 @@ int isx_knn_rescore(const void* store, const float* rnorm, int64_t n, const void
                     int q, int d, const int32_t* cand, int kc, int64_t index_base, int k, float* out_scores,
                     int32_t* out_idx, isx_stream_t stream);
 
+/* Multi-vector (maxsim) image search, stage 1 of 2: the per-(query row, group) maxima.  store, queries,
+ * their inverse norms, q and d as for isx_knn_search; row_group: int32 n, the group (image) id of every
+ * store row (any order; rows of one group need not be consecutive).  cell_max: fp32 q x num_groups,
+ * row-major, indexed in 64 bits, written in place: this call first sets every entry to -inf, then
+ * entry [c][g - group_base] receives the largest fl(dot(q_c, e_r) * rnorm(e_r)) over the rows r of
+ * group g, i.e. the score isx_knn_search reports for (c, r) before the query's inverse norm; so
+ * fl(cell_max[c][g - group_base] * query_rnorm[c]) is bit for bit the best isx_knn_search score of row c
+ * over group g (-0 is stored as +0).  Rows whose group lies outside [group_base, group_base +
+ * num_groups) write nothing.  The maxima are formed in the search kernel's epilogue and merged by atomic
+ * max on the float (signed-int max for values >= 0, unsigned-int min for values < 0): the score matrix
+ * never exists.  workspace: at least ISX_KNN_RANGE_WORKSPACE_BYTES of device memory. */
+int isx_knn_maxsim(const void* store, const float* store_rnorm, const int32_t* row_group, int64_t n,
+                   const void* queries, const float* query_rnorm, int q, int d, int64_t group_base,
+                   int64_t num_groups, float* cell_max, void* workspace, size_t workspace_bytes,
+                   isx_stream_t stream);
+/* Stage 2: set scores and top-k.  Query set s is the rows [set_offsets[s], set_offsets[s + 1]) (int64,
+ * device memory, num_sets + 1 entries, non-decreasing in [0, q]).  For every column col in [col_begin,
+ * col_end) of cell_max (as written by isx_knn_maxsim), score(s, col) = the fp32 sum over the set's rows
+ * c in ascending order of fl(cell_max[c][col] * query_rnorm[c]), divided (correctly rounded) by the
+ * set's size; columns scoring -inf (groups without rows) are skipped.  records: num_sets x k packed
+ * 8-byte records {fp32 score bits, int32 group_base + col}, the best k ordered by (score desc, group
+ * asc), padded with (-inf, -1); an empty set gets padding only.  1 <= k <= 128.  Records of several
+ * column blocks merge with isx_topk_merge_packed. */
+int isx_maxsim_sets_topk(const float* cell_max, const float* query_rnorm, int q, int64_t num_groups,
+                         int64_t col_begin, int64_t col_end, const int64_t* set_offsets, int num_sets, int k,
+                         int64_t group_base, void* records, isx_stream_t stream);
+
 /* ---- ROI masks on the feature-map grid (SURVEY.md 8f-4) ---------------------------------------
  * geometry.py:14-65 `create_roi_mask`: rasterio.features.rasterize(shapes, out_shape=(hf, wf),
  * transform=Affine.scale(w / wf, h / hf), fill=0, all_touched=True) * class_index.  rasterio / GDAL
